@@ -2,7 +2,7 @@
 """Benchmark of the dense-correspondence matching path (BASELINE.json metric: image pairs / s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload navi|scannet|spair|all]
-                    [--pairs P] [--features backbone|gaussian] [--dtype f16|bf16|tf32]
+                    [--pairs P] [--features backbone|gaussian] [--dtype f16|bf16|tf32] [--dump-outputs DIR]
 
 One "step" = one batch of PAIRS_PER_STEP synthetic image pairs through the hot path (kernels 1-3 + scoring).
 The HEADLINE workload (top-level keys of the one JSON line) is BASELINE.json configs[1]: NAVI-shaped pairs, ViT-B/16 @
@@ -204,12 +204,60 @@ def cpu_pairs_per_s(ctx, workload, budget_s=12.0, max_pairs=6):
             "sample": f"{done} pairs of the same workload through oracle/restated.py (CPU fp32 torch port, exact brute-force k-NN)"}
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def write_outputs(ctx, dirname, prefix, arrays):
+    """--dump-outputs: every array as dirname/<prefix>_<name>.npy (rank 0 only).  The inputs are seeded, so two builds
+    run with the same arguments can be compared file by file."""
+    import numpy as np
+
+    if ctx.rank != 0:
+        return
+    ctx.dumped_bytes = getattr(ctx, "dumped_bytes", 0) + sum(a.nbytes for a in arrays.values())
+    if ctx.dumped_bytes > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs would write {ctx.dumped_bytes} bytes (at most {DUMP_MAX_BYTES})")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(dirname, f"{prefix}_{name}.npy"), a)
+
+
+def dense_outputs(last, pool_dev, pool_ids, acc):
+    """The matches a caller of the timed path holds after its last step: per pair the selected (query row, target row,
+    weight, mutual-NN flag) of mv_k3_topk_matches, entries past the pair's live match count set to -1, and the recall hit
+    counters of the whole timed region.  A lane of the CUDA-graph pipeline overwrites its results with its next pair, so
+    of the last step the last pair of every lane is still held (all pairs without the graph): those are written."""
+    import numpy as np
+
+    held = {}
+    for j, (p, r) in enumerate(last):
+        held[id(r)] = (j, p, r)
+    rows = sorted(held.values(), key=lambda x: x[0])
+    k = max(max(r.k, 1) for _, _, r in rows)
+    src, dst, wgt, mut = (np.full((len(rows), k), -1.0, dtype=dt) for dt in (np.float64, np.float64, np.float32, np.float32))
+    count, pair, pos = (np.zeros(len(rows)) for _ in range(3))
+    for i, (j, p, r) in enumerate(rows):
+        n = int(r.k_dev.item())
+        sel = r.sel_src[:n].long()
+        src[i, :n] = sel.cpu().numpy()
+        dst[i, :n] = r.sel_dst[:n].cpu().numpy()
+        wgt[i, :n] = r.sel_weight[:n].cpu().numpy()
+        mut[i, :n] = r.mutual[sel].cpu().numpy()
+        count[i] = n
+        pair[i] = pool_ids[next(s for s, q in enumerate(pool_dev) if q is p)]
+        pos[i] = j
+    return {"pair": pair, "position_in_step": pos, "match_count": count, "sel_src": src, "sel_dst": dst, "sel_weight": wgt,
+            "sel_mutual": mut, "hits": acc.hits.cpu().double().numpy()}
+
+
 # --------------------------------------------------------------------------------------------------------------
 # the two dense workloads (NAVI / ScanNet shaped)
 # --------------------------------------------------------------------------------------------------------------
-def run_dense(ctx, workload, steps, warmup, fixed_pairs=0, light=False):
+def run_dense(ctx, workload, steps, warmup, fixed_pairs=0, light=False, dump=None):
     """one dense workload -> record.  fixed_pairs > 0: strong scaling over a fixed seeded set (configs[3]).
-    light: only the device-resident arm and the end-to-end helper arm (the secondary workloads of a default run)."""
+    light: only the device-resident arm and the end-to-end helper arm (the secondary workloads of a default run).
+    dump: directory that receives the matches of the timed region's last step (dense_outputs)."""
     args, mv, dev, world, rank = ctx.args, ctx.mv, ctx.dev, ctx.world, ctx.rank
     C_, ev, L = mv.correspondence, mv.evaluation, mv._lib
     hbm_peak, tc_peak, tc_sustained, peak_kind = peaks()
@@ -264,10 +312,14 @@ def run_dense(ctx, workload, steps, warmup, fixed_pairs=0, light=False):
     else:
         sched = [[pool_dev[(s * PAIRS_PER_STEP + j) % POOL] for j in range(PAIRS_PER_STEP)] for s in range(steps)]
 
-    def run_sched(which, a=acc):
-        for s in which:
+    def run_sched(which, a=acc, keep=False):
+        """keep: -> [(pair, MatchResult)] of the last step (what --dump-outputs writes); without it no result is held,
+        so that an eager (--no-graph) pass frees every pair's buffers as before"""
+        which = list(which)
+        for s in (which[:-1] if keep else which):
             for p in sched[s % len(sched)]:
                 pair_device(p, a)
+        return [(p, pair_device(p, a)) for p in sched[which[-1] % len(sched)]] if keep and which else []
 
     # ---------------- device-resident arm (value) ----------------
     run_sched(range(warmup))
@@ -280,13 +332,15 @@ def run_dense(ctx, workload, steps, warmup, fixed_pairs=0, light=False):
     ctx.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    run_sched(range(steps))
+    last = run_sched(range(steps), keep=bool(dump))
     if gm is not None:
         gm.join()
     acc.all_reduce()  # the path's only collective: int64 hit counts
     e1.record()
     ctx.barrier()
     clocks = sampler.stop()
+    if dump:
+        write_outputs(ctx, dump, workload, dense_outputs(last, pool_dev, pool_ids, acc))
     launches = L.LAUNCHES["count"]
     ms_total = ctx.max_over_ranks(e0.elapsed_time(e1))
     summary = acc.summary()
@@ -602,9 +656,10 @@ SPAIR_BATCH = 2368  # pairs per step (one launch) = 8 per CTA at 2 CTAs x 148 SM
 SPAIR_BATCH_E2E = 1184  # pairs per step of the end-to-end arm (1.4 GB of pinned host memory per rank)
 
 
-def run_spair(ctx, steps, warmup):
+def run_spair(ctx, steps, warmup, dump=None):
     """SPair-shaped pairs, (2, 768, 14, 14) features + 20 key points, a step = SPAIR_BATCH pairs through
-    spair.compute_errors_batch (one fused launch).  HBM-bound: the roofline figure is the feature bytes read per launch."""
+    spair.compute_errors_batch (one fused launch).  HBM-bound: the roofline figure is the feature bytes read per launch.
+    dump: directory that receives the four (B, K) results of the last timed launch and the PCK counts."""
     mv, dev, world, rank = ctx.mv, ctx.dev, ctx.world, ctx.rank
     sp, L = mv.spair, mv._lib
     hbm_peak, _, _, peak_kind = peaks()
@@ -629,13 +684,18 @@ def run_spair(ctx, steps, warmup):
     sampler = ClockSampler(ctx.local_rank).start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(steps):
+    for _ in range(steps - 1):
         step(d)
+    last = step(d)
     if world > 1:
         ctx.dist.all_reduce(hits, op=ctx.dist.ReduceOp.SUM)  # the path's only collective: PCK counts
     e1.record()
     ctx.barrier()
     clocks = sampler.stop()
+    if dump:
+        names = ("error_same", "error_nn", "index_nn", "pred")
+        arrays = {nm: t.cpu().to(torch.float32 if t.is_floating_point() else torch.float64).numpy() for nm, t in zip(names, last)}
+        write_outputs(ctx, dump, "spair", dict(arrays, hits=hits.cpu().double().numpy()))
     launches = L.LAUNCHES["count"]
     ms_total = ctx.max_over_ranks(e0.elapsed_time(e1))
     value = world * steps * B / (ms_total * 1e-3)
@@ -830,7 +890,9 @@ def h2d_link_probe(ctx, bytes_per_pair):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of the headline workload (default 20); the ScanNet / SPair records of --workload all time "
+                         "max(3, K // 4) / max(5, K // 2) steps, and --pairs sets its own count (the two do not combine)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="all", choices=["all", "navi", "scannet", "spair"],
@@ -853,7 +915,14 @@ def main():
     ap.add_argument("--feat-layout", default="chw", choices=["chw", "hwc"],
                     help="memory layout of the (C, h, w) feature tensors handed to the path: chw = contiguous, as the "
                          "reference's tokens_to_output returns them; hwc = channel-last views (ViT token order), no transpose kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of each workload, write what its last step computed as DIR/<workload>_<name>.npy")
     args = ap.parse_args()
+    if args.pairs and args.steps is not None:
+        ap.error("--pairs P times ceil(P / N / 32) steps of its fixed set; it does not take --steps")
+    args.steps = 20 if args.steps is None else args.steps
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -866,10 +935,11 @@ def main():
         print(json.dumps({"k1": k1_record(ctx), "k1_grid": ctx.mv.correspondence._CFG["k1_grid"]}), flush=True)
         return
     head = "navi" if args.workload == "all" else args.workload
+    dump = args.dump_outputs
     if head == "spair":
-        line = run_spair(ctx, args.steps, args.warmup)
+        line = run_spair(ctx, args.steps, args.warmup, dump=dump)
     else:
-        line = run_dense(ctx, head, args.steps, args.warmup, fixed_pairs=args.pairs)
+        line = run_dense(ctx, head, args.steps, args.warmup, fixed_pairs=args.pairs, dump=dump)
         if ctx.world == 1 and ctx.rank == 0 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_pairs_per_s(ctx, head)
     line["host_binding"] = ctx.binding
@@ -877,7 +947,8 @@ def main():
         line["e2e"]["h2d_link"] = h2d_link_probe(ctx, line["e2e"]["h2d_bytes_per_step"] / line["config"]["pairs_per_step"])
     if args.workload == "all":
         sub_steps = max(3, args.steps // 4)
-        line["workloads"] = {"scannet": run_dense(ctx, "scannet", sub_steps, 3, light=True), "spair": run_spair(ctx, max(5, args.steps // 2), 3)}
+        line["workloads"] = {"scannet": run_dense(ctx, "scannet", sub_steps, 3, light=True, dump=dump),
+                             "spair": run_spair(ctx, max(5, args.steps // 2), 3, dump=dump)}
         if ctx.world == 1 and ctx.rank == 0 and not args.no_cpu_baseline:
             line["workloads"]["scannet"]["cpu_baseline"] = cpu_pairs_per_s(ctx, "scannet", budget_s=10.0, max_pairs=3)
         if not args.pairs:

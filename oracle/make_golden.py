@@ -1,7 +1,8 @@
 """TEST INFRASTRUCTURE ONLY.  Generate tests/golden/*.npz by running the reference's OWN module
-(/root/reference/evals/utils/correspondence.py, imported unmodified through oracle/reference_loader.py
+(evals/utils/correspondence.py of a checkout of the reference project at oracle/_ref/ or
+$MV_REFERENCE_ROOT, imported unmodified through oracle/reference_loader.py
 with the exact brute-force faiss stand-in) on the seeded synthetic inputs of
-midvision-probe_b200/synthetic.py.  Run in the build container only:
+midvision-probe_b200/synthetic.py.  Needs that checkout:
 
     python -m oracle.make_golden
 

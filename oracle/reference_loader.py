@@ -1,14 +1,14 @@
-"""TEST INFRASTRUCTURE ONLY.  Import the reference's own matching code, unmodified, from /root/reference.
+"""TEST INFRASTRUCTURE ONLY.  Import the reference's own matching code, unmodified, from a checkout of the
+reference project: $MV_REFERENCE_ROOT, or oracle/_ref/ (git-ignored; the reference is not part of this repository).
 
-Only usable in the build container (the reference tree does not travel to the GPU box); callers must
-check `available()` first.  Used by oracle/make_golden.py and by the CPU tests that pin
-oracle/restated.py to the real thing.
+Callers must check `available()` first.  Used by oracle/make_golden.py and by the CPU tests that pin
+oracle/restated.py to the real thing (tests/test_oracle.py, which falls back to stored values without it).
 """
 import importlib
 import os
 import sys
 
-REFERENCE_ROOT = os.environ.get("MV_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("MV_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available():
@@ -106,7 +106,7 @@ def spair_evaluate_dataset_reference(pairs, thresh=0.10):
 
 def navi_error_block_reference(feats_0, feats_1, xyz_grid_0, xyz_grid_1, Rt_gt, intrinsics, num_corr, scale_factor=0.25):
     """Execute the reference's OWN NAVI evaluation loop -- the text of evaluate_navi_correspondence.py from
-    `num_instances = len(loader.dataset)` up to the CSV header (lines 174-221), read from /root/reference at call time,
+    `num_instances = len(loader.dataset)` up to the CSV header (lines 174-221), read from REFERENCE_ROOT at call time,
     never copied into this repo -- with the script's names bound to the reference's own functions (faiss shimmed),
     tqdm / wandb / print silenced and cfg / loader replaced by stand-ins.  Returns the variables the block leaves
     behind."""

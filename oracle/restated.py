@@ -1,10 +1,10 @@
 """TEST INFRASTRUCTURE ONLY -- CPU restatement (fp32 torch on the host) of the reference's matching path.
 
-Each function names the reference lines it follows (paths relative to /root/reference).  The k-NN
+Each function names the reference lines it follows (paths relative to the reference project's root).  The k-NN
 backend of the reference, faiss-gpu 1.8.0 GpuIndexFlatL2 (not in the tree; README.md:60), is restated
 from its published behaviour: exact brute-force squared-L2 search, ascending, int64 labels.
 
-Checked against (a) the reference's own module imported from /root/reference and (b) the golden vectors
+Checked against (a) the reference's own module imported from a checkout of it (oracle/reference_loader.py; where present) and (b) the golden vectors
 under tests/golden/ by tests/test_oracle.py.  Never imported by the product.
 """
 import torch

@@ -1,6 +1,6 @@
 """Pin oracle/restated.py: against the golden vectors produced by the reference's own module
-(tests/golden, made by oracle/make_golden.py) and, where /root/reference is present, against that
-module directly on fresh inputs."""
+(tests/golden, made by oracle/make_golden.py) and, where a checkout of the reference is present (oracle/_ref/ or
+$MV_REFERENCE_ROOT, oracle/reference_loader.py), against that module directly on fresh inputs."""
 import numpy as np
 import pytest
 import torch
