@@ -283,6 +283,29 @@ int mv_k2_profile_read(float* ms_out, int max_n);
 int mv_k2_profile_dims(int* nmc_out, int max_n);
 int mv_k2_unpack_col(const unsigned long long* col_best, int m, float* col_val, int32_t* col_idx, mv_stream_t stream);
 
+/* ---- k > 2 nearest neighbours: kernel 2 with a row top-KP epilogue + an fp32 re-rank ------------ */
+/* The same GEMM as mv_k2_sim_top2_ld with an epilogue that keeps the kp (8 or 16) largest S[i, :] of every row instead of
+ * the top-2 and the column arg-max:
+ *   row_val/row_idx (n_max, kp): values descending, ties to the lower column; missing entries (m < kp, columns past *m_dev,
+ *                                rows past *n_dev) = MV_SIM_MASKED / -1.
+ * Positions 0 and 1 equal mv_k2_sim_top2_ld's row outputs bit for bit on the same operands and cluster form (stream-K off).
+ * The schedule is always tile-granular (mv_k2_set_streamk does not apply) and the launch is not recorded by
+ * mv_k2_profile_*.  Other arguments as mv_k2_sim_top2_ld; workspace from mv_k2_topk_workspace_bytes (0 for a bad kp). */
+size_t mv_k2_topk_workspace_bytes(int n_max, int m_max, int kp);
+int mv_k2_sim_topk_ld(const void* A, int lda, const void* B, int ldb, int n_max, int m_max, int C, const int32_t* n_dev,
+                      const int32_t* m_dev, int dtype, int cluster, int kp, float* row_val, int32_t* row_idx, void* workspace,
+                      size_t workspace_bytes, mv_stream_t stream);
+/* fp32 re-rank of kp candidates per query (cand (n_max, kp) int32, e.g. row_idx above; -1 = no candidate): the distance of
+ * query row Q[i] (n_max, ldq) to every candidate row T[j] (ldt) over C columns --
+ *   MV_METRIC_L2SQ     sum (q - t)^2                                  (faiss' squared L2)
+ *   MV_METRIC_COSINE   1 - q.t / (max(|q|, 1e-8) * max(|t|, 1e-8))    (kernel 3's cosine distance)
+ * -- sorted ascending, ties to the lower index; out_dist / out_idx (n_max, k) receive the first k, 1 <= k <= kp
+ * (missing: +inf / -1, also for rows past *n_dev).  128-bit loads when C and both pitches are multiples of 4 floats. */
+#define MV_METRIC_L2SQ 0
+#define MV_METRIC_COSINE 1
+int mv_knn_rerank(const float* Q, int ldq, const float* T, int ldt, int C, const int32_t* n_dev, int n_max, const int32_t* cand,
+                  int kp, int k, int metric, float* out_dist, int32_t* out_idx, mv_stream_t stream);
+
 /* ---- kernel 3: fp32 distance recompute, ratio test, mutual check, selection, scoring ---- */
 /* Per query row i with candidates j0, j1 = row_idx[i]:  d_k = 1 - cos(A32[i], B32[j_k]) in fp32
  * (knn_points, correspondence.py:53-58); candidates are re-ranked so d_0 <= d_1 (row_idx is updated

@@ -52,6 +52,9 @@ PROTOTYPES = {
     "mv_k2_profile_read": (c_int, [P, c_int]),
     "mv_k2_profile_dims": (c_int, [P, c_int]),
     "mv_k2_unpack_col": (c_int, [P, c_int, P, P, P]),
+    "mv_k2_topk_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "mv_k2_sim_topk_ld": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, P, P, c_int, c_int, c_int, P, P, P, c_size_t, P]),
+    "mv_knn_rerank": (c_int, [P, c_int, P, c_int, c_int, P, c_int, P, c_int, c_int, c_int, P, P, P]),
     "mv_k3_ratio_mutual": (c_int, [P, P, c_int, P, c_int, P, P, c_int, P, P, P, P]),
     "mv_k3_ratio_mutual_split": (c_int, [P, P, P, P, c_int, P, c_int, P, P, c_int, P, P, P, P]),
     "mv_k3_ratio_mutual_f16c": (c_int, [P, P, P, P, c_int, c_int, P, P, c_int, P, P, c_int, P, P, P, P]),
@@ -77,13 +80,14 @@ MV_FEAT_F32, MV_FEAT_BF16, MV_FEAT_F16 = 0, 1, 2
 MV_LR_MAX_SOURCE_PIXELS = 1024
 MV_SIM_MASKED = -3.0e38
 MV_MAX_THRESHOLDS = 16
+MV_METRIC_L2SQ, MV_METRIC_COSINE = 0, 1
 
 _lib = None
 
 # kernels launched per entry point (for bench.py's gpu_launches claim); memsets are not counted
 KERNELS_PER_CALL = {
     "mv_chw_to_hwc": 1, "mv_feat_to_hwc_f32": 1, "mv_compact_valid": 1, "mv_geom_backproject": 1, "mv_geom_project_coords": 1,
-    "mv_geom_grid_coords": 1, "mv_geom_keypoint_coords": 1, "mv_k1_sample_normalize": 1, "mv_k1_sample_f16c": 1, "mv_k1_sample_tf32c": 1, "mv_rows_center": 2, "mv_rows_dot": 1, "mv_rank_of_valid": 1, "mv_k1_grid_f16c": 1, "mv_lr_unit_rows": 1, "mv_lr_gram_exact": 2, "mv_lr_build_query": 1, "mv_lr_build_target": 1, "mv_k3_ratio_mutual_lr": 1, "mv_k2_sim_top2": 2, "mv_k2_sim_top2_ld": 2, "mv_k2_affinity": 2, "mv_affinity_threshold": 1, "mv_cosine_2afc": 1,
+    "mv_geom_grid_coords": 1, "mv_geom_keypoint_coords": 1, "mv_k1_sample_normalize": 1, "mv_k1_sample_f16c": 1, "mv_k1_sample_tf32c": 1, "mv_rows_center": 2, "mv_rows_dot": 1, "mv_rank_of_valid": 1, "mv_k1_grid_f16c": 1, "mv_lr_unit_rows": 1, "mv_lr_gram_exact": 2, "mv_lr_build_query": 1, "mv_lr_build_target": 1, "mv_k3_ratio_mutual_lr": 1, "mv_k2_sim_top2": 2, "mv_k2_sim_top2_ld": 2, "mv_k2_affinity": 2, "mv_k2_sim_topk_ld": 2, "mv_knn_rerank": 1, "mv_affinity_threshold": 1, "mv_cosine_2afc": 1,
     "mv_k2_unpack_col": 1, "mv_k3_ratio_mutual": 1, "mv_k3_ratio_mutual_split": 1, "mv_k3_ratio_mutual_f16c": 1, "mv_k3_topk_matches": 1, "mv_k3_score": 1, "mv_gather_rows": 1,
     "mv_pack_matches": 1, "mv_argmax_rows": 1, "mv_k3_spair_errors": 1, "mv_spair_match_batch": 1,
 }

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libmvmatch.so")
-SOURCES = ["api.cu", "k1_sample.cu", "k1_grid.cu", "k2_sim.cu", "lr_gram.cu", "k3_score.cu", "spair_batch.cu", "stage.cu"]
+SOURCES = ["api.cu", "k1_sample.cu", "k1_grid.cu", "k2_sim.cu", "lr_gram.cu", "k3_score.cu", "knn_rerank.cu", "spair_batch.cu", "stage.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

@@ -220,6 +220,18 @@ class MatchResult:
     __slots__ = ("k", "k_dev", "sel_src", "sel_dst", "sel_weight", "mutual", "row_idx", "dists", "weight", "col_best")
 
 
+def _k2_operands(A16, A32, B16, B32, C):
+    """kernel 2's operands for prepared rows of C channels under the configured operand type: (A, B, columns of the
+    product, MV_DTYPE_*).  The 16-bit rows, or the centred tf32c planes, which ride in the same slot; plain fp32 rows
+    for tf32 without them.  f16c / tf32c rows add their 8 augmentation columns to the product."""
+    tf32 = _CFG["dtype"] == "tf32"
+    f16 = _CFG["dtype"] == "f16"
+    tf32c = tf32 and A16 is not None and B16 is not None
+    A, B = (A16, B16) if (not tf32 or tf32c) else (A32, B32)
+    Ck = C + 8 if (f16 or tf32c) else C
+    return A, B, Ck, L.MV_DTYPE_TF32 if tf32 else (L.MV_DTYPE_F16 if f16 else L.MV_DTYPE_BF16)
+
+
 def match_rows(A16, A32, B16, B32, n, m, num_corr, ratio_test=True, n_dev=None, m_dev=None, want_topk=True, run_k3=True,
                A_lo=None, B_lo=None, center_B=None, C=None, proposal=None):
     """kernel 2 + kernel 3 on prepared rows.
@@ -249,14 +261,10 @@ def match_rows(A16, A32, B16, B32, n, m, num_corr, ratio_test=True, n_dev=None, 
     lib = L.load()
     ws_bytes = lib.mv_k2_workspace_bytes(n, m)
     ws = _empty((ws_bytes,), torch.uint8, dev)
-    tf32c = tf32 and A16 is not None and B16 is not None  # centred tf32 operand planes ride in the operand-rows slot
-    A = A16 if (not tf32 or tf32c) else A32
-    B = B16 if (not tf32 or tf32c) else B32
     if split:
         C = A_lo.shape[1]
-    ld = A.shape[1]
-    Ck = C + 8 if (f16 or tf32c) else C  # f16c / tf32c rows: the 8 augmentation columns take part in the product
-    k2_A, k2_B, k2_dtype = A, B, L.MV_DTYPE_TF32 if tf32 else (L.MV_DTYPE_F16 if f16 else L.MV_DTYPE_BF16)
+    k2_A, k2_B, Ck, k2_dtype = _k2_operands(A16, A32, B16, B32, C)
+    ld = k2_A.shape[1]
     if proposal is not None:
         k2_A, k2_B, Ck = proposal
         k2_dtype = L.MV_DTYPE_F16
@@ -336,11 +344,13 @@ def _rows_pair(X_f, Y_f, dev):
 # ------------------------------------------------------------------------------------------------
 def faiss_knn(query, target, k):
     """L2 k-NN: (squared L2 distances ascending, int64 indices).  correspondence.py:14-23.
-    k <= 2 (every call site) runs on kernel 2; larger k takes the exact blocked search of _exact_knn_blocks.
+    k <= 16 runs on kernel 2 wherever the target has at least k rows; larger k, and targets with fewer than k rows, take
+    the exact blocked search of _exact_knn_blocks (which returns min(k, m) columns).
 
-    Neighbours are PROPOSED at tf32 precision (kernel 2's two best per row); the fp32 distances of the two decide
-    their order.  Ranking tolerance: a neighbour whose squared distance is within ~1e-3 relative of the second
-    candidate's can be missed (the north-star gap rule); missing neighbours (target smaller than k) come back as
+    Neighbours are PROPOSED at tf32 precision -- kernel 2's two best per row for k <= 2, its row top-KP epilogue
+    (KP = 8 for k <= 6, 16 up to k = 16) otherwise -- and fp32 distances recomputed from the rows decide their order
+    (mv_knn_rerank for k > 2).  Ranking tolerance: a neighbour whose squared distance is within ~1e-3 relative of the
+    last candidate's can be missed (the north-star gap rule); missing neighbours (target smaller than k) come back as
     (-1, inf) like faiss.
     The search runs on kernel 2 through the identity ||q-t||^2 = ||q||^2 + ||t||^2 - 2 q.t : the rows are
     extended by (1, -||t||^2/2) split into tf32-exact pieces so that the inner-product order is the L2
@@ -353,10 +363,40 @@ def faiss_knn(query, target, k):
     n, C = q.shape
     m = t.shape[0]
     if k > 2:
-        d, idx = _exact_knn_blocks(q, t, int(k))
-        return d.to(in_dev), idx.to(in_dev)
+        if not _fused_knn_applies(n, m, int(k)):
+            d, idx = _exact_knn_blocks(q, t, int(k))
+            return d.to(in_dev), idx.to(in_dev)
+        qe, te = _l2_operands(q, t)
+        cand = _topk_candidates(qe, te, n, m, qe.shape[1], L.MV_DTYPE_TF32, int(k))
+        d, idx = _rerank(q, t, cand, int(k), L.MV_METRIC_L2SQ)
+        return d.to(in_dev), idx.long().to(in_dev)
     if k < 1:
         raise ValueError("k must be positive")
+    qe, te = _l2_operands(q, t)
+    saved = dict(_CFG)
+    try:
+        _CFG["dtype"] = "tf32"
+        r = match_rows(None, qe, None, te, n, m, 0, want_topk=False, run_k3=False)
+    finally:
+        _CFG.update(saved)
+    # both candidates always: the tf32 product only PROPOSES them, their fp32 distances decide the order (so k = 1
+    # also returns the better of the two); a missing neighbour (m < k) is faiss's (-1, inf), never a wrapped index
+    idx = r.row_idx.long()
+    have = idx >= 0
+    d = ((q[:, None, :] - t[idx.clamp(min=0)]) ** 2).sum(dim=-1)
+    d = torch.where(have, d, torch.full_like(d, float("inf")))
+    swap = d[:, 1] < d[:, 0]
+    d = torch.where(swap[:, None], d.flip(1), d)
+    idx = torch.where(swap[:, None], idx.flip(1), idx)
+    return d[:, :k].contiguous().to(in_dev), idx[:, :k].contiguous().to(in_dev)
+
+
+def _l2_operands(q, t):
+    """kernel 2's tf32 operands of an L2 search: (n, Cp) query rows and (m, Cp) target rows whose inner-product order along
+    a row is the squared-L2 order."""
+    dev = q.device
+    n, C = q.shape
+    m = t.shape[0]
     # extra columns: q' = [q, 1, 1, 1, 0..], t' = [t, h0, h1, h2, 0..] with h0+h1+h2 = -||t||^2/2, each piece
     # holding <= 10 mantissa bits so the tf32 tensor-core product does not round it
     half = -0.5 * (t * t).sum(dim=1)
@@ -377,28 +417,45 @@ def faiss_knn(query, target, k):
     te[:, :C] = t - t.mean(dim=0, keepdim=True) if m > 1 else t
     for i, p in enumerate(pieces):
         te[:, C + i] = p
-    saved = dict(_CFG)
-    try:
-        _CFG["dtype"] = "tf32"
-        r = match_rows(None, qe, None, te, n, m, 0, want_topk=False, run_k3=False)
-    finally:
-        _CFG.update(saved)
-    # both candidates always: the tf32 product only PROPOSES them, their fp32 distances decide the order (so k = 1
-    # also returns the better of the two); a missing neighbour (m < k) is faiss's (-1, inf), never a wrapped index
-    idx = r.row_idx.long()
-    have = idx >= 0
-    d = ((q[:, None, :] - t[idx.clamp(min=0)]) ** 2).sum(dim=-1)
-    d = torch.where(have, d, torch.full_like(d, float("inf")))
-    swap = d[:, 1] < d[:, 0]
-    d = torch.where(swap[:, None], d.flip(1), d)
-    idx = torch.where(swap[:, None], idx.flip(1), idx)
-    return d[:, :k].contiguous().to(in_dev), idx[:, :k].contiguous().to(in_dev)
+    return qe, te
+
+
+_FUSED_K_MAX = 16  # longest row list of kernel 2's top-KP epilogue
+
+
+def _fused_knn_applies(n, m, k):
+    """whether k > 2 neighbours come from kernel 2's top-KP epilogue + the fp32 re-rank (else: _exact_knn_blocks)."""
+    return 3 <= k <= _FUSED_K_MAX and n >= 1 and m >= k
+
+
+def _topk_candidates(A, B, n, m, Ck, dtype, k):
+    """kernel 2 with the row top-KP epilogue on operand rows A (n, pitch) / B (m, pitch) over Ck columns: (n, KP) int32
+    candidate columns, best first.  KP = 8 for k <= 6, else 16: at least two spare candidates wherever the list allows."""
+    kp = 8 if k <= 6 else 16
+    dev = A.device
+    row_val = _empty((n, kp), torch.float32, dev)
+    row_idx = _empty((n, kp), torch.int32, dev)
+    ws_bytes = L.load().mv_k2_topk_workspace_bytes(n, m, kp)
+    ws = _empty((ws_bytes,), torch.uint8, dev)
+    L.call("mv_k2_sim_topk_ld", L.ptr(A), A.shape[1], L.ptr(B), B.shape[1], n, m, Ck, None, None, dtype, _CFG["cluster"], kp,
+           L.ptr(row_val), L.ptr(row_idx), L.ptr(ws), c_size_t(ws_bytes), _stream())
+    return row_idx
+
+
+def _rerank(Q, T, cand, k, metric):
+    """fp32 distances of every query's candidates (mv_knn_rerank): the k nearest, ascending, ties to the lower index."""
+    n, C = Q.shape
+    dist = _empty((n, k), torch.float32, Q.device)
+    idx = _empty((n, k), torch.int32, Q.device)
+    L.call("mv_knn_rerank", L.ptr(Q), Q.stride(0), L.ptr(T), T.stride(0), C, None, n, L.ptr(cand), cand.shape[1], k, metric,
+           L.ptr(dist), L.ptr(idx), _stream())
+    return dist, idx
 
 
 def _exact_knn_blocks(q, t, k):
-    """k > 2 neighbours (no call site in the reference asks for them): exact fp32 squared-L2 top-k on the device in
-    row blocks, ||q||^2 - 2 q.t + ||t||^2 like faiss's flat index.  Not the fused kernel -- kernel 2's epilogue
-    keeps two candidates per row -- but it keeps the interface complete without a CPU path."""
+    """exact fp32 squared-L2 top-k on the device in row blocks, ||q||^2 - 2 q.t + ||t||^2 like faiss's flat index: the
+    k > 2 searches kernel 2 does not serve (k > 16, targets with fewer than k rows) and the reference the fused path is
+    tested against."""
     k = min(k, t.shape[0])
     prev = torch.backends.cuda.matmul.allow_tf32
     torch.backends.cuda.matmul.allow_tf32 = False
@@ -424,12 +481,16 @@ def knn_points(X_f, Y_f, K=1, metric="euclidean"):
     cosine: rows are L2-normalised, neighbours come from kernel 2 and the distances 1 - cos are
     recomputed in fp32 by kernel 3, exactly the reference's order of operations (:47-58).
     euclidean: exact L2 neighbours through faiss_knn, distances = ||x - y||_2 (:55-56).
-    K > 2 (no call site in the reference) takes the exact blocked search of _exact_knn_blocks.
+    3 <= K <= 16 (no call site in the reference) runs on kernel 2's row top-KP epilogue wherever there are at least K
+    targets: euclidean through faiss_knn; cosine on the rows of the configured operand type (C % 8 == 0) with the fp32
+    re-rank of mv_knn_rerank for the distances.  Other K > 2 take the exact blocked search of _exact_knn_blocks.
     """
     assert metric in ["cosine", "euclidean"]
     dev = _device()
     in_dev = X_f.device
-    if K > 2:
+    n, m = X_f.shape[0], Y_f.shape[0]
+    fused = _fused_knn_applies(n, m, int(K)) and (metric == "euclidean" or X_f.shape[-1] % 8 == 0)
+    if K > 2 and not fused:
         X, Y = _f32(X_f, dev), _f32(Y_f, dev)
         if metric == "cosine":
             X, Y = torch.nn.functional.normalize(X, dim=-1), torch.nn.functional.normalize(Y, dim=-1)
@@ -449,6 +510,11 @@ def knn_points(X_f, Y_f, K=1, metric="euclidean"):
     if X_f.shape[0] == 0 or Y_f.shape[0] < K:
         raise ValueError(f"knn_points: {X_f.shape[0]} queries against {Y_f.shape[0]} targets for K={K}")
     (A16, A32), (B16, B32), mu = _rows_pair(X_f, Y_f, dev)
+    if K > 2:
+        A, B, Ck, dtype = _k2_operands(A16, A32, B16, B32, A32.shape[1])
+        cand = _topk_candidates(A, B, n, m, Ck, dtype, int(K))
+        d, idx = _rerank(A32, B32, cand, int(K), L.MV_METRIC_COSINE)
+        return d.to(in_dev), idx.long().to(in_dev)
     r = match_rows(A16, A32, B16, B32, X_f.shape[0], Y_f.shape[0], 0, want_topk=False, center_B=mu)
     return r.dists[:, :K].to(in_dev), r.row_idx[:, :K].long().to(in_dev)
 

@@ -27,6 +27,12 @@
 // Scheduling: the (super row block, column tile) list is cut into gridDim/MC equal contiguous ranges, so
 // every SM gets the same number of tiles (+-1); a row block that is split between CTAs leaves partial
 // top-2 records in the workspace which k2_merge_rows_kernel folds (ties: lower column).
+//
+// The same main loop also serves k > 2 nearest neighbours (k2_sim_topk_kernel, mv_k2_sim_topk_ld): its epilogue keeps
+// the KP (8 or 16) best columns of every row in registers -- a list sorted descending, updated by an unrolled
+// compare-and-shift -- and does no column work.  A chunk is only looked at when its maximum beats the list's last entry;
+// then its best column is inserted and knocked out until none beats it.  Partial lists go to the workspace like the
+// top-2 records and k2_merge_topk_kernel folds them into (n_max, KP) outputs.  Stream-K is never used there.
 #include <cuda.h>
 
 #include <stdlib.h>
@@ -66,6 +72,14 @@ constexpr int EPI_CW = 16;        // columns per TMEM read (chunk)
 constexpr int PART_COLS = BN / EPI_PARTS, PART_CHUNKS = PART_COLS / EPI_CW;
 constexpr int EPI_WARP0 = 4;
 constexpr int COL_SMEM_BYTES = 2 * 4 * BN * 8;  // [2 buffers][4 warps][256 columns] (max bits, ballot)
+// Epilogue shape of a kernel variant: KP == 0 is the top-2 + column arg-max epilogue above; KP > 0 the row top-KP one.
+template <int KP> struct Epi {
+  // a 16-entry list (32 registers) spills at the 96 registers of 20 warps: 12 warps, 168 registers
+  static constexpr int PARTS = KP == 16 ? 2 : EPI_PARTS;
+  static constexpr int THREADS = 32 * EPI_WARP0 + 128 * PARTS;
+  static constexpr int CHUNKS = BN / PARTS / EPI_CW;
+};
+static_assert(Epi<0>::THREADS == K2_THREADS, "the top-2 kernel keeps its 20 warps");
 template <bool PAIR> constexpr int k2_smem_bytes() { return 1024 /*align slack*/ + Ring<PAIR>::BYTES + COL_SMEM_BYTES + 256 /*barriers*/; }
 
 struct K2Sched {
@@ -138,6 +152,23 @@ __device__ __forceinline__ bool better(float x, int j, float y, int k) {
   return x > y || (x == y && (unsigned)j < (unsigned)k);
 }
 
+// Insert (x, j) into a list sorted descending, dropping its last entry.  Static indices only: the list stays in registers.
+// BY_INDEX = false compares values alone, for candidates that arrive in ascending column order (an equal value then
+// already sits in the list with a lower column); true breaks ties by the lower column (better()).
+template <int KP, bool BY_INDEX>
+__device__ __forceinline__ void list_insert(float (&lv)[KP], int (&li)[KP], float x, int j) {
+  bool up[KP];  // x goes above entry r
+#pragma unroll
+  for (int r = 0; r < KP; ++r) up[r] = BY_INDEX ? better(x, j, lv[r], li[r]) : x > lv[r];
+#pragma unroll
+  for (int r = KP - 1; r > 0; --r) {
+    lv[r] = up[r - 1] ? lv[r - 1] : (up[r] ? x : lv[r]);
+    li[r] = up[r - 1] ? li[r - 1] : (up[r] ? j : li[r]);
+  }
+  lv[0] = up[0] ? x : lv[0];
+  li[0] = up[0] ? j : li[0];
+}
+
 struct __align__(8) Barriers {
   unsigned long long full[MAX_STAGES];
   unsigned long long empty[MAX_STAGES];
@@ -149,10 +180,11 @@ struct __align__(8) Barriers {
 // MC: CTAs per cluster (consecutive row blocks of one super row block).  PAIR (MC == 2): the two CTAs form a
 // cta_group::2 pair -- ONE 256 x 256 MMA per k-step issued by the rank-0 CTA, each CTA supplying its 128 rows of
 // A and its 128 of the 256 columns of B and receiving its 128 rows of the accumulator in its own TMEM.
-template <bool TF32, int MC, bool PAIR>
-__global__ void __launch_bounds__(K2_THREADS, 1)
-    k2_sim_top2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, K2Params p) {
+// KP selects the epilogue (Epi<KP>); the producer, MMA issuer, TMEM allocation and schedule are shared.
+template <bool TF32, int MC, bool PAIR, int KP>
+__device__ __forceinline__ void k2_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const K2Params& p) {
   static_assert(!PAIR || MC == 2, "a CTA pair is a cluster of two");
+  static_assert(KP == 0 || KP == 8 || KP == 16, "row lists of 8 or 16 entries");
   constexpr int STAGES = Ring<PAIR>::STAGES;
   constexpr int STAGE_BYTES = Ring<PAIR>::STAGE_BYTES;
   extern __shared__ uint8_t smem_raw[];
@@ -169,7 +201,7 @@ __global__ void __launch_bounds__(K2_THREADS, 1)
   const int m = p.m_dev ? min(*p.m_dev, p.m_max) : p.m_max;
 
   // clusters beyond sch.G (fewer tiles than clusters) own nothing
-  const K2Sched sch = make_sched(n, m, MC, p.clusters, p.kblocks, p.streamk);
+  const K2Sched sch = make_sched(n, m, MC, p.clusters, p.kblocks, KP ? 0 : p.streamk);
   const bool has_work = cluster_id < sch.G && sch.T > 0;
   const unsigned long long u_beg = has_work ? sched_begin(sch, cluster_id) : 0ull;
   const unsigned long long u_end = has_work ? sched_begin(sch, cluster_id + 1) : 0ull;
@@ -223,7 +255,7 @@ __global__ void __launch_bounds__(K2_THREADS, 1)
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(smem_u32(&bars->tmem_full[a]), 1);
-      mbar_init(smem_u32(&bars->tmem_empty[a]), PAIR ? 8 * EPI_PARTS : 4 * EPI_PARTS);  // PAIR: the epilogue warps of BOTH CTAs (rank 0's barrier)
+      mbar_init(smem_u32(&bars->tmem_empty[a]), PAIR ? 8 * Epi<KP>::PARTS : 4 * Epi<KP>::PARTS);  // PAIR: the epilogue warps of BOTH CTAs (rank 0's barrier)
     }
     mbar_fence_init();
   }
@@ -317,6 +349,89 @@ __global__ void __launch_bounds__(K2_THREADS, 1)
       }
       acc ^= 1;
       if (acc == 0) acc_phase ^= 1u;
+    }
+  } else if (KP > 0 && warp >= EPI_WARP0) {
+    if constexpr (KP > 0) {
+      // ================================ top-KP epilogue (rows only) ================================
+      // same warp layout as the top-2 epilogue: Epi<KP>::PARTS warps per TMEM lane quarter, thread = one row of the tile
+      // and one column part.  Columns reach a thread in ascending order within a row block, so value comparisons alone
+      // keep ties on the lower column.
+      constexpr int PARTS = Epi<KP>::PARTS, CHUNKS = Epi<KP>::CHUNKS;
+      const int ew = warp & 3;
+      const int part = (warp - EPI_WARP0) >> 2;
+      const int e = ew * 32 + lane;
+      float lv[KP];
+      int li[KP];
+      int cur_sb = -1;
+      int acc = 0;
+      uint32_t acc_phase = 0;
+      auto flush = [&](int sb) {
+        float4* dst = p.partial + (((size_t)(cluster_id + sb) * (BM * MC) + rank * BM + e) * PARTS + part) * (KP / 2);
+#pragma unroll
+        for (int r = 0; r < KP / 2; ++r)
+          dst[r] = make_float4(lv[2 * r], __int_as_float(li[2 * r]), lv[2 * r + 1], __int_as_float(li[2 * r + 1]));
+      };
+      auto chunk_max = [](const float (&v)[EPI_CW]) {
+        float g[EPI_CW / 2];
+#pragma unroll
+        for (int q = 0; q < EPI_CW / 2; ++q) g[q] = fmaxf(v[2 * q], v[2 * q + 1]);
+#pragma unroll
+        for (int w = EPI_CW / 4; w > 0; w >>= 1)
+#pragma unroll
+          for (int q = 0; q < w; ++q) g[q] = fmaxf(g[q], g[q + w]);
+        return g[0];
+      };
+      for (unsigned long long step = 0; step < n_items; ++step) {
+        const unsigned long long t = item_at(step).t;
+        const int sb = (int)(t / (unsigned)sch.n_ct), ct = (int)(t - (unsigned long long)sb * sch.n_ct);
+        if (sb != cur_sb) {
+          if (cur_sb >= 0) flush(cur_sb);
+#pragma unroll
+          for (int r = 0; r < KP; ++r) {
+            lv[r] = -CUDART_INF_F;
+            li[r] = -1;
+          }
+          cur_sb = sb;
+        }
+        const int row0 = (sb * MC + rank) * BM, col0 = ct * BN;
+        const bool edge = (row0 + BM > n) || (col0 + BN > m);
+        const bool row_ok = row0 + e < n;
+
+        mbar_wait(smem_u32(&bars->tmem_full[acc]), acc_phase);
+        tc_fence_after();
+        const uint32_t taddr = tmem_base + (uint32_t)acc * BN + ((uint32_t)(ew * 32) << 16);
+#pragma unroll 1
+        for (int ch = part * CHUNKS; ch < (part + 1) * CHUNKS; ++ch) {
+          float v[EPI_CW];
+          tmem_ld_32x16(taddr + ch * EPI_CW, v);
+          const int cb = col0 + ch * EPI_CW;
+          if (edge) {
+#pragma unroll
+            for (int q = 0; q < EPI_CW; ++q) v[q] = (row_ok && cb + q < m) ? v[q] : -CUDART_INF_F;
+          }
+          // insert the chunk's best column (the lowest of equal ones) and knock it out, while it beats the last entry
+          float best = chunk_max(v);
+          while (best > lv[KP - 1]) {
+            int qb = 0;
+#pragma unroll
+            for (int q = EPI_CW - 1; q >= 0; --q) qb = v[q] == best ? q : qb;
+            list_insert<KP, false>(lv, li, best, cb + qb);
+#pragma unroll
+            for (int q = 0; q < EPI_CW; ++q) v[q] = q == qb ? -CUDART_INF_F : v[q];
+            best = chunk_max(v);
+          }
+          __syncwarp();  // the next tcgen05.ld is warp-collective
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) {
+          if (PAIR) mbar_arrive_cluster(map_to_cta(smem_u32(&bars->tmem_empty[acc]), 0));
+          else mbar_arrive(smem_u32(&bars->tmem_empty[acc]));
+        }
+        acc ^= 1;
+        if (acc == 0) acc_phase ^= 1u;
+      }
+      if (cur_sb >= 0) flush(cur_sb);
     }
   } else if (warp >= EPI_WARP0) {
     // ===================================== epilogue =========================================
@@ -517,6 +632,64 @@ __global__ void __launch_bounds__(K2_THREADS, 1)
   }
 }
 
+template <bool TF32, int MC, bool PAIR>
+__global__ void __launch_bounds__(K2_THREADS, 1)
+    k2_sim_top2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, K2Params p) {
+  k2_body<TF32, MC, PAIR, 0>(tmA, tmB, p);
+}
+
+template <bool TF32, int MC, bool PAIR, int KP>
+__global__ void __launch_bounds__(Epi<KP>::THREADS, 1)
+    k2_sim_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, K2Params p) {
+  k2_body<TF32, MC, PAIR, KP>(tmA, tmB, p);
+}
+
+// fold the partial top-KP lists of every row (Epi<KP>::PARTS column parts per CTA that worked on the row); write
+// (n_max, KP) values descending / indices, ties to the lower column, missing entries MV_MASKED_F / -1
+template <int MC, int KP>
+__global__ void k2_merge_topk_kernel(int clusters, const float4* __restrict__ partial, const int32_t* __restrict__ n_dev, int n_max,
+                                     const int32_t* __restrict__ m_dev, int m_max, float* __restrict__ row_val,
+                                     int32_t* __restrict__ row_idx) {
+  constexpr int PARTS = Epi<KP>::PARTS;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_max) return;
+  const int n = n_dev ? min(*n_dev, n_max) : n_max;
+  const int m = m_dev ? min(*m_dev, m_max) : m_max;
+  float lv[KP];
+  int li[KP];
+#pragma unroll
+  for (int r = 0; r < KP; ++r) {
+    lv[r] = -CUDART_INF_F;
+    li[r] = -1;
+  }
+  if (i < n && m > 0) {
+    const K2Sched s = make_sched(n, m, MC, clusters, 1, 0);
+    const int sb = i / (BM * MC);
+    const int c_first = sched_owner(s, (unsigned long long)sb * s.n_ct);
+    const int c_last = sched_owner(s, (unsigned long long)(sb + 1) * s.n_ct - 1);
+    for (int c = c_first; c <= c_last; ++c) {
+      for (int q = 0; q < PARTS; ++q) {
+        const float4* rec = partial + (((size_t)(c + sb) * (BM * MC) + (i - sb * BM * MC)) * PARTS + q) * (KP / 2);
+        // each partial list is sorted: stop at its first entry that does not make the list
+#pragma unroll 1
+        for (int h = 0; h < KP / 2; ++h) {
+          const float4 r = rec[h];
+          const int ja = __float_as_int(r.y), jb = __float_as_int(r.w);
+          if (ja < 0 || !better(r.x, ja, lv[KP - 1], li[KP - 1])) break;
+          list_insert<KP, true>(lv, li, r.x, ja);
+          if (jb < 0 || !better(r.z, jb, lv[KP - 1], li[KP - 1])) break;
+          list_insert<KP, true>(lv, li, r.z, jb);
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < KP; ++r) {
+    row_val[(size_t)KP * i + r] = li[r] >= 0 ? lv[r] : MV_MASKED_F;
+    row_idx[(size_t)KP * i + r] = li[r];
+  }
+}
+
 // fold the partial top-2 records of every row; write (n_max, 2) value / index pairs
 template <int MC>
 __global__ void k2_merge_rows_kernel(int clusters, int kblocks, int streamk, const float4* __restrict__ partial, const int32_t* __restrict__ n_dev,
@@ -637,18 +810,24 @@ int pick_mc(int cluster) { return cluster <= 1 ? 1 : (cluster >= 4 ? 4 : 2); }
 
 // persistent grid: one CTA per SM, but never more clusters than can be resident at once (GPC
 // boundaries strand SMs for cluster sizes that do not divide a GPC), or the grid runs in two waves
-template <bool TF32, int MC, bool PAIR = false>
+template <bool TF32, int MC, bool PAIR, int KP>
+constexpr auto k2_kernel() {
+  if constexpr (KP == 0) return k2_sim_top2_kernel<TF32, MC, PAIR>;
+  else return k2_sim_topk_kernel<TF32, MC, PAIR, KP>;
+}
+
+template <bool TF32, int MC, bool PAIR = false, int KP = 0>
 int k2_max_clusters() {
   static int cache[MV_MAX_DEVICES];
   int& cached = cache[mv_device_slot()];
   if (cached) return cached;
-  auto kern = k2_sim_top2_kernel<TF32, MC, PAIR>;
+  auto kern = k2_kernel<TF32, MC, PAIR, KP>();
   int n = mv_sm_count() / MC;
   constexpr int K2_SMEM_BYTES = k2_smem_bytes<PAIR>();
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_BYTES) == cudaSuccess && MC > 1) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(mv_sm_count() / MC * MC);
-    cfg.blockDim = dim3(K2_THREADS);
+    cfg.blockDim = dim3(Epi<KP>::THREADS);
     cfg.dynamicSmemBytes = K2_SMEM_BYTES;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -665,18 +844,19 @@ int k2_max_clusters() {
   return cached;
 }
 
+template <int KP = 0>
 int k2_grid(int mc, bool tf32, bool pair = false) {
   int clusters;
   if (mc == 1) clusters = mv_sm_count();
-  else if (pair) clusters = tf32 ? k2_max_clusters<true, 2, true>() : k2_max_clusters<false, 2, true>();
-  else if (mc == 2) clusters = tf32 ? k2_max_clusters<true, 2>() : k2_max_clusters<false, 2>();
-  else clusters = tf32 ? k2_max_clusters<true, 4>() : k2_max_clusters<false, 4>();
+  else if (pair) clusters = tf32 ? k2_max_clusters<true, 2, true, KP>() : k2_max_clusters<false, 2, true, KP>();
+  else if (mc == 2) clusters = tf32 ? k2_max_clusters<true, 2, false, KP>() : k2_max_clusters<false, 2, false, KP>();
+  else clusters = tf32 ? k2_max_clusters<true, 4, false, KP>() : k2_max_clusters<false, 4, false, KP>();
   return clusters * mc;
 }
 
-template <bool TF32, int MC, bool PAIR = false>
+template <bool TF32, int MC, bool PAIR = false, int KP = 0>
 int launch_k2(const CUtensorMap& tmA, const CUtensorMap& tmB, const K2Params& p, int grid, cudaStream_t st) {
-  auto kern = k2_sim_top2_kernel<TF32, MC, PAIR>;
+  auto kern = k2_kernel<TF32, MC, PAIR, KP>();
   constexpr int K2_SMEM_BYTES = k2_smem_bytes<PAIR>();
   static bool done[MV_MAX_DEVICES];
   bool& attr_done = done[mv_device_slot()];
@@ -686,7 +866,7 @@ int launch_k2(const CUtensorMap& tmA, const CUtensorMap& tmB, const K2Params& p,
   }
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(K2_THREADS);
+  cfg.blockDim = dim3(Epi<KP>::THREADS);
   cfg.dynamicSmemBytes = K2_SMEM_BYTES;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
@@ -700,6 +880,28 @@ int launch_k2(const CUtensorMap& tmA, const CUtensorMap& tmB, const K2Params& p,
   return MV_OK;
 }
 
+// the instantiation for an operand type and cluster form
+template <int KP>
+int launch_k2_form(bool tf32, int mc, bool pair, const CUtensorMap& tmA, const CUtensorMap& tmB, const K2Params& p, int grid,
+                   cudaStream_t st) {
+  if (pair) return tf32 ? launch_k2<true, 2, true, KP>(tmA, tmB, p, grid, st) : launch_k2<false, 2, true, KP>(tmA, tmB, p, grid, st);
+  if (tf32) {
+    if (mc == 1) return launch_k2<true, 1, false, KP>(tmA, tmB, p, grid, st);
+    if (mc == 2) return launch_k2<true, 2, false, KP>(tmA, tmB, p, grid, st);
+    return launch_k2<true, 4, false, KP>(tmA, tmB, p, grid, st);
+  }
+  if (mc == 1) return launch_k2<false, 1, false, KP>(tmA, tmB, p, grid, st);
+  if (mc == 2) return launch_k2<false, 2, false, KP>(tmA, tmB, p, grid, st);
+  return launch_k2<false, 4, false, KP>(tmA, tmB, p, grid, st);
+}
+
+// partial top-KP lists: (clusters + n_sb_max) slots of MC * 128 rows x Epi<KP>::PARTS column parts x KP (value, index) pairs
+size_t k2_topk_partial_bytes(int n_max, int mc, int clusters, int kp) {
+  const int n_sb_max = (n_max + BM * mc - 1) / (BM * mc);
+  const int parts = kp == 8 ? Epi<8>::PARTS : Epi<16>::PARTS;
+  return ((size_t)(clusters + n_sb_max) * (BM * mc) * parts * kp * sizeof(float2) + 255) / 256 * 256;
+}
+
 // ---- optional timing of the GEMM kernel alone (bench.py's roofline): events recorded right around the launch of
 // k2_sim_top2_kernel, so that the figure is the kernel's own duration and not memset + kernel + row merge
 struct K2Profile {
@@ -708,6 +910,79 @@ struct K2Profile {
   int capacity = 0, count = 0;
 };
 thread_local K2Profile g_k2_prof;
+
+// operand checks shared by the kernel-2 entry points; no CUDA call
+int k2_check_operands(const char* fn, int lda, int ldb, int n_max, int m_max, int C, int dtype, const void* A, const void* B,
+                      const void* workspace) {
+  MV_REQUIRE(lda >= C && ldb >= C && (lda * (dtype == MV_DTYPE_TF32 ? 4 : 2)) % 16 == 0 && (ldb * (dtype == MV_DTYPE_TF32 ? 4 : 2)) % 16 == 0,
+             MV_E_ALIGN, "%s: row pitches (%d, %d) must be >= C and a multiple of 16 bytes", fn, lda, ldb);
+  MV_REQUIRE(dtype == MV_DTYPE_BF16 || dtype == MV_DTYPE_TF32 || dtype == MV_DTYPE_F16, MV_E_ARG, "%s: unknown dtype %d", fn, dtype);
+  MV_REQUIRE(n_max > 0 && m_max > 0 && C > 0, MV_E_ARG, "%s: sizes must be positive", fn);
+  MV_REQUIRE(n_max <= (1 << 20) && m_max <= (1 << 20), MV_E_RANGE, "%s: at most 2^20 rows per side", fn);
+  const bool tf32 = dtype == MV_DTYPE_TF32;
+  MV_REQUIRE(C % (tf32 ? 4 : 8) == 0, MV_E_ALIGN, "%s: C=%d must be a multiple of %d", fn, C, tf32 ? 4 : 8);
+  MV_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)workspace & 15) == 0, MV_E_ALIGN,
+             "%s: A, B and workspace must be 16-byte aligned", fn);
+  return MV_OK;
+}
+
+// A launch of kernel 2 whose arguments passed k2_check_operands: device check, cluster form, grid and the parameters
+// every epilogue shares (the caller fills in the outputs and the workspace pointers)
+struct K2Launch {
+  K2Params p;
+  int grid, mc;
+  bool tf32, pair;
+};
+template <int KP>
+int k2_prepare(const char* fn, int n_max, int m_max, int C, const int32_t* n_dev, const int32_t* m_dev, int dtype, int cluster,
+               K2Launch& k) {
+  int dev = 0, cc = 0;
+  MV_CUDA(cudaGetDevice(&dev));
+  MV_CUDA(cudaDeviceGetAttribute(&cc, cudaDevAttrComputeCapabilityMajor, dev));
+  MV_REQUIRE(cc == 10, MV_E_ARCH, "%s: needs an sm_100 device (found compute capability %d.x)", fn, cc);
+  k.tf32 = dtype == MV_DTYPE_TF32;
+  if (cluster == MV_CLUSTER_AUTO) {
+    // measured on B200 (tools/k2_sweep.sh): once a tile's MMA time clearly exceeds its epilogue time (K >= 1536
+    // bf16 / 768 tf32 elements) the CTA pair wins (1612 vs 1520 TFLOP/s at 19200^2 x 2048); below that the
+    // epilogue co-limits and the looser coupling of two multicast CTAs is faster (1423 vs 1343 at K = 768)
+    cluster = (C >= (k.tf32 ? 768 : 1536)) ? MV_CLUSTER_PAIR : 2;
+  }
+  k.pair = cluster == MV_CLUSTER_PAIR;  // cta_group::2: two SMs on one 256 x 256 MMA tile
+  k.mc = k.pair ? 2 : pick_mc(cluster);
+  // (5.4 tiles per SM at the NAVI shape leave 10 % of the last tile-time idle; running two pairs' kernel 2 side by
+  // side on half the SMs each -- 10.8 tiles per SM -- was measured: same pairs/s, the pipeline's other kernels
+  // already fill that tail)
+  k.grid = k2_grid<KP>(k.mc, k.tf32, k.pair);
+  K2Params& p = k.p;
+  p = K2Params{};
+  p.clusters = k.grid / k.mc;
+  p.n_dev = n_dev;
+  p.m_dev = m_dev;
+  p.n_max = n_max;
+  p.m_max = m_max;
+  const int ke = k.tf32 ? 32 : 64;
+  p.kblocks = (C + ke - 1) / ke;
+  const int kstep = ke / 4;  // K elements per MMA: 16 (16-bit operands) / 8 (tf32)
+  p.tail_steps = (C - (p.kblocks - 1) * ke + kstep - 1) / kstep;
+  p.ab_fmt = k.tf32 ? 2u : (dtype == MV_DTYPE_F16 ? 0u : 1u);
+  return MV_OK;
+}
+
+int k2_operand_maps(CUtensorMap* tmA, CUtensorMap* tmB, const void* A, int lda, const void* B, int ldb, int n_max, int m_max,
+                    int C, int dtype, int mc) {
+  int rc = make_operand_map(tmA, A, n_max, C, lda, dtype, BM);
+  if (rc) return rc;
+  return make_operand_map(tmB, B, m_max, C, ldb, dtype, BN / mc);
+}
+
+size_t k2_topk_workspace_bytes(int n_max, int kp) {
+  size_t worst = 0;
+  for (int mc = 1; mc <= 4; mc *= 2) {
+    const size_t b = k2_topk_partial_bytes(n_max, mc, mv_sm_count() / mc, kp);
+    if (b > worst) worst = b;
+  }
+  return worst;
+}
 
 }  // namespace
 
@@ -780,47 +1055,16 @@ int mv_k2_affinity(const void* A, int lda, const void* B, int ldb, int n_max, in
   MV_REQUIRE(!S_out || (ld_s >= m_max && ld_s % 4 == 0 && ((uintptr_t)S_out & 15) == 0), MV_E_ALIGN,
              "mv_k2_affinity: S_out must be 16-byte aligned with a row pitch >= m_max that is a multiple of 4 floats");
   MV_REQUIRE(A && B && row_val && row_idx && col_best && workspace, MV_E_ARG, "mv_k2_sim_top2: null pointer");
-  MV_REQUIRE(lda >= C && ldb >= C && (lda * (dtype == MV_DTYPE_TF32 ? 4 : 2)) % 16 == 0 && (ldb * (dtype == MV_DTYPE_TF32 ? 4 : 2)) % 16 == 0,
-             MV_E_ALIGN, "mv_k2_sim_top2: row pitches (%d, %d) must be >= C and a multiple of 16 bytes", lda, ldb);
-  MV_REQUIRE(dtype == MV_DTYPE_BF16 || dtype == MV_DTYPE_TF32 || dtype == MV_DTYPE_F16, MV_E_ARG, "mv_k2_sim_top2: unknown dtype %d", dtype);
-  MV_REQUIRE(n_max > 0 && m_max > 0 && C > 0, MV_E_ARG, "mv_k2_sim_top2: sizes must be positive");
-  MV_REQUIRE(n_max <= (1 << 20) && m_max <= (1 << 20), MV_E_RANGE, "mv_k2_sim_top2: at most 2^20 rows per side");
-  const bool tf32 = dtype == MV_DTYPE_TF32;
-  MV_REQUIRE(C % (tf32 ? 4 : 8) == 0, MV_E_ALIGN, "mv_k2_sim_top2: C=%d must be a multiple of %d", C, tf32 ? 4 : 8);
-  MV_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)workspace & 15) == 0, MV_E_ALIGN,
-             "mv_k2_sim_top2: A, B and workspace must be 16-byte aligned");
-  int dev = 0, cc = 0;
-  MV_CUDA(cudaGetDevice(&dev));
-  MV_CUDA(cudaDeviceGetAttribute(&cc, cudaDevAttrComputeCapabilityMajor, dev));
-  MV_REQUIRE(cc == 10, MV_E_ARCH, "mv_k2_sim_top2: needs an sm_100 device (found compute capability %d.x)", cc);
-
-  if (cluster == MV_CLUSTER_AUTO) {
-    // measured on B200 (tools/k2_sweep.sh): once a tile's MMA time clearly exceeds its epilogue time (K >= 1536
-    // bf16 / 768 tf32 elements) the CTA pair wins (1612 vs 1520 TFLOP/s at 19200^2 x 2048); below that the
-    // epilogue co-limits and the looser coupling of two multicast CTAs is faster (1423 vs 1343 at K = 768)
-    cluster = (C >= (tf32 ? 768 : 1536)) ? MV_CLUSTER_PAIR : 2;
-  }
-  const bool pair = cluster == MV_CLUSTER_PAIR;  // cta_group::2: two SMs on one 256 x 256 MMA tile
-  const int mc = pair ? 2 : pick_mc(cluster);
-  // (5.4 tiles per SM at the NAVI shape leave 10 % of the last tile-time idle; running two pairs' kernel 2 side by
-  // side on half the SMs each -- 10.8 tiles per SM -- was measured: same pairs/s, the pipeline's other kernels
-  // already fill that tail)
-  const int grid = k2_grid(mc, tf32, pair);
-  K2Params p;
-  p.clusters = grid / mc;
-  const size_t part_bytes = k2_partial_bytes(n_max, mc, p.clusters);
-  const size_t need = part_bytes + k2_streamk_bytes(grid);
+  int rc = k2_check_operands("mv_k2_sim_top2", lda, ldb, n_max, m_max, C, dtype, A, B, workspace);
+  if (rc) return rc;
+  K2Launch k;
+  rc = k2_prepare<0>("mv_k2_sim_top2", n_max, m_max, C, n_dev, m_dev, dtype, cluster, k);
+  if (rc) return rc;
+  K2Params& p = k.p;
+  const size_t part_bytes = k2_partial_bytes(n_max, k.mc, p.clusters);
+  const size_t need = part_bytes + k2_streamk_bytes(k.grid);
   MV_REQUIRE(workspace_bytes >= need, MV_E_WORKSPACE, "mv_k2_sim_top2: workspace has %zu bytes, %zu needed",
              workspace_bytes, need);
-  p.n_dev = n_dev;
-  p.m_dev = m_dev;
-  p.n_max = n_max;
-  p.m_max = m_max;
-  const int ke = tf32 ? 32 : 64;
-  p.kblocks = (C + ke - 1) / ke;
-  const int kstep = ke / 4;  // K elements per MMA: 16 (16-bit operands) / 8 (tf32)
-  p.tail_steps = (C - (p.kblocks - 1) * ke + kstep - 1) / kstep;
-  p.ab_fmt = tf32 ? 2u : (dtype == MV_DTYPE_F16 ? 0u : 1u);
   p.partial = reinterpret_cast<float4*>(workspace);
   p.flags = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(workspace) + part_bytes);
   p.frag = reinterpret_cast<float4*>(reinterpret_cast<uint8_t*>(workspace) + part_bytes + SK_FLAG_BYTES);
@@ -830,9 +1074,7 @@ int mv_k2_affinity(const void* A, int lda, const void* B, int ldb, int n_max, in
   p.ld_s = ld_s;
 
   CUtensorMap tmA, tmB;
-  int rc = make_operand_map(&tmA, A, n_max, C, lda, dtype, BM);
-  if (rc) return rc;
-  rc = make_operand_map(&tmB, B, m_max, C, ldb, dtype, BN / mc);
+  rc = k2_operand_maps(&tmA, &tmB, A, lda, B, ldb, n_max, m_max, C, dtype, k.mc);
   if (rc) return rc;
 
   cudaStream_t st = mv_cuda_stream(stream);
@@ -841,17 +1083,7 @@ int mv_k2_affinity(const void* A, int lda, const void* B, int ldb, int n_max, in
   K2Profile& pr = g_k2_prof;
   const bool timed = pr.count < pr.capacity;
   if (timed) MV_CUDA(cudaEventRecord(pr.ev[2 * pr.count], st));
-  if (pair) {
-    rc = tf32 ? launch_k2<true, 2, true>(tmA, tmB, p, grid, st) : launch_k2<false, 2, true>(tmA, tmB, p, grid, st);
-  } else if (tf32) {
-    if (mc == 1) rc = launch_k2<true, 1>(tmA, tmB, p, grid, st);
-    else if (mc == 2) rc = launch_k2<true, 2>(tmA, tmB, p, grid, st);
-    else rc = launch_k2<true, 4>(tmA, tmB, p, grid, st);
-  } else {
-    if (mc == 1) rc = launch_k2<false, 1>(tmA, tmB, p, grid, st);
-    else if (mc == 2) rc = launch_k2<false, 2>(tmA, tmB, p, grid, st);
-    else rc = launch_k2<false, 4>(tmA, tmB, p, grid, st);
-  }
+  rc = launch_k2_form<0>(k.tf32, k.mc, k.pair, tmA, tmB, p, k.grid, st);
   if (rc) return rc;
   if (timed) {
     MV_CUDA(cudaEventRecord(pr.ev[2 * pr.count + 1], st));
@@ -861,9 +1093,57 @@ int mv_k2_affinity(const void* A, int lda, const void* B, int ldb, int n_max, in
     ++pr.count;
   }
   const int mt = 256;
+  const int mc = k.mc;
   if (mc == 1) k2_merge_rows_kernel<1><<<(n_max + mt - 1) / mt, mt, 0, st>>>(p.clusters, p.kblocks, p.streamk, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
   else if (mc == 2) k2_merge_rows_kernel<2><<<(n_max + mt - 1) / mt, mt, 0, st>>>(p.clusters, p.kblocks, p.streamk, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
   else k2_merge_rows_kernel<4><<<(n_max + mt - 1) / mt, mt, 0, st>>>(p.clusters, p.kblocks, p.streamk, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+  MV_LAUNCH_CHECK();
+  return MV_OK;
+}
+
+size_t mv_k2_topk_workspace_bytes(int n_max, int m_max, int kp) {
+  (void)m_max;
+  if (kp != 8 && kp != 16) return 0;
+  return k2_topk_workspace_bytes(n_max > 0 ? n_max : 1, kp);
+}
+
+int mv_k2_sim_topk_ld(const void* A, int lda, const void* B, int ldb, int n_max, int m_max, int C, const int32_t* n_dev,
+                      const int32_t* m_dev, int dtype, int cluster, int kp, float* row_val, int32_t* row_idx, void* workspace,
+                      size_t workspace_bytes, mv_stream_t stream) {
+  MV_REQUIRE(A && B && row_val && row_idx && workspace, MV_E_ARG, "mv_k2_sim_topk_ld: null pointer");
+  MV_REQUIRE(kp == 8 || kp == 16, MV_E_RANGE, "mv_k2_sim_topk_ld: kp=%d must be 8 or 16", kp);
+  int rc = k2_check_operands("mv_k2_sim_topk_ld", lda, ldb, n_max, m_max, C, dtype, A, B, workspace);
+  if (rc) return rc;
+  // the worst case over the cluster forms, so that the check needs no device
+  const size_t need = k2_topk_workspace_bytes(n_max, kp);
+  MV_REQUIRE(workspace_bytes >= need, MV_E_WORKSPACE, "mv_k2_sim_topk_ld: workspace has %zu bytes, %zu needed",
+             workspace_bytes, need);
+  K2Launch k;
+  rc = kp == 8 ? k2_prepare<8>("mv_k2_sim_topk_ld", n_max, m_max, C, n_dev, m_dev, dtype, cluster, k)
+               : k2_prepare<16>("mv_k2_sim_topk_ld", n_max, m_max, C, n_dev, m_dev, dtype, cluster, k);
+  if (rc) return rc;
+  K2Params& p = k.p;
+  p.partial = reinterpret_cast<float4*>(workspace);
+  p.streamk = 0;  // tile-granular schedule only: no head fragments, no flags
+
+  CUtensorMap tmA, tmB;
+  rc = k2_operand_maps(&tmA, &tmB, A, lda, B, ldb, n_max, m_max, C, dtype, k.mc);
+  if (rc) return rc;
+  cudaStream_t st = mv_cuda_stream(stream);
+  rc = kp == 8 ? launch_k2_form<8>(k.tf32, k.mc, k.pair, tmA, tmB, p, k.grid, st)
+               : launch_k2_form<16>(k.tf32, k.mc, k.pair, tmA, tmB, p, k.grid, st);
+  if (rc) return rc;
+  const int mt = 128, blocks = (n_max + mt - 1) / mt;
+  const int mc = k.mc;
+  if (kp == 8) {
+    if (mc == 1) k2_merge_topk_kernel<1, 8><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+    else if (mc == 2) k2_merge_topk_kernel<2, 8><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+    else k2_merge_topk_kernel<4, 8><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+  } else {
+    if (mc == 1) k2_merge_topk_kernel<1, 16><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+    else if (mc == 2) k2_merge_topk_kernel<2, 16><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+    else k2_merge_topk_kernel<4, 16><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+  }
   MV_LAUNCH_CHECK();
   return MV_OK;
 }
