@@ -405,6 +405,17 @@ int mv_spair_match_batch(const float* feats, int B, int C, int h, int w, const f
                          int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
                          unsigned long long* hits, unsigned long long* confusion, int conf_dim, mv_stream_t stream);
 
+/* mv_spair_match_batch on a map of any MV_FEAT_* element type: feats (B, 2, C, h, w) contiguous fp32, bf16 or fp16 (the
+ * output of an autocast backbone), read as it is -- a 16-bit map streams half the bytes and is widened on the chip.
+ * Widening is exact and the kernel keeps the fp32 form's channel chunks and summation order, so the outputs are BIT-
+ * IDENTICAL to mv_spair_match_batch on the map widened to fp32, in either heat-map precision.  feat_dtype = MV_FEAT_F32
+ * is mv_spair_match_batch.  Errors, checked before any CUDA call: an unknown feat_dtype (MV_E_ARG), feats not aligned to
+ * its element size (MV_E_ALIGN), and those of mv_spair_match_batch. */
+int mv_spair_match_batch_typed(const void* feats, int feat_dtype, int B, int C, int h, int w, const float* kps_i,
+                               const float* kps_j, int K, int kp_stride, const float* thresh_scale, float image_size,
+                               float pck_thresh, int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
+                               unsigned long long* hits, unsigned long long* confusion, int conf_dim, mv_stream_t stream);
+
 /* Precision of the batched kernel's heat map (the einsum of evaluate_spair_correspondence.py:82) on the tensor cores:
  * 3 (default) = every product as three tf32 MMAs (hi*hi + hi*lo + lo*hi, ~21 mantissa bits: the arg-max equals the fp32
  * reference's wherever the top-2 heat-map gap exceeds 1e-5); 1 = one tf32 MMA, operands rounded to 10 mantissa bits with

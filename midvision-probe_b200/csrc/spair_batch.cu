@@ -2,7 +2,9 @@
 //
 //   mv_spair_match_batch   per pair: bilinear key-point features of the normalised map, K x (h*w) heat map with
 //                          the per-pixel normalisation folded in, arg-max, key-point error matrix, PCK counts
-//                          -- one CTA per pair, fp32 throughout
+//                          -- one CTA per pair, fp32 arithmetic throughout
+//   mv_spair_match_batch_typed   the same on an fp32, bf16 or fp16 map: 16-bit maps are read as they are and widened
+//                          on the chip, with the fp32 results of the widened map bit for bit
 //
 // Reference behaviour being reproduced (file:line in /root/reference):
 //   evaluate_spair_correspondence.py:59     feats = F.normalize(feats, p=2, dim=1)
@@ -20,6 +22,9 @@
 #include <math_constants.h>
 #include <stdlib.h>
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include <type_traits>
 
 #include "common.cuh"
@@ -32,8 +37,21 @@ constexpr int SPB_THREADS = 256;
 constexpr int SPB_MAX_HW = 1 << 20;  // pixels per feature map (2500 at the reference's 800 x 800 input)
 constexpr float SPB_NORM_EPS = 1e-12f;  // F.normalize default eps
 
+// element type T of the maps: float, or the __nv_bfloat16 / __half output of an autocast backbone.  Every 16-bit value is
+// an fp32 value (widening is exact), and every one is also exactly a tf32 value (8 / 11 significant bits, fp32's exponent
+// range): the kernels widen on load from global or shared memory and then run the fp32 arithmetic unchanged.
+__device__ __forceinline__ float sp_f32(float v) { return v; }
+__device__ __forceinline__ float sp_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float sp_f32(__half v) { return __half2float(v); }
+// two neighbouring values, one 8-byte (float) or 4-byte (16-bit) aligned load
+__device__ __forceinline__ float2 sp_f32x2(const float* v) { return *reinterpret_cast<const float2*>(v); }
+__device__ __forceinline__ float2 sp_f32x2(const __nv_bfloat16* v) {
+  return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(v));
+}
+__device__ __forceinline__ float2 sp_f32x2(const __half* v) { return __half22float2(*reinterpret_cast<const __half2*>(v)); }
+
 struct SpairBatchParams {
-  const float* feats;  // (B, 2, C, h, w)
+  const void* feats;  // (B, 2, C, h, w) of the launch's element type
   const float* kps_i;  // (B, K, stride)
   const float* kps_j;
   const float* thresh_scale;  // (B)
@@ -52,7 +70,7 @@ struct SpairBatchParams {
 // dynamic shared memory: q[C][KT], the key-point features of the current tile
 // blockDim.x = min(SPB_THREADS, h*w rounded up to a warp): thread = pixel in the heat-map pass, so a 14 x 14 map
 // runs 7 warps with 87 % of the lanes busy instead of 8 warps with 77 %.
-template <int KT>
+template <typename T, int KT>
 __global__ void __launch_bounds__(SPB_THREADS) spair_batch_kernel(SpairBatchParams p) {
   extern __shared__ float4 spb_dyn[];
   __shared__ SpairScoreShared score;
@@ -68,8 +86,8 @@ __global__ void __launch_bounds__(SPB_THREADS) spair_batch_kernel(SpairBatchPara
   const int nthr = blockDim.x, nwarp = nthr >> 5;
 
   for (int b = blockIdx.x; b < p.B; b += gridDim.x) {
-    const float* fi = p.feats + (size_t)b * 2 * C * hw;
-    const float* fj = fi + (size_t)C * hw;
+    const T* fi = static_cast<const T*>(p.feats) + (size_t)b * 2 * C * hw;
+    const T* fj = fi + (size_t)C * hw;
     const float* ki = p.kps_i + (size_t)b * K * p.stride;
     const float* kj = p.kps_j + (size_t)b * K * p.stride;
 
@@ -100,11 +118,11 @@ __global__ void __launch_bounds__(SPB_THREADS) spair_batch_kernel(SpairBatchPara
       const int slices = max(1, nthr / ntap);
       for (int item = tid; item < ntap * slices; item += nthr) {
         const int tp = item % ntap, sl = item / ntap;
-        const float* src = fi + s_tap[tp >> 2][tp & 3];
+        const T* src = fi + s_tap[tp >> 2][tp & 3];
         float ss = 0.f;
 #pragma unroll 16
         for (int c = sl; c < C; c += slices) {
-          const float v = __ldg(src + (size_t)c * hw);
+          const float v = sp_f32(__ldg(src + (size_t)c * hw));
           ss = fmaf(v, v, ss);
         }
         atomicAdd(&s_ss[tp >> 2][tp & 3], ss);
@@ -124,11 +142,11 @@ __global__ void __launch_bounds__(SPB_THREADS) spair_batch_kernel(SpairBatchPara
       for (int idx = tid; idx < C * KT; idx += nthr) {
         const int c = idx / KT, k = idx - c * KT;
         const int kk = k0 + min(k, kt - 1);
-        const float* src = fi + (size_t)c * hw;
-        float acc = __ldg(src + s_tap[kk][0]) * s_wt[kk][0];
-        acc = fmaf(__ldg(src + s_tap[kk][1]), s_wt[kk][1], acc);
-        acc = fmaf(__ldg(src + s_tap[kk][2]), s_wt[kk][2], acc);
-        acc = fmaf(__ldg(src + s_tap[kk][3]), s_wt[kk][3], acc);
+        const T* src = fi + (size_t)c * hw;
+        float acc = sp_f32(__ldg(src + s_tap[kk][0])) * s_wt[kk][0];
+        acc = fmaf(sp_f32(__ldg(src + s_tap[kk][1])), s_wt[kk][1], acc);
+        acc = fmaf(sp_f32(__ldg(src + s_tap[kk][2])), s_wt[kk][2], acc);
+        acc = fmaf(sp_f32(__ldg(src + s_tap[kk][3])), s_wt[kk][3], acc);
         q[idx] = (k < kt) ? acc : 0.f;
       }
       __syncthreads();
@@ -147,12 +165,12 @@ __global__ void __launch_bounds__(SPB_THREADS) spair_batch_kernel(SpairBatchPara
 #pragma unroll
         for (int k = 0; k < KT; ++k) acc[k] = 0.f;
         float ss = 0.f;
-        const float* col = fj + px;
+        const T* col = fj + px;
         int c0 = 0;
         for (; c0 + 16 <= C; c0 += 16) {
           float v[16];
 #pragma unroll
-          for (int u = 0; u < 16; ++u) v[u] = __ldg(col + (size_t)(c0 + u) * hw);  // 16 loads in flight
+          for (int u = 0; u < 16; ++u) v[u] = sp_f32(__ldg(col + (size_t)(c0 + u) * hw));  // 16 loads in flight
 #pragma unroll
           for (int u = 0; u < 16; ++u) {
             ss = fmaf(v[u], v[u], ss);
@@ -168,7 +186,7 @@ __global__ void __launch_bounds__(SPB_THREADS) spair_batch_kernel(SpairBatchPara
           }
         }
         for (; c0 < C; ++c0) {
-          const float v = __ldg(col + (size_t)c0 * hw);
+          const float v = sp_f32(__ldg(col + (size_t)c0 * hw));
           ss = fmaf(v, v, ss);
 #pragma unroll
           for (int k = 0; k < KT; ++k) acc[k] = fmaf(q[(size_t)c0 * KT + k], v, acc[k]);
@@ -325,7 +343,12 @@ constexpr int sps_q_floats(int cc) {  // one q buffer
 // TERMS: 3 = 3xTF32 (fp32-grade heat map, the default), 1 = one tf32 MMA per tile (mv_spair_set_heatmap_terms(1): operands
 // rounded to 10 mantissa bits, the north star's "tf32 inputs, fp32 accumulation" -- arg-max equal wherever the fp32 top-2 gap
 // of the heat map exceeds 1e-3)
-template <int KT, bool MMA, int TERMS = 3>
+// T = __nv_bfloat16 / __half: the slots hold the 16-bit rows as they are in global memory (half the bytes of a slot, twice
+// the ring stages), and pass N, step Q and step H widen what they read.  The channel chunks, their order and each thread's
+// channel order are those of T = float, so every fp32 sum is the same sum: the outputs are those of the fp32 kernel on the
+// widened map, bit for bit.  Step H's A operand (the map value) is exactly a tf32 value, its 3xTF32 low half zero: the
+// lo * hi MMA, whose products are all zero, and the A split are skipped.
+template <typename T, int KT, bool MMA, int TERMS = 3>
 __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(SpairBatchParams p) {
   using namespace sm100;
   extern __shared__ __align__(16) float4 sps_dyn[];
@@ -336,12 +359,13 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
   __shared__ int s_bi[SPS_WARPS][KT];
   __shared__ __align__(8) unsigned long long full[SPS_MAX_STAGES], empty[SPS_MAX_STAGES];
   constexpr bool REV = SPS_QREV && MMA;  // the CUDA-core form keeps the channel order (and the bits) of the first form
+  constexpr bool F32 = std::is_same<T, float>::value;
   const int C = p.C, hw = p.h * p.w, K = p.K, rs = hw;
   constexpr int cc = SPS_CC;
   const int nstage = p.stages;
-  const int slot_floats = 2 * cc * rs;
-  float* ring = reinterpret_cast<float*>(sps_dyn);                  // [stages][2 * cc rows][rs]
-  float* qbuf = ring + (size_t)nstage * slot_floats;                // [2][cc][KT]
+  const int slot_elems = 2 * cc * rs;  // a multiple of 8: slots and the q buffers after them stay 16-byte aligned
+  T* ring = reinterpret_cast<T*>(sps_dyn);                          // [stages][2 * cc rows][rs]
+  float* qbuf = reinterpret_cast<float*>(ring + (size_t)nstage * slot_elems);  // [2][cc][KT]
   float* pix_ss = qbuf + 2 * sps_q_floats<KT, MMA>(cc);             // [hw]
   float* score_mem = pix_ss + ((hw + 3) & ~3);                      // [K][K + 1] errors, 2 counters
   const SpairScoreView score{score_mem, K + 1, reinterpret_cast<unsigned int*>(score_mem + K * (K + 1))};
@@ -368,18 +392,19 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
     const uint64_t pol_keep = SPS_HINTS == 1 ? L2_EVICT_LAST : L2_EVICT_NORMAL;
     const uint64_t pol_stream = SPS_HINTS ? L2_EVICT_FIRST : L2_EVICT_NORMAL;
     // rows [c0, c0 + rows) of one map into a slot at float offset `at`
-    auto rows_in = [&](const float* map, int c0, int rows, int at, uint64_t pol) {
-      bulk_load_1d_hint(smem_u32(ring + (size_t)stage * slot_floats + at), map + (size_t)c0 * hw, (uint32_t)(rows * hw) * 4u,
-                        smem_u32(&full[stage]), pol);
+    // (rows * hw * sizeof(T) bytes: a multiple of 16 for every chunk, the tail included, as C and cc are multiples of 8)
+    auto rows_in = [&](const T* map, int c0, int rows, int at, uint64_t pol) {
+      bulk_load_1d_hint(smem_u32(ring + (size_t)stage * slot_elems + at), map + (size_t)c0 * hw,
+                        (uint32_t)(rows * hw) * (uint32_t)sizeof(T), smem_u32(&full[stage]), pol);
     };
     if (lane != 0) return;
     for (int b = blockIdx.x; b < p.B; b += gridDim.x) {
-      const float* fi = p.feats + (size_t)b * 2 * C * hw;
-      const float* fj = fi + (size_t)C * hw;
+      const T* fi = static_cast<const T*>(p.feats) + (size_t)b * 2 * C * hw;
+      const T* fj = fi + (size_t)C * hw;
       for (int c0 = 0; c0 < C; c0 += 2 * cc) {  // pass N
         const int rows = min(2 * cc, C - c0);
         mbar_wait(smem_u32(&empty[stage]), phase ^ 1u);
-        mbar_arrive_expect_tx(smem_u32(&full[stage]), (uint32_t)(rows * hw) * 4u);
+        mbar_arrive_expect_tx(smem_u32(&full[stage]), (uint32_t)(rows * hw) * (uint32_t)sizeof(T));
         rows_in(fi, c0, rows, 0, pol_keep);
         if (++stage == nstage) { stage = 0; phase ^= 1u; }
       }
@@ -388,7 +413,7 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
         for (int cq = 0; cq < nchunk; ++cq) {
           const int c0 = (REV ? nchunk - 1 - cq : cq) * cc, rows = min(cc, C - c0);
           mbar_wait(smem_u32(&empty[stage]), phase ^ 1u);
-          mbar_arrive_expect_tx(smem_u32(&full[stage]), (uint32_t)(2 * rows * hw) * 4u);
+          mbar_arrive_expect_tx(smem_u32(&full[stage]), (uint32_t)(2 * rows * hw) * (uint32_t)sizeof(T));
           rows_in(fi, c0, rows, 0, pol_i);
           rows_in(fj, c0, rows, cc * rs, pol_j);
           if (++stage == nstage) { stage = 0; phase ^= 1u; }
@@ -442,14 +467,14 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
           float* qb = qbuf + (g_chunk & 1) * QF;
           mbar_wait(smem_u32(&full[stage]), phase);
           if (g_chunk >= 2) bar_sync(5 + (g_chunk & 1), SPS_QH);
-          const float* sti = ring + (size_t)stage * slot_floats;
+          const T* sti = ring + (size_t)stage * slot_elems;
           if (q_on) {
             for (int c = cg; c < rows; c += G) {
-              const float* src = sti + c * rs;
-              float a = src[tap[0]] * wq[0];
-              a = fmaf(src[tap[1]], wq[1], a);
-              a = fmaf(src[tap[2]], wq[2], a);
-              a = fmaf(src[tap[3]], wq[3], a);
+              const T* src = sti + c * rs;
+              float a = sp_f32(src[tap[0]]) * wq[0];
+              a = fmaf(sp_f32(src[tap[1]]), wq[1], a);
+              a = fmaf(sp_f32(src[tap[2]]), wq[2], a);
+              a = fmaf(sp_f32(src[tap[3]]), wq[3], a);
               a = (k < kt) ? a : 0.f;
               if constexpr (MMA) {
                 uint32_t hi, lo;
@@ -506,12 +531,12 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
       for (int c0 = 0; c0 < C; c0 += 2 * cc) {
         const int rows = min(2 * cc, C - c0);
         mbar_wait(smem_u32(&full[stage]), phase);
-        const float* st = ring + (size_t)stage * slot_floats + px;
+        const T* st = ring + (size_t)stage * slot_elems + px;
         if (has_px && SPS_NULL != 1) {
           for (int c = 0; c < rows; c += 8) {
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
-              const float v = st[(c + u) * rs];
+              const float v = sp_f32(st[(c + u) * rs]);
               ss = fmaf(v, v, ss);
             }
           }
@@ -556,17 +581,17 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
         const int c0 = (REV ? nchunk - 1 - cq : cq) * cc, rows = min(cc, C - c0);
         float* qb = qbuf + ((SPS_QW > 0 ? g_chunk : (unsigned)cq) & 1) * QF;
         mbar_wait(smem_u32(&full[stage]), phase);
-        const float* sti = ring + (size_t)stage * slot_floats;
-        const float* stj = sti + cc * rs;
+        const T* sti = ring + (size_t)stage * slot_elems;
+        const T* stj = sti + cc * rs;
         // ---- step Q: q[c][k] = sum_t wt * f_i[c][tap] / max(||f_i[tap]||, eps): the grid_sample of the normalised map ----
         for (int idx = tid; idx < rows * KT && SPS_NULL != 1 && SPS_NULL != 3 && SPS_QW == 0; idx += SPS_CONS) {
           const int c = idx / KT, k = idx - c * KT;
           const int kk = k0 + min(k, kt - 1);
-          const float* src = sti + c * rs;
-          float a = src[s_tap[kk][0]] * s_wt[kk][0];
-          a = fmaf(src[s_tap[kk][1]], s_wt[kk][1], a);
-          a = fmaf(src[s_tap[kk][2]], s_wt[kk][2], a);
-          a = fmaf(src[s_tap[kk][3]], s_wt[kk][3], a);
+          const T* src = sti + c * rs;
+          float a = sp_f32(src[s_tap[kk][0]]) * s_wt[kk][0];
+          a = fmaf(sp_f32(src[s_tap[kk][1]]), s_wt[kk][1], a);
+          a = fmaf(sp_f32(src[s_tap[kk][2]]), s_wt[kk][2], a);
+          a = fmaf(sp_f32(src[s_tap[kk][3]]), s_wt[kk][3], a);
           a = (k < kt) ? a : 0.f;
           if constexpr (MMA) {
             uint32_t hi, lo;
@@ -583,7 +608,7 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
         // ---- step H: heat[k][px] += sum_c q[c][k] * f_j[c][px], the pixel's norm accumulated alongside ----
         if constexpr (MMA) {
           if (warp_live && SPS_NULL != 1 && SPS_NULL != 2) {
-            const float* aj = stj + 32 * wid + 2 * g;
+            const T* aj = stj + 32 * wid + 2 * g;
             const float4* bq = reinterpret_cast<const float4*>(qb) + lane;
             // the two run-time facts of a K step -- 8-byte loads possible, second tile live -- are dispatched once per chunk, so
             // that the K steps themselves are branch-free and the scheduler can lift the next step's loads above this step's MMAs
@@ -602,18 +627,20 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
               }
               // A fragments: pixels 16 i + 2 g, + 1 (fragment rows g, g + 8 of tile i) of channels t and t + 4, each pair one
               // LDS.64 straight into its half of the operand's register quad (the tensor core ignores the low mantissa bits, so
-              // the loaded values ARE the hi operand).  Pixels beyond h*w read whatever follows in the slot (finite or not:
-              // their rows are never looked at).
-              const float* r0 = aj + (ks + t) * rs;
-              const float* r1 = r0 + 4 * rs;
+              // the loaded values ARE the hi operand).  16-bit rows: each pair one 32-bit load, widened in registers; with an
+              // odd h*w every other row starts at an odd element, and all four values are single 16-bit loads.  Pixels beyond
+              // h*w read whatever follows in the slot (finite or not: their rows are never looked at).
+              const T* r0 = aj + (ks + t) * rs;
+              const T* r1 = r0 + 4 * rs;
               float av[2][4];
 #pragma unroll
               for (int i = 0; i < NTILE; ++i) {  // NTILE == 1: the warp's second 16 pixels lie beyond the map
                 if constexpr (VEC2) {
-                  const float2 x0 = *reinterpret_cast<const float2*>(r0 + 16 * i), x1 = *reinterpret_cast<const float2*>(r1 + 16 * i);
+                  const float2 x0 = sp_f32x2(r0 + 16 * i), x1 = sp_f32x2(r1 + 16 * i);
                   av[i][0] = x0.x, av[i][1] = x0.y, av[i][2] = x1.x, av[i][3] = x1.y;
                 } else {
-                  av[i][0] = r0[16 * i], av[i][1] = r0[16 * i + 1], av[i][2] = r1[16 * i], av[i][3] = r1[16 * i + 1];
+                  av[i][0] = sp_f32(r0[16 * i]), av[i][1] = sp_f32(r0[16 * i + 1]);
+                  av[i][2] = sp_f32(r1[16 * i]), av[i][3] = sp_f32(r1[16 * i + 1]);
                 }
               }
 #pragma unroll
@@ -624,10 +651,13 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
                 ssr[i][1] = fmaf(av[i][3], av[i][3], ssr[i][1]);
                 uint32_t ah[4], al[4];
 #pragma unroll
-                for (int e = 0; e < 4; ++e) split_tf32(av[i][e], ah[e], al[e]);
+                for (int e = 0; e < 4; ++e) {
+                  if constexpr (F32) split_tf32(av[i][e], ah[e], al[e]);
+                  else ah[e] = __float_as_uint(av[i][e]);  // a widened 16-bit value is its own hi half; lo = 0
+                }
 #pragma unroll
                 for (int j = 0; j < NT8; ++j) {
-                  if (SPS_NULL != 4 && SPS_NULL != 5 && TERMS == 3) mma_tf32(d[i][j], al, bh[j][0], bh[j][1]);
+                  if (SPS_NULL != 4 && SPS_NULL != 5 && TERMS == 3 && F32) mma_tf32(d[i][j], al, bh[j][0], bh[j][1]);
                   if (SPS_NULL != 4 && SPS_NULL != 5 && TERMS == 3) mma_tf32(d[i][j], ah, bl[j][0], bl[j][1]);
                   if (SPS_NULL != 5) mma_tf32(d[i][j], ah, bh[j][0], bh[j][1]);
                 }
@@ -640,21 +670,21 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
               for (int ks = 0; ks < rows; ks += 8) kstep(ks);
             }
             };
-            using T = std::true_type;
-            using F = std::false_type;
+            using Y = std::true_type;
+            using N = std::false_type;
             if (vec2) {
-              if (tile1_live) h_chunk(T{}, T{});
-              else h_chunk(T{}, F{});
+              if (tile1_live) h_chunk(Y{}, Y{});
+              else h_chunk(Y{}, N{});
             } else {
-              if (tile1_live) h_chunk(F{}, T{});
-              else h_chunk(F{}, F{});
+              if (tile1_live) h_chunk(N{}, Y{});
+              else h_chunk(N{}, N{});
             }
           }
         } else {
           if (has_px) {
-            const float* sj = stj + px;
+            const T* sj = stj + px;
             for (int c = 0; c < rows; ++c) {
-              const float v = sj[c * rs];
+              const float v = sp_f32(sj[c * rs]);
               ssp = fmaf(v, v, ssp);
               const float4* qc = reinterpret_cast<const float4*>(qb + c * KT);
 #pragma unroll
@@ -780,7 +810,7 @@ struct SpsPlan {
   size_t smem;
   bool ok;
 };
-SpsPlan sps_plan(const SpairBatchParams& p, int KT) {
+SpsPlan sps_plan(const SpairBatchParams& p, int KT, size_t elem) {
   SpsPlan pl{};
   const int hw = p.h * p.w;
   static const int off = getenv("MVMATCH_SPAIR_STREAM") && getenv("MVMATCH_SPAIR_STREAM")[0] == '0';
@@ -790,7 +820,7 @@ SpsPlan sps_plan(const SpairBatchParams& p, int KT) {
   const int cc = SPS_CC, rs = hw;
   const size_t qf = mma ? (size_t)(cc / 8) * ((KT + 7) / 8) * 128 : (size_t)cc * KT;
   const size_t fixed = (2 * qf + (size_t)((hw + 3) & ~3) + (size_t)((p.K * (p.K + 1) + 2 + 3) & ~3)) * sizeof(float);
-  const size_t slot = (size_t)2 * cc * rs * sizeof(float);
+  const size_t slot = (size_t)2 * cc * rs * elem;  // 16-bit maps: half the bytes, twice the stages (5 against 2 at 14 x 14)
   // SPS_CTAS CTAs per SM: 227 KB less 1 KB reserved and ~4 KB of static shared memory per CTA
   const size_t budget = ((227u << 10) / SPS_CTAS) - (5u << 10);
   int stages = env_stages > 0 ? env_stages : (fixed + 2 * slot <= budget ? (int)((budget - fixed) / slot) : 2);
@@ -804,12 +834,13 @@ SpsPlan sps_plan(const SpairBatchParams& p, int KT) {
   return pl;
 }
 
-template <int KT>
+template <typename T, int KT>
 int launch_spair_stream(const SpairBatchParams& p, const SpsPlan& pl, cudaStream_t st) {
   // MVMATCH_SPAIR_MMA=0: the heat-map step on the CUDA cores (the arithmetic of the first form)
   static const bool mma = !(getenv("MVMATCH_SPAIR_MMA") && getenv("MVMATCH_SPAIR_MMA")[0] == '0');
   const bool one_term = mma && g_spair_terms == 1;
-  auto kern = !mma ? spair_stream_kernel<KT, false> : one_term ? spair_stream_kernel<KT, true, 1> : spair_stream_kernel<KT, true, 3>;
+  auto kern = !mma ? spair_stream_kernel<T, KT, false>
+                   : one_term ? spair_stream_kernel<T, KT, true, 1> : spair_stream_kernel<T, KT, true, 3>;
   static size_t opted[MV_MAX_DEVICES][3];
   size_t& opted_in = opted[mv_device_slot()][!mma ? 0 : one_term ? 2 : 1];
   if (pl.smem > opted_in) {
@@ -834,12 +865,12 @@ int launch_spair_stream(const SpairBatchParams& p, const SpsPlan& pl, cudaStream
   return MV_OK;
 }
 
-template <int KT>
+template <typename T, int KT>
 int launch_spair_batch(const SpairBatchParams& p, cudaStream_t st) {
-  const SpsPlan pl = sps_plan(p, KT);
-  if (pl.ok) return launch_spair_stream<KT>(p, pl, st);
+  const SpsPlan pl = sps_plan(p, KT, sizeof(T));
+  if (pl.ok) return launch_spair_stream<T, KT>(p, pl, st);
   const size_t smem = (size_t)p.C * KT * sizeof(float);
-  auto kern = spair_batch_kernel<KT>;
+  auto kern = spair_batch_kernel<T, KT>;
   static size_t opted[MV_MAX_DEVICES];  // per device; static + dynamic shared memory above 48 KB needs the opt-in
   size_t& opted_in = opted[mv_device_slot()];
   if (opted_in < (24u << 10)) opted_in = 24 << 10;
@@ -864,22 +895,38 @@ int launch_spair_batch(const SpairBatchParams& p, cudaStream_t st) {
   return MV_OK;
 }
 
-}  // namespace
+// key-point tile = accumulators per thread; the first form's tile features (C * KT floats) must fit shared memory
+template <typename T>
+int launch_spair_tiles(const SpairBatchParams& p, cudaStream_t st) {
+  const size_t budget = 160u << 10;
+  const size_t per_k = (size_t)p.C * sizeof(float);
+  const int K = p.K;
+  if (K > 24 && 32 * per_k <= budget) return launch_spair_batch<T, 32>(p, st);
+  if (K > 20 && 24 * per_k <= budget) return launch_spair_batch<T, 24>(p, st);
+  if (K > 16 && 20 * per_k <= budget) return launch_spair_batch<T, 20>(p, st);  // SPair-71k: up to 20 key points for most classes
+  if (K > 12 && 16 * per_k <= budget) return launch_spair_batch<T, 16>(p, st);
+  if (K > 8 && 12 * per_k <= budget) return launch_spair_batch<T, 12>(p, st);
+  return launch_spair_batch<T, 8>(p, st);
+}
 
-extern "C" {
-
-int mv_spair_match_batch(const float* feats, int B, int C, int h, int w, const float* kps_i, const float* kps_j, int K,
-                         int kp_stride, const float* thresh_scale, float image_size, float pck_thresh,
-                         int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
-                         unsigned long long* hits, unsigned long long* confusion, int conf_dim, mv_stream_t stream) {
-  MV_REQUIRE(B >= 0 && C > 0 && h > 0 && w > 0, MV_E_ARG, "mv_spair_match_batch: bad sizes");
-  MV_REQUIRE((B == 0 || K == 0) || (feats && kps_i && kps_j && thresh_scale), MV_E_ARG,
-             "mv_spair_match_batch: null pointer");
-  MV_REQUIRE(h * w <= SPB_MAX_HW, MV_E_RANGE, "mv_spair_match_batch: h*w=%d exceeds %d pixels", h * w, SPB_MAX_HW);
-  MV_REQUIRE(K >= 0 && K <= 64, MV_E_RANGE, "mv_spair_match_batch: K=%d must be in [0, 64]", K);
-  MV_REQUIRE(kp_stride >= 3 && image_size > 0.f, MV_E_ARG, "mv_spair_match_batch: bad key-point layout");
-  MV_REQUIRE(!confusion || conf_dim >= K, MV_E_ARG, "mv_spair_match_batch: conf_dim=%d must be >= K=%d", conf_dim, K);
+// mv_spair_match_batch (feat_dtype = MV_FEAT_F32) and mv_spair_match_batch_typed; `fn` names the entry point in errors
+int spair_match_batch(const char* fn, const void* feats, int feat_dtype, int B, int C, int h, int w, const float* kps_i,
+                      const float* kps_j, int K, int kp_stride, const float* thresh_scale, float image_size, float pck_thresh,
+                      int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn, unsigned long long* hits,
+                      unsigned long long* confusion, int conf_dim, mv_stream_t stream) {
+  MV_REQUIRE(feat_dtype == MV_FEAT_F32 || feat_dtype == MV_FEAT_BF16 || feat_dtype == MV_FEAT_F16, MV_E_ARG,
+             "%s: unknown feature dtype %d", fn, feat_dtype);
+  MV_REQUIRE(B >= 0 && C > 0 && h > 0 && w > 0, MV_E_ARG, "%s: bad sizes", fn);
+  MV_REQUIRE((B == 0 || K == 0) || (feats && kps_i && kps_j && thresh_scale), MV_E_ARG, "%s: null pointer", fn);
+  const uintptr_t elem = feat_dtype == MV_FEAT_F32 ? 4 : 2;
+  MV_REQUIRE(((uintptr_t)feats & (elem - 1)) == 0, MV_E_ALIGN, "%s: feats must be aligned to its %d-byte elements", fn,
+             (int)elem);
+  MV_REQUIRE(h * w <= SPB_MAX_HW, MV_E_RANGE, "%s: h*w=%d exceeds %d pixels", fn, h * w, SPB_MAX_HW);
+  MV_REQUIRE(K >= 0 && K <= 64, MV_E_RANGE, "%s: K=%d must be in [0, 64]", fn, K);
+  MV_REQUIRE(kp_stride >= 3 && image_size > 0.f, MV_E_ARG, "%s: bad key-point layout", fn);
+  MV_REQUIRE(!confusion || conf_dim >= K, MV_E_ARG, "%s: conf_dim=%d must be >= K=%d", fn, conf_dim, K);
   if (B == 0 || K == 0) return MV_OK;
+  MV_REQUIRE(8 * (size_t)C * sizeof(float) <= (160u << 10), MV_E_RANGE, "%s: C=%d too large for the key-point tile", fn, C);
   SpairBatchParams p;
   p.feats = feats;
   p.kps_i = kps_i;
@@ -902,16 +949,30 @@ int mv_spair_match_batch(const float* feats, int B, int C, int h, int w, const f
   p.conf_dim = conf_dim;
   p.stages = p.cc = p.rs = 0;
   cudaStream_t st = mv_cuda_stream(stream);
-  // key-point tile = accumulators per thread; the tile's features (C * KT floats) must fit shared memory
-  const size_t budget = 160u << 10;
-  const size_t per_k = (size_t)C * sizeof(float);
-  MV_REQUIRE(8 * per_k <= budget, MV_E_RANGE, "mv_spair_match_batch: C=%d too large for the key-point tile", C);
-  if (K > 24 && 32 * per_k <= budget) return launch_spair_batch<32>(p, st);
-  if (K > 20 && 24 * per_k <= budget) return launch_spair_batch<24>(p, st);
-  if (K > 16 && 20 * per_k <= budget) return launch_spair_batch<20>(p, st);  // SPair-71k: up to 20 key points for most classes
-  if (K > 12 && 16 * per_k <= budget) return launch_spair_batch<16>(p, st);
-  if (K > 8 && 12 * per_k <= budget) return launch_spair_batch<12>(p, st);
-  return launch_spair_batch<8>(p, st);
+  if (feat_dtype == MV_FEAT_BF16) return launch_spair_tiles<__nv_bfloat16>(p, st);
+  if (feat_dtype == MV_FEAT_F16) return launch_spair_tiles<__half>(p, st);
+  return launch_spair_tiles<float>(p, st);
+}
+
+}  // namespace
+
+extern "C" {
+
+int mv_spair_match_batch(const float* feats, int B, int C, int h, int w, const float* kps_i, const float* kps_j, int K,
+                         int kp_stride, const float* thresh_scale, float image_size, float pck_thresh,
+                         int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
+                         unsigned long long* hits, unsigned long long* confusion, int conf_dim, mv_stream_t stream) {
+  return spair_match_batch("mv_spair_match_batch", feats, MV_FEAT_F32, B, C, h, w, kps_i, kps_j, K, kp_stride, thresh_scale,
+                           image_size, pck_thresh, pred_flat, error_same, error_nn, index_nn, hits, confusion, conf_dim, stream);
+}
+
+int mv_spair_match_batch_typed(const void* feats, int feat_dtype, int B, int C, int h, int w, const float* kps_i,
+                               const float* kps_j, int K, int kp_stride, const float* thresh_scale, float image_size,
+                               float pck_thresh, int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
+                               unsigned long long* hits, unsigned long long* confusion, int conf_dim, mv_stream_t stream) {
+  return spair_match_batch("mv_spair_match_batch_typed", feats, feat_dtype, B, C, h, w, kps_i, kps_j, K, kp_stride,
+                           thresh_scale, image_size, pck_thresh, pred_flat, error_same, error_nn, index_nn, hits, confusion,
+                           conf_dim, stream);
 }
 
 int mv_spair_set_heatmap_terms(int terms) {

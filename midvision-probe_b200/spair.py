@@ -73,11 +73,17 @@ def compute_errors_batch(feats, kps_i, kps_j, thresh_scale, image_size, pck_thre
     thresh_scale: (B,) tensor or sequence.  Returns device tensors (error_same, error_nn, index_nn, pred), each
     (B, K): entries of key points that are not in both images are -1 (the reference drops them, :96-98);
     pred is the flat arg-max pixel of each heat map (:83).  hits / confusion accumulate like
-    compute_errors_from_features.  Everything is fp32 on the device (mv_spair_match_batch); nothing syncs.
+    compute_errors_from_features.  Nothing syncs.
+
+    A bf16 or fp16 feats (an autocast backbone's output, on the host or the device) is uploaded and made contiguous as
+    it is, and the kernel reads the 16-bit map (mv_spair_match_batch_typed): half the bytes, widened exactly on the chip,
+    and the same results, bit for bit, as for feats.float().  Any other dtype is converted to fp32 first.  The key
+    points and the arithmetic are fp32 throughout.
     """
     dev = C_._device()
     st = C_._stream()
-    f = C_._f32(feats, dev)
+    f16 = feats.dtype in (torch.bfloat16, torch.float16)
+    f = feats.detach().to(device=dev, non_blocking=True).contiguous() if f16 else C_._f32(feats, dev)
     B, two, C, h, w = f.shape
     if two != 2:
         raise ValueError("feats must be (B, 2, C, h, w)")
@@ -95,9 +101,13 @@ def compute_errors_batch(feats, kps_i, kps_j, thresh_scale, image_size, pck_thre
     err_same = torch.empty((B, K), dtype=torch.float32, device=dev)
     err_nn = torch.empty((B, K), dtype=torch.float32, device=dev)
     idx_nn = torch.empty((B, K), dtype=torch.int32, device=dev)
-    L.call("mv_spair_match_batch", L.ptr(f), B, C, h, w, L.ptr(ki), L.ptr(kj), K, ki.shape[2], L.ptr(ts),
-           c_float(float(image_size)), c_float(float(pck_thresh)), L.ptr(pred), L.ptr(err_same), L.ptr(err_nn),
-           L.ptr(idx_nn), L.ptr(hits), L.ptr(confusion), 0 if confusion is None else confusion.shape[1], st)
+    rest = (B, C, h, w, L.ptr(ki), L.ptr(kj), K, ki.shape[2], L.ptr(ts), c_float(float(image_size)),
+            c_float(float(pck_thresh)), L.ptr(pred), L.ptr(err_same), L.ptr(err_nn), L.ptr(idx_nn), L.ptr(hits),
+            L.ptr(confusion), 0 if confusion is None else confusion.shape[1], st)
+    if f16:
+        L.call("mv_spair_match_batch_typed", L.ptr(f), C_._FEAT_DTYPES[f.dtype], *rest)
+    else:
+        L.call("mv_spair_match_batch", L.ptr(f), *rest)
     return err_same, err_nn, idx_nn, pred
 
 
