@@ -416,6 +416,25 @@ int mv_spair_match_batch_typed(const void* feats, int feat_dtype, int B, int C, 
                                float pck_thresh, int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
                                unsigned long long* hits, unsigned long long* confusion, int conf_dim, mv_stream_t stream);
 
+/* mv_spair_match_batch_typed with a caller workspace, for large maps (50 x 50 at the reference's 800-pixel input).  When
+ * h*w > 256, C % 8 == 0 and feats is 16-byte aligned it takes the tiled form: the pixels of image j are split into 256-pixel
+ * tiles over many CTAs, so that one pair spreads over the GPU, in four launches on `stream` (tap norms, key-point features,
+ * tiles, scoring) with no host sync.  Otherwise it is exactly mv_spair_match_batch_typed and the workspace is not used.
+ * Same outputs and contract: the arg-max equals the fp32 reference's wherever the top-2 heat-map gap exceeds 1e-5 (1e-3
+ * with mv_spair_set_heatmap_terms(1)), ties go to the lower pixel, and a bf16 / fp16 map gives the bits of its fp32
+ * widening through the same form.  A pair's results do not depend on the batch it is in.  workspace: device memory of at
+ * least mv_spair_tiled_workspace_bytes(B, C, h, w, K) bytes, any alignment, used by this call only (not between calls on
+ * other streams).  Errors, checked before any CUDA call: those of mv_spair_match_batch_typed, and MV_E_WORKSPACE for a
+ * missing or short workspace when the tiled form is taken. */
+int mv_spair_match_batch_tiled(const void* feats, int feat_dtype, int B, int C, int h, int w, const float* kps_i,
+                               const float* kps_j, int K, int kp_stride, const float* thresh_scale, float image_size,
+                               float pck_thresh, int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
+                               unsigned long long* hits, unsigned long long* confusion, int conf_dim, void* workspace,
+                               size_t workspace_bytes, mv_stream_t stream);
+/* Workspace bytes of mv_spair_match_batch_tiled for B pairs of (C, h, w) maps and K key-point slots (any element type);
+ * 0 for bad sizes and when there is no work (B == 0 or K == 0). */
+size_t mv_spair_tiled_workspace_bytes(int B, int C, int h, int w, int K);
+
 /* Precision of the batched kernel's heat map (the einsum of evaluate_spair_correspondence.py:82) on the tensor cores:
  * 3 (default) = every product as three tf32 MMAs (hi*hi + hi*lo + lo*hi, ~21 mantissa bits: the arg-max equals the fp32
  * reference's wherever the top-2 heat-map gap exceeds 1e-5); 1 = one tf32 MMA, operands rounded to 10 mantissa bits with

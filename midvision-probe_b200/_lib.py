@@ -68,6 +68,9 @@ PROTOTYPES = {
                                      c_int, P]),
     "mv_spair_match_batch_typed": (c_int, [P, c_int, c_int, c_int, c_int, c_int, P, P, c_int, c_int, P, c_float, c_float, P, P,
                                            P, P, P, P, c_int, P]),
+    "mv_spair_match_batch_tiled": (c_int, [P, c_int, c_int, c_int, c_int, c_int, P, P, c_int, c_int, P, c_float, c_float, P, P,
+                                           P, P, P, P, c_int, P, c_size_t, P]),
+    "mv_spair_tiled_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
 }
 
 # enums of include/mvmatch.h
@@ -92,6 +95,7 @@ KERNELS_PER_CALL = {
     "mv_geom_grid_coords": 1, "mv_geom_keypoint_coords": 1, "mv_k1_sample_normalize": 1, "mv_k1_sample_f16c": 1, "mv_k1_sample_tf32c": 1, "mv_rows_center": 2, "mv_rows_dot": 1, "mv_rank_of_valid": 1, "mv_k1_grid_f16c": 1, "mv_lr_unit_rows": 1, "mv_lr_gram_exact": 2, "mv_lr_build_query": 1, "mv_lr_build_target": 1, "mv_k3_ratio_mutual_lr": 1, "mv_k2_sim_top2": 2, "mv_k2_sim_top2_ld": 2, "mv_k2_affinity": 2, "mv_k2_sim_topk_ld": 2, "mv_knn_rerank": 1, "mv_affinity_threshold": 1, "mv_cosine_2afc": 1,
     "mv_k2_unpack_col": 1, "mv_k3_ratio_mutual": 1, "mv_k3_ratio_mutual_split": 1, "mv_k3_ratio_mutual_f16c": 1, "mv_k3_topk_matches": 1, "mv_k3_score": 1, "mv_gather_rows": 1,
     "mv_pack_matches": 1, "mv_argmax_rows": 1, "mv_k3_spair_errors": 1, "mv_spair_match_batch": 1, "mv_spair_match_batch_typed": 1,
+    "mv_spair_match_batch_tiled": 4,  # the tiled form (h*w > 256); otherwise it is the one launch of _typed
 }
 LAUNCHES = {"count": 0}
 

@@ -5,6 +5,8 @@
 //                          -- one CTA per pair, fp32 arithmetic throughout
 //   mv_spair_match_batch_typed   the same on an fp32, bf16 or fp16 map: 16-bit maps are read as they are and widened
 //                          on the chip, with the fp32 results of the widened map bit for bit
+//   mv_spair_match_batch_tiled   the same with a caller workspace: maps above 256 pixels take the tiled form of
+//                          spair_tiled.cu (one pair over many CTAs) instead of this file's first form
 //
 // Reference behaviour being reproduced (file:line in /root/reference):
 //   evaluate_spair_correspondence.py:59     feats = F.normalize(feats, p=2, dim=1)
@@ -22,50 +24,17 @@
 #include <math_constants.h>
 #include <stdlib.h>
 
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
-
 #include <type_traits>
 
 #include "common.cuh"
 #include "sm100_ptx.cuh"
+#include "spair_common.cuh"
 #include "spair_score.cuh"
 
 namespace {
 
 constexpr int SPB_THREADS = 256;
 constexpr int SPB_MAX_HW = 1 << 20;  // pixels per feature map (2500 at the reference's 800 x 800 input)
-constexpr float SPB_NORM_EPS = 1e-12f;  // F.normalize default eps
-
-// element type T of the maps: float, or the __nv_bfloat16 / __half output of an autocast backbone.  Every 16-bit value is
-// an fp32 value (widening is exact), and every one is also exactly a tf32 value (8 / 11 significant bits, fp32's exponent
-// range): the kernels widen on load from global or shared memory and then run the fp32 arithmetic unchanged.
-__device__ __forceinline__ float sp_f32(float v) { return v; }
-__device__ __forceinline__ float sp_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
-__device__ __forceinline__ float sp_f32(__half v) { return __half2float(v); }
-// two neighbouring values, one 8-byte (float) or 4-byte (16-bit) aligned load
-__device__ __forceinline__ float2 sp_f32x2(const float* v) { return *reinterpret_cast<const float2*>(v); }
-__device__ __forceinline__ float2 sp_f32x2(const __nv_bfloat16* v) {
-  return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(v));
-}
-__device__ __forceinline__ float2 sp_f32x2(const __half* v) { return __half22float2(*reinterpret_cast<const __half2*>(v)); }
-
-struct SpairBatchParams {
-  const void* feats;  // (B, 2, C, h, w) of the launch's element type
-  const float* kps_i;  // (B, K, stride)
-  const float* kps_j;
-  const float* thresh_scale;  // (B)
-  int B, C, h, w, K, stride;
-  float image_size, pck;
-  int32_t* pred;  // (B, K)
-  float* error_same;
-  float* error_nn;
-  int32_t* index_nn;
-  unsigned long long* hits;
-  unsigned long long* confusion;
-  int conf_dim;
-  int stages, cc, rs;  // streaming form: ring depth, channels per half slot, row stride in floats (set by the launcher)
-};
 
 // dynamic shared memory: q[C][KT], the key-point features of the current tile
 // blockDim.x = min(SPB_THREADS, h*w rounded up to a warp): thread = pixel in the heat-map pass, so a 14 x 14 map
@@ -304,39 +273,6 @@ static_assert(SPS_CC % 8 == 0 && SPS_CC >= 8, "whole K steps");
 #ifndef SPS_HINTS
 #define SPS_HINTS 1
 #endif
-
-// m16n8k8 tf32 tensor-core step (legacy warp-level MMA: the heat map of a pair is 196 x 20 x 768, far below a tcgen05 tile)
-__device__ __forceinline__ void mma_tf32(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-// x = hi + lo with hi exactly representable in tf32 (the tensor core drops the low 13 mantissa bits of its operands);
-// hi*hi + hi*lo + lo*hi carries ~21 mantissa bits ("3xTF32")
-// (the AND sits in an asm block: seen by the compiler, it is dropped for the MMA operand -- the tensor core ignores those bits --
-// and kept for the subtraction, and the raw values are then MOVed into the operand's register quad: three instructions per
-// value instead of two)
-__device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
-  asm("and.b32 %0, %1, 0xffffe000;" : "=r"(hi) : "r"(__float_as_uint(x)));
-  lo = __float_as_uint(x - __uint_as_float(hi));
-}
-
-// where q[c][k] of a chunk sits in its buffer.  Tensor-core pass: per K step (8 channels) and N tile j (8 key points) the
-// B fragment of lane (g, t) -- channels t and t + 4 of key point 8 j + g, each already split into its tf32 halves -- is one
-// float4 {hi(t), hi(t + 4), lo(t), lo(t + 4)} (the register pairs the MMA takes, no moves), lanes in order: a conflict-free
-// LDS.128, and the split is done once per value by step Q instead of once per warp by step H.  Columns beyond KT stay zero
-// from the start of the kernel.
-template <int KT, bool MMA>
-__device__ __forceinline__ int sps_q_off(int c, int k) {
-  if (!MMA) return c * KT + k;
-  constexpr int NT8 = (KT + 7) / 8;
-  const int c8 = c & 7;
-  return (((c >> 3) * NT8 + (k >> 3)) * 32 + ((k & 7) << 2) + (c8 & 3)) * 4 + (c8 >> 2);
-}
-template <int KT, bool MMA>
-constexpr int sps_q_floats(int cc) {  // one q buffer
-  return MMA ? (cc / 8) * ((KT + 7) / 8) * 128 : cc * KT;
-}
 
 // MMA: the heat-map step on the tensor cores -- pixels on M (16 per tile, 2 tiles per warp), key points on N (8 per tile),
 // 8 channels per K step, 3xTF32 -- instead of 21 FFMA + 6 LDS per channel and pixel.
@@ -802,7 +738,6 @@ __global__ void __launch_bounds__(SPS_THREADS, SPS_CTAS) spair_stream_kernel(Spa
   }
 }
 
-int g_spair_terms = 3;  // mv_spair_set_heatmap_terms
 
 // shared-memory plan of the streaming form
 struct SpsPlan {
@@ -838,7 +773,7 @@ template <typename T, int KT>
 int launch_spair_stream(const SpairBatchParams& p, const SpsPlan& pl, cudaStream_t st) {
   // MVMATCH_SPAIR_MMA=0: the heat-map step on the CUDA cores (the arithmetic of the first form)
   static const bool mma = !(getenv("MVMATCH_SPAIR_MMA") && getenv("MVMATCH_SPAIR_MMA")[0] == '0');
-  const bool one_term = mma && g_spair_terms == 1;
+  const bool one_term = mma && spair_heatmap_terms() == 1;
   auto kern = !mma ? spair_stream_kernel<T, KT, false>
                    : one_term ? spair_stream_kernel<T, KT, true, 1> : spair_stream_kernel<T, KT, true, 3>;
   static size_t opted[MV_MAX_DEVICES][3];
@@ -909,11 +844,13 @@ int launch_spair_tiles(const SpairBatchParams& p, cudaStream_t st) {
   return launch_spair_batch<T, 8>(p, st);
 }
 
-// mv_spair_match_batch (feat_dtype = MV_FEAT_F32) and mv_spair_match_batch_typed; `fn` names the entry point in errors
+// mv_spair_match_batch (feat_dtype = MV_FEAT_F32), mv_spair_match_batch_typed and, with `tiled`,
+// mv_spair_match_batch_tiled; `fn` names the entry point in errors
 int spair_match_batch(const char* fn, const void* feats, int feat_dtype, int B, int C, int h, int w, const float* kps_i,
                       const float* kps_j, int K, int kp_stride, const float* thresh_scale, float image_size, float pck_thresh,
                       int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn, unsigned long long* hits,
-                      unsigned long long* confusion, int conf_dim, mv_stream_t stream) {
+                      unsigned long long* confusion, int conf_dim, mv_stream_t stream, bool tiled = false,
+                      void* workspace = nullptr, size_t workspace_bytes = 0) {
   MV_REQUIRE(feat_dtype == MV_FEAT_F32 || feat_dtype == MV_FEAT_BF16 || feat_dtype == MV_FEAT_F16, MV_E_ARG,
              "%s: unknown feature dtype %d", fn, feat_dtype);
   MV_REQUIRE(B >= 0 && C > 0 && h > 0 && w > 0, MV_E_ARG, "%s: bad sizes", fn);
@@ -927,6 +864,13 @@ int spair_match_batch(const char* fn, const void* feats, int feat_dtype, int B, 
   MV_REQUIRE(!confusion || conf_dim >= K, MV_E_ARG, "%s: conf_dim=%d must be >= K=%d", fn, conf_dim, K);
   if (B == 0 || K == 0) return MV_OK;
   MV_REQUIRE(8 * (size_t)C * sizeof(float) <= (160u << 10), MV_E_RANGE, "%s: C=%d too large for the key-point tile", fn, C);
+  // the tiled form: maps above the streaming form's 256 pixels, whole K steps of channels, 16-byte aligned maps
+  tiled = tiled && h * w > 256 && C % 8 == 0 && ((uintptr_t)feats & 15) == 0;
+  if (tiled) {
+    const size_t need = spair_tiled_workspace_bytes(B, C, K);
+    MV_REQUIRE(workspace && workspace_bytes >= need, MV_E_WORKSPACE, "%s: workspace of %zu bytes, %zu needed", fn,
+               workspace ? workspace_bytes : (size_t)0, need);
+  }
   SpairBatchParams p;
   p.feats = feats;
   p.kps_i = kps_i;
@@ -949,12 +893,20 @@ int spair_match_batch(const char* fn, const void* feats, int feat_dtype, int B, 
   p.conf_dim = conf_dim;
   p.stages = p.cc = p.rs = 0;
   cudaStream_t st = mv_cuda_stream(stream);
+  if (tiled) {
+    if (feat_dtype == MV_FEAT_BF16) return spair_tiled_launch<__nv_bfloat16>(p, workspace, st);
+    if (feat_dtype == MV_FEAT_F16) return spair_tiled_launch<__half>(p, workspace, st);
+    return spair_tiled_launch<float>(p, workspace, st);
+  }
   if (feat_dtype == MV_FEAT_BF16) return launch_spair_tiles<__nv_bfloat16>(p, st);
   if (feat_dtype == MV_FEAT_F16) return launch_spair_tiles<__half>(p, st);
   return launch_spair_tiles<float>(p, st);
 }
 
 }  // namespace
+
+static int g_spair_terms = 3;  // mv_spair_set_heatmap_terms
+int spair_heatmap_terms() { return g_spair_terms; }
 
 extern "C" {
 
@@ -973,6 +925,21 @@ int mv_spair_match_batch_typed(const void* feats, int feat_dtype, int B, int C, 
   return spair_match_batch("mv_spair_match_batch_typed", feats, feat_dtype, B, C, h, w, kps_i, kps_j, K, kp_stride,
                            thresh_scale, image_size, pck_thresh, pred_flat, error_same, error_nn, index_nn, hits, confusion,
                            conf_dim, stream);
+}
+
+int mv_spair_match_batch_tiled(const void* feats, int feat_dtype, int B, int C, int h, int w, const float* kps_i,
+                               const float* kps_j, int K, int kp_stride, const float* thresh_scale, float image_size,
+                               float pck_thresh, int32_t* pred_flat, float* error_same, float* error_nn, int32_t* index_nn,
+                               unsigned long long* hits, unsigned long long* confusion, int conf_dim, void* workspace,
+                               size_t workspace_bytes, mv_stream_t stream) {
+  return spair_match_batch("mv_spair_match_batch_tiled", feats, feat_dtype, B, C, h, w, kps_i, kps_j, K, kp_stride,
+                           thresh_scale, image_size, pck_thresh, pred_flat, error_same, error_nn, index_nn, hits, confusion,
+                           conf_dim, stream, true, workspace, workspace_bytes);
+}
+
+size_t mv_spair_tiled_workspace_bytes(int B, int C, int h, int w, int K) {
+  if (B < 0 || C <= 0 || h <= 0 || w <= 0 || (size_t)h * w > (size_t)SPB_MAX_HW || K < 0 || K > 64) return 0;
+  return spair_tiled_workspace_bytes(B, C, K);
 }
 
 int mv_spair_set_heatmap_terms(int terms) {

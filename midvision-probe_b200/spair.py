@@ -79,6 +79,11 @@ def compute_errors_batch(feats, kps_i, kps_j, thresh_scale, image_size, pck_thre
     it is, and the kernel reads the 16-bit map (mv_spair_match_batch_typed): half the bytes, widened exactly on the chip,
     and the same results, bit for bit, as for feats.float().  Any other dtype is converted to fp32 first.  The key
     points and the arithmetic are fp32 throughout.
+
+    Maps above 256 pixels (50 x 50 at the reference's 800-pixel input) go to mv_spair_match_batch_tiled, which spreads
+    each pair over many CTAs in 256-pixel tiles, with a workspace allocated here as a uint8 tensor.  The contract is the
+    same in every form: arg-max equal to the fp32 reference's wherever its top-2 heat-map gap exceeds 1e-5 (1e-3 under
+    set_heatmap_precision("tf32")), and a 16-bit map bit-identical to its fp32 widening.
     """
     dev = C_._device()
     st = C_._stream()
@@ -103,11 +108,16 @@ def compute_errors_batch(feats, kps_i, kps_j, thresh_scale, image_size, pck_thre
     idx_nn = torch.empty((B, K), dtype=torch.int32, device=dev)
     rest = (B, C, h, w, L.ptr(ki), L.ptr(kj), K, ki.shape[2], L.ptr(ts), c_float(float(image_size)),
             c_float(float(pck_thresh)), L.ptr(pred), L.ptr(err_same), L.ptr(err_nn), L.ptr(idx_nn), L.ptr(hits),
-            L.ptr(confusion), 0 if confusion is None else confusion.shape[1], st)
-    if f16:
-        L.call("mv_spair_match_batch_typed", L.ptr(f), C_._FEAT_DTYPES[f.dtype], *rest)
+            L.ptr(confusion), 0 if confusion is None else confusion.shape[1])
+    dtype = C_._FEAT_DTYPES[f.dtype] if f16 else L.MV_FEAT_F32
+    if h * w > 256:
+        nbytes = L.load().mv_spair_tiled_workspace_bytes(B, C, h, w, K)
+        ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=dev)
+        L.call("mv_spair_match_batch_tiled", L.ptr(f), dtype, *rest, L.ptr(ws), c_size_t(nbytes), st)
+    elif f16:
+        L.call("mv_spair_match_batch_typed", L.ptr(f), dtype, *rest, st)
     else:
-        L.call("mv_spair_match_batch", L.ptr(f), *rest)
+        L.call("mv_spair_match_batch", L.ptr(f), *rest, st)
     return err_same, err_nn, idx_nn, pred
 
 
