@@ -322,7 +322,9 @@ int mv_k3_ratio_mutual_split(const uint16_t* A_hi, const uint16_t* A_lo, const u
 
 /* The same on f16c rows (mv_k1_sample_f16c): A_hi (n, pitch) / A_lo (n, C) query rows, B_hi / B_lo target rows,
  * center_B (C floats or NULL) the centre the target rows are relative to; every element is rebuilt as
- * float(hi) + float(lo) * 2^-11 (+ center_B) before the identical fp32 arithmetic. */
+ * float(hi) + float(lo) * 2^-11 (+ center_B) before the identical fp32 arithmetic.  With center_B, a rebuilt target row
+ * of squared norm below 1e-10 counts as a zero row (distance 1, as for a zero vector): a zero row stored relative to
+ * the centre rebuilds to a residual of ~2^-22 |center_B| per element, not to 0.  The rows are L2-normalised (norm 1 or 0). */
 int mv_k3_ratio_mutual_f16c(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* B_hi, const uint16_t* B_lo, int C, int pitch,
                             const float* center_B, const int32_t* n_dev, int n_max, int32_t* row_idx,
                             const unsigned long long* col_best, int ratio_test, float* dists, float* weight, uint8_t* mutual,

@@ -29,6 +29,7 @@ namespace {
 constexpr float COS_EPS = 1e-8f;     // torch.nn.functional.cosine_similarity default eps
 constexpr float RATIO_CLAMP = 1e-9f; // calculate_ratio_test clamps
 constexpr float MISSING_DIST = 2.0f; // distance reported for a candidate that does not exist (m < 2)
+constexpr float F16C_ZERO_SS = 1e-10f;  // f16c target rows: squared norms below this are the rebuild residual of a zero row
 
 // ------------------------------------------------------------------------------------------
 // ratio / mutual: one warp per query row
@@ -179,6 +180,15 @@ __global__ void __launch_bounds__(RATIO_THREADS, 6) k3_ratio_mutual_kernel(ROWS 
     }
   }
   if (!live || lane != 0 || wsub != 0) return;
+  if constexpr (sizeof(ROWS) == sizeof(RowsF16c)) {
+    // a zero target row stored relative to the centre rebuilds as hi + lo * 2^-11 + mu: a residual of up to ~2^-21 |mu| per
+    // element (norm ~4e-8 for |mu| ~ 1), not 0, whose cosine with the query is rounding noise.  The rows are L2-normalised
+    // (norm 1, or 0 for a zero input row), so a rebuilt row below F16C_ZERO_SS is that residual: cosine 0, as for a zero row
+    if (rows.center_B) {
+      if (aa < F16C_ZERO_SS) xa = 0.f;
+      if (bb < F16C_ZERO_SS) xb = 0.f;
+    }
+  }
   const float nx = fmaxf(sqrtf(xx), COS_EPS);
   float d0 = j0 >= 0 ? 1.f - xa / (nx * fmaxf(sqrtf(aa), COS_EPS)) : MISSING_DIST;
   float d1 = j1 >= 0 ? 1.f - xb / (nx * fmaxf(sqrtf(bb), COS_EPS)) : MISSING_DIST;

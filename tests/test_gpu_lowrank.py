@@ -42,7 +42,18 @@ def sides(mv, kind, p):
 
 @pytest.mark.parametrize("kind,shape", [("depth", dict(C=256, h=15, w=20, H=60, W=80)), ("depth", dict(C=64, h=7, w=9, H=40, W=52)),
                                         ("xyz", dict(C=256, h=14, w=14, H=56, W=56, radius=22.0)),
-                                        ("xyz", dict(C=128, h=9, w=11, H=36, W=44, radius=15.0))])
+                                        ("xyz", dict(C=128, h=9, w=11, H=36, W=44, radius=15.0)),
+                                        # every width of lr_build_query (KT = ceil(hwp / 64) -> 8, 13, 16) up to the 1024-pixel limit.  The
+                                        # top-2 error is the fp16 rounding of A - c_i at the best candidates' taps; it does not depend on the
+                                        # width (an fp16 emulation of the operands gives the same 1.2-1.6e-4 at 14 x 14 and 32 x 32, C = 256)
+                                        # but on how far those taps sit below the row's maximum: it grows with sparse targets (a 1.3x
+                                        # upsample or 90 % of the pixels invalid: 2-3e-4) and, for the 16 bicubic taps (sum |B| ~ 2.8), with
+                                        # the 1 / sqrt(C) spread of the cosines between Gaussian features (C = 128: 2.4e-4 at 28 x 28,
+                                        # 1.6e-4 already at 14 x 14).  So these shapes keep the regime of the ones above: a dense 4x upsample,
+                                        # C = 256 for the bicubic ones
+                                        ("depth", dict(C=256, h=18, w=20, H=36, W=40)), ("xyz", dict(C=256, h=16, w=21, H=32, W=42, radius=30.0)),
+                                        ("depth", dict(C=256, h=24, w=24, H=96, W=96)), ("xyz", dict(C=256, h=28, w=28, H=112, W=112, radius=50.0)),
+                                        ("depth", dict(C=128, h=30, w=30, H=120, W=120)), ("xyz", dict(C=256, h=32, w=32, H=128, W=128, radius=56.0))])
 @pytest.mark.parametrize("exact", [False, True])
 def test_operand_product_equals_the_cosine_similarity(mv, syn, kind, shape, exact):
     """exact=False: cosine Gram of fp16 unit rows from kernel 2; exact=True: fp32 Gram of the raw rows from the CUDA cores"""
@@ -57,9 +68,9 @@ def test_operand_product_equals_the_cosine_similarity(mv, syn, kind, shape, exac
     hw = h * w
     hwp = (hw + 7) // 8 * 8
     assert K == hwp + 8
-    A, B = A[:, :K].float().cpu().double(), B[:, :K].float().cpu().double()
+    A, B = A[:, :K].double(), B[:, :K].double()  # fp64 on the device: the widest shapes have ~15k points per side
     S = A @ B.t()
-    a, b = F.normalize(f0, dim=-1).double(), F.normalize(f1, dim=-1).double()
+    a, b = F.normalize(f0, dim=-1).double().cuda(), F.normalize(f1, dim=-1).double().cuda()
     S_ref = a @ b.t()
     err = (S - S_ref).abs()
     # fp16 operands: 2^-11 relative on entries of magnitude <= 1, a handful of terms per product
@@ -99,7 +110,8 @@ def test_helpers_with_the_lowrank_proposal_match_the_oracle(mv, syn, lowrank_on,
         assert int((diff > 2e-5).sum()) <= 5 and float(diff.max()) < 5e-3, (kind, seed, float(diff.max()))
 
 
-@pytest.mark.parametrize("C,h,w,taps", [(2048, 15, 20, 2), (256, 9, 7, 4), (3072, 12, 12, 4), (320, 28, 28, 2)])
+@pytest.mark.parametrize("C,h,w,taps", [(2048, 15, 20, 2), (256, 9, 7, 4), (3072, 12, 12, 4), (320, 28, 28, 2),
+                                         (128, 32, 32, 4), (256, 31, 33, 2)])  # off1 = 1024: the limit
 def test_exact_gram_is_fp32_exact(mv, C, h, w, taps):
     """mv_lr_gram_exact against an fp64 product: every entry it promises (the whole cross block, the same-image entries whose
     indices are at most `reach` apart) to ~1 ulp (blocked fp32 accumulation), symmetric, pad rows zero, snorm / rsnorm from
