@@ -385,11 +385,17 @@ __device__ __forceinline__ float dot4(const float4& v, float ss) {
 // window) while the THREADS / 32 CONSUMER warps run phase B of sub-run i; two windows, full / empty mbarriers.  The window
 // fill is bound by L2 -> SM bandwidth (128 MB of reads for a NAVI-shaped side) and the row writes by HBM: with one phase
 // after the other (PW == 0) a side costs the sum, here the larger of the two.
-template <int MODE, int NITW, int W, int G, int OUTS, int THREADS, int MINB, int PW = 0>
+// BULK > 0: f16c split rows leave through bulk stores: each warp stages its point's hi row (C + 8 fp16, augmentation
+// columns included) and lo row (C fp16), BULK pieces of C / BULK channels at a time, in a slot of its own behind the
+// window, and its lane 0 copies them to global memory with cp.async.bulk.  The warp goes on as soon as a piece is handed
+// over, so the window fill of the next sub-run runs while the last rows of this one drain.
+template <int MODE, int NITW, int W, int G, int OUTS, int THREADS, int MINB, int PW = 0, int BULK = 0>
 __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Params p, int nslots, uint32_t c4_magic) {
   static_assert(W == 1 || W == 2 || W == 4, "team size");
   static_assert(G >= 1 && G <= 4 && (THREADS / 32) % W == 0 && (W == 1 || THREADS / 32 / W <= 4), "team layout");
   static_assert(PW == 0 || MODE != MV_SAMPLE_ROWS, "the row-copy mode has no window to produce");
+  static_assert(!BULK || (W == 1 && G == 1 && NITW > 0 && OUTS == K1W_OUT_SPLIT && PW == 0 && MODE != MV_SAMPLE_ROWS),
+                "bulk row stores: one warp per point, whole rows in registers, f16c split rows only");
   extern __shared__ float4 k1w_dyn[];
   constexpr int NBUF = PW > 0 ? 2 : 1;
   __shared__ K1WShared<W> shb[NBUF];
@@ -416,11 +422,36 @@ __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Para
   const size_t pitch16 = f16c ? (size_t)p.pitch16 : (size_t)C;
   const bool haspd = p.pixdot != nullptr;                    // the dot product comes from per-pixel dots: nothing in the hot loop
   const bool hasdot = p.dotvec != nullptr && !haspd;
-  auto put = [&](int pt, int c, float4 o, float inv) {
+  auto scaled = [](float4 o, float inv) {
     o.x *= inv;  // inv == 1 when not normalising: exact
     o.y *= inv;
     o.z *= inv;
     o.w *= inv;
+    return o;
+  };
+  // fp16(o) of 4 channels and the residual * 2^11 (exact scaling): value = hi + lo * 2^-11 carries 22 mantissa bits
+  auto f16c_split = [](const float4& o, uint2& hi, uint2& lo) {
+    const __half2 h0 = __floats2half2_rn(o.x, o.y), h1 = __floats2half2_rn(o.z, o.w);
+    hi.x = *reinterpret_cast<const uint32_t*>(&h0);
+    hi.y = *reinterpret_cast<const uint32_t*>(&h1);
+    const float2 l = __half22float2(h0), h = __half22float2(h1);
+    const __half2 rl = __floats2half2_rn((o.x - l.x) * K1_LO_SCALE, (o.y - l.y) * K1_LO_SCALE);
+    const __half2 rh = __floats2half2_rn((o.z - h.x) * K1_LO_SCALE, (o.w - h.y) * K1_LO_SCALE);
+    lo.x = *reinterpret_cast<const uint32_t*>(&rl);
+    lo.y = *reinterpret_cast<const uint32_t*>(&rh);
+  };
+  auto centred = [&](int c, float4 o) {
+    if (p.center) {  // rows relative to the centre: the 16-bit rounding error scales with |row - center|
+      const float4 m = ld4(p.center + c);
+      o.x -= m.x;
+      o.y -= m.y;
+      o.z -= m.z;
+      o.w -= m.w;
+    }
+    return o;
+  };
+  auto put = [&](int pt, int c, float4 o, float inv) {
+    o = scaled(o, inv);
     if (has32) __stcs(reinterpret_cast<float4*>(p.out_f32 + (size_t)pt * C + c), o);
     if (p.out_op32) {  // tf32 operand rows: centred, rounded to nearest tf32 here (the tensor core would truncate)
       float4 y = o;
@@ -438,27 +469,13 @@ __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Para
       *reinterpret_cast<float4*>(p.out_op32 + (size_t)pt * p.pitch_op32 + c) = y;
     }
     if (has16) {
-      if (p.center) {  // rows relative to the centre: the 16-bit rounding error scales with |row - center|
-        const float4 m = ld4(p.center + c);
-        o.x -= m.x;
-        o.y -= m.y;
-        o.z -= m.z;
-        o.w -= m.w;
-      }
+      o = centred(c, o);
       uint2 pk;
       if (f16c) {
-        const __half2 lo = __floats2half2_rn(o.x, o.y), hi = __floats2half2_rn(o.z, o.w);
-        pk.x = *reinterpret_cast<const uint32_t*>(&lo);
-        pk.y = *reinterpret_cast<const uint32_t*>(&hi);
+        uint2 pl;
+        f16c_split(o, pk, pl);
         *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(p.out_bf16) + (size_t)pt * pitch16 + c) = pk;
-        if (haslo) {  // residual * 2^11 (exact scaling): value = hi + lo * 2^-11 carries 22 mantissa bits
-          const float2 l = __half22float2(lo), h = __half22float2(hi);
-          const __half2 rl = __floats2half2_rn((o.x - l.x) * K1_LO_SCALE, (o.y - l.y) * K1_LO_SCALE);
-          const __half2 rh = __floats2half2_rn((o.z - h.x) * K1_LO_SCALE, (o.w - h.y) * K1_LO_SCALE);
-          pk.x = *reinterpret_cast<const uint32_t*>(&rl);
-          pk.y = *reinterpret_cast<const uint32_t*>(&rh);
-          *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(p.out_lo) + (size_t)pt * C + c) = pk;
-        }
+        if (haslo) *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(p.out_lo) + (size_t)pt * C + c) = pl;
         return;
       }
       __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
@@ -474,7 +491,24 @@ __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Para
       }
     }
   };
-  // the 8 augmentation columns of an f16c row (and the fp32 r), written by one lane per row
+  // the 8 augmentation columns of an f16c row
+  auto f16c_aug = [&](float r) {
+    __half a[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) a[k] = __float2half_rn(0.f);
+    if (p.role == MV_ROLE_TARGET) {
+      a[0] = __float2half_rn(1.f);
+      a[1] = __float2half_rn(1.f);
+      a[2] = __float2half_rn(1.f / K1_LO_SCALE);
+    } else {
+      a[0] = __float2half_rn(r);
+      const float r1 = r - __half2float(a[0]);
+      a[1] = __float2half_rn(r1);
+      a[2] = __float2half_rn((r1 - __half2float(a[1])) * K1_LO_SCALE);
+    }
+    return *reinterpret_cast<const uint4*>(a);
+  };
+  // the augmentation columns (and the fp32 r), written by one lane per row
   auto put_aug = [&](int pt, float r) {
     if (p.row_dot) p.row_dot[pt] = r;
     if (p.out_op32) {  // three tf32-exact pieces of r against (1, 1, 1) of the target rows
@@ -491,20 +525,7 @@ __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Para
       *reinterpret_cast<float4*>(q + 4) = a1;
     }
     if (!f16c || !has16) return;
-    __half a[8];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) a[k] = __float2half_rn(0.f);
-    if (p.role == MV_ROLE_TARGET) {
-      a[0] = __float2half_rn(1.f);
-      a[1] = __float2half_rn(1.f);
-      a[2] = __float2half_rn(1.f / K1_LO_SCALE);
-    } else {
-      a[0] = __float2half_rn(r);
-      const float r1 = r - __half2float(a[0]);
-      a[1] = __float2half_rn(r1);
-      a[2] = __float2half_rn((r1 - __half2float(a[1])) * K1_LO_SCALE);
-    }
-    *reinterpret_cast<uint4*>(reinterpret_cast<__half*>(p.out_bf16) + (size_t)pt * pitch16 + C) = *reinterpret_cast<const uint4*>(a);
+    *reinterpret_cast<uint4*>(reinterpret_cast<__half*>(p.out_bf16) + (size_t)pt * pitch16 + C) = f16c_aug(r);
   };
   // x * (1 / max(||x||, eps)) from the per-warp partial sums of squares of the cnt rows of a group; dd (raw row .
   // dotvec) is reduced the same way and comes back as r = (normalised row) . dotvec
@@ -554,6 +575,41 @@ __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Para
     return fmaf(v.w, d.w, acc);
   };
   const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
+
+  // BULK: stage the warp's row (scaled, centred, split exactly as put / put_aug do) in BULK pieces of C / BULK channels and
+  // hand each piece to the bulk-copy engine; the last piece carries the augmentation columns.  Lane 0 issues, commits
+  // and waits on the slot's bulk groups.
+  constexpr int CP = (NITW > 0 ? NITW * 128 : 4) / (BULK > 0 ? BULK : 1);  // channels per piece
+  __half* const stage_hi = reinterpret_cast<__half*>(winb[0] + (size_t)nslots * C) + (size_t)wid_all * (2 * CP + 8);
+  __half* const stage_lo = stage_hi + CP + 8;
+  auto stage_row = [&](int pt, const float4* acc, float inv, float r) {
+#pragma unroll
+    for (int k = 0; k < (BULK > 0 ? BULK : 1); ++k) {
+      if (lane == 0) sm100::bulk_wait_group_read0();  // the slot's previous piece has been read out
+      __syncwarp();
+#pragma unroll
+      for (int i = 0; i < CP / 128; ++i) {
+        const int c = (i * 32 + lane) * 4;
+        uint2 hi, lo;
+        f16c_split(centred(k * CP + c, scaled(acc[k * (CP / 128) + i], inv)), hi, lo);
+        *reinterpret_cast<uint2*>(stage_hi + c) = hi;
+        *reinterpret_cast<uint2*>(stage_lo + c) = lo;
+      }
+      const bool last = k == BULK - 1;
+      if (lane == 0 && last) {
+        if (p.row_dot) p.row_dot[pt] = r;
+        *reinterpret_cast<uint4*>(stage_hi + CP) = f16c_aug(r);
+      }
+      sm100::fence_proxy_async_smem();  // this lane's generic-proxy writes become visible to the bulk copy
+      __syncwarp();
+      if (lane == 0) {
+        sm100::bulk_store_1d(reinterpret_cast<__half*>(p.out_bf16) + (size_t)pt * pitch16 + k * CP, sm100::smem_u32(stage_hi),
+                             (CP + (last ? 8 : 0)) * 2);
+        sm100::bulk_store_1d(reinterpret_cast<__half*>(p.out_lo) + (size_t)pt * C + k * CP, sm100::smem_u32(stage_lo), CP * 2);
+        sm100::bulk_commit_group();
+      }
+    }
+  };
 
   if (MODE == MV_SAMPLE_ROWS) {  // rows as they are, no window: a team per row
     for (int pt = pt_beg + team; pt < pt_end; pt += NTEAM) {
@@ -768,6 +824,10 @@ __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Para
           }
         }
         inverse_norms(ss, inv, dd);
+        if (BULK) {
+          stage_row(cur + t0, acc[0], inv[0], haspd ? sh.rd[t0] * inv[0] : dd[0]);
+          continue;
+        }
 #pragma unroll
         for (int j = 0; j < G; ++j) {
           if (j < cnt) {
@@ -802,6 +862,7 @@ __global__ void __launch_bounds__(THREADS + 32 * PW, MINB) k1_rows_kernel(K1Para
       __syncthreads();  // the window and the per-point scalars are rewritten by the next sub-run
       cur += shb[0].npts;
     }
+    if (BULK && lane == 0) sm100::bulk_wait_group0();  // the staging slots stay allocated until the rows are written
     return;
   }
 
@@ -923,20 +984,22 @@ __global__ void __launch_bounds__(512) center_mean_kernel(const float* __restric
   }
 }
 
-template <int MODE, int NITW, int W, int G, int OUTS, int THREADS, int MINB, int PW = 0>
+template <int MODE, int NITW, int W, int G, int OUTS, int THREADS, int MINB, int PW = 0, int BULK = 0>
 int launch_k1_inst(const K1Params& p, cudaStream_t st) {
   const int C = p.C;
+  // the bulk-store form's staging slots, one per warp: a piece of the hi row (C / BULK + 8 fp16) + of the lo row (C / BULK fp16)
+  const size_t stage = BULK ? (size_t)(THREADS / 32) * (2 * C / (BULK > 0 ? BULK : 1) + 8) * 2 : 0;
   // window bytes per CTA: MINB CTAs per SM share 227 KB (minus ~3 KB static and 1 KB reserved each); the warp-specialised
-  // form holds two windows of 108 KB
-  const int budget = (PW > 0 ? 108 : (MINB >= 3 ? 72 : (MINB == 2 ? 108 : 216))) << 10;
+  // form holds two windows of 108 KB; the bulk-store form gives the window what its staging slots leave of 110 KB
+  const int budget = BULK ? (int)((110 << 10) - stage) : (PW > 0 ? 108 : (MINB >= 3 ? 72 : (MINB == 2 ? 108 : 216))) << 10;
   int nslots = budget / (C * 4);
   if (nslots < 4) nslots = 4;    // C <= 8192: 4 slots = 128 KB, one CTA per SM
   if (nslots > 40) nslots = 40;  // more than any 32-point sub-run can use
-  const size_t smem = (MODE == MV_SAMPLE_ROWS) ? 0 : (size_t)(PW > 0 ? 2 : 1) * nslots * C * 4;
+  const size_t smem = (MODE == MV_SAMPLE_ROWS) ? 0 : (size_t)(PW > 0 ? 2 : 1) * nslots * C * 4 + stage;
   int grid = mv_sm_count() * MINB;
   if (grid > p.n_max) grid = p.n_max;
   if (grid < 1) grid = 1;
-  auto kern = k1_rows_kernel<MODE, NITW, W, G, OUTS, THREADS, MINB, PW>;
+  auto kern = k1_rows_kernel<MODE, NITW, W, G, OUTS, THREADS, MINB, PW, BULK>;
   static size_t opted[MV_MAX_DEVICES];  // per instantiation and device: the attribute belongs to the device function
   size_t& opted_in = opted[mv_device_slot()];
   if (opted_in < (44u << 10)) opted_in = 44 << 10;
@@ -991,6 +1054,21 @@ int launch_k1(const K1Params& p, cudaStream_t st) {
     K1WS_CASE(2048, 4, 4, 4)
     K1WS_CASE(768, 6, 1, 4)
 #undef K1WS_CASE
+  }
+  // C = 3072 bicubic f16c split rows (the NAVI-shaped side): rows leave through bulk stores.  With STG rows (the form
+  // below) the two CTAs of an SM start together, fill their windows (L2 -> SM reads), THEN write their rows (HBM), one
+  // ~17-point sub-run each, and a warp stalls on its own row stores.  Here each warp stages its row in two halves (6160 B
+  // slot: 1536 + 8 hi fp16, 1536 lo fp16) and goes on once a half has been read out of the slot; after its last row it
+  // goes straight to the next sub-run's window fill while the copies drain.  Shared memory per CTA, 2 CTAs per SM (168
+  // registers, 12 warps as before): 6 slots x 6160 B + a 6-column window (72 KB: 12 points per sub-run, ~2 sub-runs per
+  // CTA) = 108 KB + 2.4 KB static.  Measured on B200 at 1000 W (bench.py --k1-only, NAVI-shaped side, same box,
+  // alternating): 33.5-34.0 us vs 35.0-35.2 us with STG rows.  Rejected on the same box: whole-row slots (12 x 12304 B) with one CTA of
+  // 12 warps per SM and a 6-column window, 37.5-38.0 us (the sub-runs of one CTA run strictly one after another); thirds
+  // or quarters of a row with a 7-column window, 35.3-35.4 us.
+  if constexpr (MODE == MV_SAMPLE_BICUBIC_CLAMP) {
+    if (C == 3072 && outs == K1W_OUT_SPLIT && p.fmt16 && !p.out_op32 &&
+        ((reinterpret_cast<uintptr_t>(p.out_bf16) | reinterpret_cast<uintptr_t>(p.out_lo)) & 15) == 0)
+      return launch_k1_inst<MODE, 24, 1, 1, K1W_OUT_SPLIT, 192, 2, 0, 2>(p, st);
   }
   K1W_CASE(768, 6, 1, 4, 128, 3)    // ViT-B
   K1W_CASE(1024, 4, 2, 4, 256, 2)   // ViT-L

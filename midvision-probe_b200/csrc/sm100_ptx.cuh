@@ -1,5 +1,6 @@
 // sm100_ptx.cuh -- thin inline-PTX wrappers for the Blackwell (sm_100a) primitives kernel 2 uses:
-// mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (alloc / mma / commit / ld / fences), clusters.
+// mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (alloc / mma / commit / ld / fences), clusters; plus the 1-D bulk
+// stores kernel 1 writes its C = 3072 rows with.
 // Nothing here is generic: shapes and operand forms are exactly the ones k2_sim.cu issues.
 #pragma once
 
@@ -69,6 +70,19 @@ __device__ __forceinline__ void bulk_load_1d_hint(uint32_t dst, const void* src,
                "l"((uint64_t)src), "r"(bytes), "r"(bar), "l"(policy)
                : "memory");
 }
+// 1-D bulk copy shared -> global (16-byte aligned on both sides, size a multiple of 16), tracked in the issuing thread's
+// bulk groups: that thread commits them and does every wait on them.  Shared memory written through the generic proxy
+// needs fence_proxy_async_smem() by its writers (and a barrier to the issuer) before the copy may read it.
+__device__ __forceinline__ void bulk_store_1d(void* dst, uint32_t src, uint32_t bytes) {
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"((uint64_t)dst), "r"(src), "r"(bytes)
+               : "memory");
+}
+__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// every committed group has read its shared-memory source: the source may be rewritten
+__device__ __forceinline__ void bulk_wait_group_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+// every committed group is complete, writes included
+__device__ __forceinline__ void bulk_wait_group0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tma_prefetch_desc(const void* tmap) {
   asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)tmap) : "memory");
 }
