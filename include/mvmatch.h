@@ -295,6 +295,23 @@ size_t mv_k2_topk_workspace_bytes(int n_max, int m_max, int kp);
 int mv_k2_sim_topk_ld(const void* A, int lda, const void* B, int ldb, int n_max, int m_max, int C, const int32_t* n_dev,
                       const int32_t* m_dev, int dtype, int cluster, int kp, float* row_val, int32_t* row_idx, void* workspace,
                       size_t workspace_bytes, mv_stream_t stream);
+/* ---- mutual matching: kernel 2 with the row top-2 and the column top-2 of one product ------------- */
+/* The same GEMM as mv_k2_sim_top2_ld; its epilogue keeps the row top-2 (row_val / row_idx bit-identical to
+ * mv_k2_sim_top2_ld's on the same operands and cluster form, stream-K off) and, for every column j, the two largest S[:, j]:
+ *   col_val/col_idx (m_max, 2): values descending, ties to the lower row; missing entries (n < 2, rows past *n_dev, columns
+ *                               past *m_dev) = MV_SIM_MASKED / -1
+ *   col_best (m_max)          : the packed arg-max of mv_k2_sim_top2_ld (decode with mv_k2_unpack_col), so mv_k3_ratio_mutual*
+ *                               take it unchanged.
+ * Each CTA writes one {v1, r1, v2, r2} record per (128-row block, column) to the workspace and a merge kernel folds them in
+ * row order: no atomics, the same bits on every run.  The schedule is always tile-granular (mv_k2_set_streamk does not
+ * apply) and the launch is not recorded by mv_k2_profile_*.  Workspace from mv_k2_cols_workspace_bytes (0 for n_max or
+ * m_max <= 0): the row records plus ceil(n_max / 128) * m_max * 16 bytes. */
+size_t mv_k2_cols_workspace_bytes(int n_max, int m_max);
+int mv_k2_sim_top2_cols_ld(const void* A, int lda, const void* B, int ldb, int n_max, int m_max, int C, const int32_t* n_dev,
+                           const int32_t* m_dev, int dtype, int cluster, float* row_val, int32_t* row_idx, float* col_val,
+                           int32_t* col_idx, unsigned long long* col_best, void* workspace, size_t workspace_bytes,
+                           mv_stream_t stream);
+
 /* fp32 re-rank of kp candidates per query (cand (n_max, kp) int32, e.g. row_idx above; -1 = no candidate): the distance of
  * query row Q[i] (n_max, ldq) to every candidate row T[j] (ldt) over C columns --
  *   MV_METRIC_L2SQ     sum (q - t)^2                                  (faiss' squared L2)
@@ -330,6 +347,15 @@ int mv_k3_ratio_mutual_f16c(const uint16_t* A_hi, const uint16_t* A_lo, const ui
                             const unsigned long long* col_best, int ratio_test, float* dists, float* weight, uint8_t* mutual,
                             mv_stream_t stream);
 
+/* The same with a centre on either side: center_A (C floats or NULL) is added to the rebuilt query rows as center_B is to
+ * the target rows (and a rebuilt query row of squared norm below 1e-10 counts as a zero row).  The reverse pass of a mutual
+ * match runs with the roles swapped: the target-role rows (relative to the centre) are then the queries, so
+ * A = target rows with center_A = their centre, B = query-role rows with center_B = NULL. */
+int mv_k3_ratio_mutual_f16c_ab(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* B_hi, const uint16_t* B_lo, int C,
+                               int pitch, const float* center_A, const float* center_B, const int32_t* n_dev, int n_max,
+                               int32_t* row_idx, const unsigned long long* col_best, int ratio_test, float* dists, float* weight,
+                               uint8_t* mutual, mv_stream_t stream);
+
 /* MaskCut's thresholded affinity (evals/models/maskcut_processor.py:103-106): A[i][j] = S[i][j] > tau ? 1 : eps, written as
  * fp32, and count[i] = #{j : S[i][j] > tau} (so that d_i = count + (m - count) * eps is exact in any precision).  S (n, ld_s). */
 int mv_affinity_threshold(const float* S, int n, int m, int ld_s, float tau, float eps, float* A_out, int32_t* count, mv_stream_t stream);
@@ -346,6 +372,17 @@ int mv_cosine_2afc(const float* ref, const float* left, const float* right, int 
 int mv_k3_topk_matches(const float* weight, const int32_t* row_idx, const int32_t* n_dev, int n_max,
                        int num_corr, int32_t* sel_src, int32_t* sel_dst, float* sel_weight, int32_t* k_dev,
                        mv_stream_t stream);
+
+/* Mutual matches from both re-ranked directions of one product: row_idx (n_max, 2) / weight_f (n_max) are the forward
+ * outputs of a mv_k3_ratio_mutual* call (ratio weights or d0 by ratio_test), col_idx (m, 2) / weight_r (m) those of the
+ * reverse call (roles swapped, the column candidates of mv_k2_sim_top2_cols_ld as its row_idx, ratio weights).  Query i is
+ * mutual iff col_idx[row_idx[i][0]][0] == i; mutual[i] (optional) receives that flag, weight[i] the selection weight
+ * min(weight_f[i], weight_r[row_idx[i][0]]) with ratio_test, weight_f[i] without, -inf for a query that is not mutual.
+ * Then the k = min(num_corr, #mutual) largest weights, sorted descending (ties: lower row): sel_* have num_corr entries,
+ * *k_dev receives k (it never leaves the device).  num_corr <= 16384, n_max <= 2^20. */
+int mv_k3_mutual_select(const int32_t* row_idx, const float* weight_f, const int32_t* col_idx, const float* weight_r,
+                        const int32_t* n_dev, int n_max, int ratio_test, int num_corr, float* weight, uint8_t* mutual,
+                        int32_t* sel_src, int32_t* sel_dst, float* sel_weight, int32_t* k_dev, mv_stream_t stream);
 
 /* Scoring of the selected matches (callers: evaluate_navi_correspondence.py:183-212,
  * render_scannet_correspondence.py:211-217, :253-264, :131-147):

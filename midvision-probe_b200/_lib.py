@@ -54,11 +54,15 @@ PROTOTYPES = {
     "mv_k2_unpack_col": (c_int, [P, c_int, P, P, P]),
     "mv_k2_topk_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "mv_k2_sim_topk_ld": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, P, P, c_int, c_int, c_int, P, P, P, c_size_t, P]),
+    "mv_k2_cols_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "mv_k2_sim_top2_cols_ld": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, P, P, c_int, c_int, P, P, P, P, P, P, c_size_t, P]),
     "mv_knn_rerank": (c_int, [P, c_int, P, c_int, c_int, P, c_int, P, c_int, c_int, c_int, P, P, P]),
     "mv_k3_ratio_mutual": (c_int, [P, P, c_int, P, c_int, P, P, c_int, P, P, P, P]),
     "mv_k3_ratio_mutual_split": (c_int, [P, P, P, P, c_int, P, c_int, P, P, c_int, P, P, P, P]),
     "mv_k3_ratio_mutual_f16c": (c_int, [P, P, P, P, c_int, c_int, P, P, c_int, P, P, c_int, P, P, P, P]),
+    "mv_k3_ratio_mutual_f16c_ab": (c_int, [P, P, P, P, c_int, c_int, P, P, P, c_int, P, P, c_int, P, P, P, P]),
     "mv_k3_topk_matches": (c_int, [P, P, P, c_int, c_int, P, P, P, P, P]),
+    "mv_k3_mutual_select": (c_int, [P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, P, P, P]),
     "mv_k3_score": (c_int, [P, P, P, c_int, P, P, P, P, P, P, c_int, P, c_int, P, P, P, P, P, P]),
     "mv_gather_rows": (c_int, [P, c_int, P, P, c_int, P, P]),
     "mv_pack_matches": (c_int, [P, P, P, P, c_int, P, P, P, P, P, P, P, P]),
@@ -92,8 +96,8 @@ _lib = None
 # kernels launched per entry point (for bench.py's gpu_launches claim); memsets are not counted
 KERNELS_PER_CALL = {
     "mv_chw_to_hwc": 1, "mv_feat_to_hwc_f32": 1, "mv_compact_valid": 1, "mv_geom_backproject": 1, "mv_geom_project_coords": 1,
-    "mv_geom_grid_coords": 1, "mv_geom_keypoint_coords": 1, "mv_k1_sample_normalize": 1, "mv_k1_sample_f16c": 1, "mv_k1_sample_tf32c": 1, "mv_rows_center": 2, "mv_rows_dot": 1, "mv_rank_of_valid": 1, "mv_k1_grid_f16c": 1, "mv_lr_unit_rows": 1, "mv_lr_gram_exact": 2, "mv_lr_build_query": 1, "mv_lr_build_target": 1, "mv_k3_ratio_mutual_lr": 1, "mv_k2_sim_top2": 2, "mv_k2_sim_top2_ld": 2, "mv_k2_affinity": 2, "mv_k2_sim_topk_ld": 2, "mv_knn_rerank": 1, "mv_affinity_threshold": 1, "mv_cosine_2afc": 1,
-    "mv_k2_unpack_col": 1, "mv_k3_ratio_mutual": 1, "mv_k3_ratio_mutual_split": 1, "mv_k3_ratio_mutual_f16c": 1, "mv_k3_topk_matches": 1, "mv_k3_score": 1, "mv_gather_rows": 1,
+    "mv_geom_grid_coords": 1, "mv_geom_keypoint_coords": 1, "mv_k1_sample_normalize": 1, "mv_k1_sample_f16c": 1, "mv_k1_sample_tf32c": 1, "mv_rows_center": 2, "mv_rows_dot": 1, "mv_rank_of_valid": 1, "mv_k1_grid_f16c": 1, "mv_lr_unit_rows": 1, "mv_lr_gram_exact": 2, "mv_lr_build_query": 1, "mv_lr_build_target": 1, "mv_k3_ratio_mutual_lr": 1, "mv_k2_sim_top2": 2, "mv_k2_sim_top2_ld": 2, "mv_k2_affinity": 2, "mv_k2_sim_topk_ld": 2, "mv_k2_sim_top2_cols_ld": 3, "mv_knn_rerank": 1, "mv_affinity_threshold": 1, "mv_cosine_2afc": 1,
+    "mv_k2_unpack_col": 1, "mv_k3_ratio_mutual": 1, "mv_k3_ratio_mutual_split": 1, "mv_k3_ratio_mutual_f16c": 1, "mv_k3_ratio_mutual_f16c_ab": 1, "mv_k3_mutual_select": 3, "mv_k3_topk_matches": 1, "mv_k3_score": 1, "mv_gather_rows": 1,
     "mv_pack_matches": 1, "mv_argmax_rows": 1, "mv_k3_spair_errors": 1, "mv_spair_match_batch": 1, "mv_spair_match_batch_typed": 1,
     "mv_spair_match_batch_tiled": 4,  # the tiled form (h*w > 256); otherwise it is the one launch of _typed
 }

@@ -25,7 +25,7 @@ __all__ = [
     "faiss_knn", "knn_points", "get_correspondences_ratio_test", "calculate_ratio_test", "get_topk_matches",
     "get_grid", "grid_to_pointcloud", "sample_pointcloud_features", "argmax_2d", "project_3dto2d", "error_auc",
     "estimate_correspondence_depth", "estimate_correspondence_xyz", "compute_binned_performance",
-    "set_match_precision", "match_rows", "prepare_depth_side", "prepare_xyz_side", "MatchResult",
+    "set_match_precision", "match_rows", "prepare_depth_side", "prepare_xyz_side", "MatchResult", "get_mutual_correspondences",
 ]
 
 # operand type of kernel 2:
@@ -215,9 +215,21 @@ def _row_format(rows=None):
 
 
 class MatchResult:
-    """Device-side outputs of one directional match (kernels 2 + 3)."""
+    """Device-side outputs of one directional match (kernels 2 + 3).
 
-    __slots__ = ("k", "k_dev", "sel_src", "sel_dst", "sel_weight", "mutual", "row_idx", "dists", "weight", "col_best")
+    k is the selection's length on the host (min(num_corr, n)); k_dev its live length on the device.  mutual is the
+    one-sided flag of kernel 3 (the query is the tensor-core arg-max of its best column, col_best).  A mutual match
+    (match_rows(..., mutual=True)) also carries the reverse direction of the same product: col_idx (m, 2) the re-ranked
+    two best rows of every column, col_dists / col_weight their fp32 distances and ratio weights, mutual_rr the two-sided
+    flag on the re-ranked candidates and mutual_weight the selection weight (-inf where not mutual); its selection holds
+    only mutual queries, so k_dev may be below k."""
+
+    __slots__ = ("k", "k_dev", "sel_src", "sel_dst", "sel_weight", "mutual", "row_idx", "dists", "weight", "col_best",
+                 "col_idx", "col_dists", "col_weight", "mutual_rr", "mutual_weight")
+
+    def __init__(self):
+        for name in self.__slots__:
+            setattr(self, name, None)
 
 
 def _k2_operands(A16, A32, B16, B32, C):
@@ -233,7 +245,7 @@ def _k2_operands(A16, A32, B16, B32, C):
 
 
 def match_rows(A16, A32, B16, B32, n, m, num_corr, ratio_test=True, n_dev=None, m_dev=None, want_topk=True, run_k3=True,
-               A_lo=None, B_lo=None, center_B=None, C=None, proposal=None):
+               A_lo=None, B_lo=None, center_B=None, C=None, proposal=None, mutual=False):
     """kernel 2 + kernel 3 on prepared rows.
 
     A16/B16: (n, C)/(m, C) bf16 rows or (n, pitch)/(m, pitch) fp16 f16c rows (query / target role; None when the
@@ -244,6 +256,9 @@ def match_rows(A16, A32, B16, B32, n, m, num_corr, ratio_test=True, n_dev=None, 
     n, m are the live counts when n_dev/m_dev are None, otherwise upper bounds.
     proposal: (A_op, B_op, K) fp16 operand rows of _lowrank_operands -- kernel 2 then ranks their product over K columns
     (the same cosine similarities in the basis of the source pixels) while kernel 3 still reads the exact rows.
+    mutual: kernel 2 also keeps every column's two best rows (mv_k2_sim_top2_cols_ld), kernel 3 re-ranks them with the roles
+    swapped, and the selection is the top num_corr of the mutual queries by min(forward, reverse) ratio weight
+    (mv_k3_mutual_select; MatchResult).
     """
     ref = A32 if A32 is not None else A16
     dev = ref.device
@@ -259,8 +274,6 @@ def match_rows(A16, A32, B16, B32, n, m, num_corr, ratio_test=True, n_dev=None, 
     row_idx = _empty((n, 2), torch.int32, dev)
     col_best = _empty((m,), torch.int64, dev)
     lib = L.load()
-    ws_bytes = lib.mv_k2_workspace_bytes(n, m)
-    ws = _empty((ws_bytes,), torch.uint8, dev)
     if split:
         C = A_lo.shape[1]
     k2_A, k2_B, Ck, k2_dtype = _k2_operands(A16, A32, B16, B32, C)
@@ -268,42 +281,89 @@ def match_rows(A16, A32, B16, B32, n, m, num_corr, ratio_test=True, n_dev=None, 
     if proposal is not None:
         k2_A, k2_B, Ck = proposal
         k2_dtype = L.MV_DTYPE_F16
-    prof = _PROFILE.get("k2_events")
-    if prof is not None:
-        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        ev0.record()
-    L.call("mv_k2_sim_top2_ld", L.ptr(k2_A), k2_A.shape[1], L.ptr(k2_B), k2_B.shape[1], n, m, Ck, L.ptr(n_dev), L.ptr(m_dev),
-           k2_dtype, _CFG["cluster"], L.ptr(row_val),
-           L.ptr(row_idx), L.ptr(col_best), L.ptr(ws), c_size_t(ws_bytes), st)
-    if prof is not None:
-        ev1.record()
-        prof.append((ev0, ev1, (n, m, Ck, n_dev, m_dev)))
+    if mutual:
+        res.col_idx = _k2_cols(k2_A, k2_B, n, m, Ck, n_dev, m_dev, k2_dtype, row_val, row_idx, col_best)
+    else:
+        ws_bytes = lib.mv_k2_workspace_bytes(n, m)
+        ws = _empty((ws_bytes,), torch.uint8, dev)
+        prof = _PROFILE.get("k2_events")
+        if prof is not None:
+            ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            ev0.record()
+        L.call("mv_k2_sim_top2_ld", L.ptr(k2_A), k2_A.shape[1], L.ptr(k2_B), k2_B.shape[1], n, m, Ck, L.ptr(n_dev), L.ptr(m_dev),
+               k2_dtype, _CFG["cluster"], L.ptr(row_val),
+               L.ptr(row_idx), L.ptr(col_best), L.ptr(ws), c_size_t(ws_bytes), st)
+        if prof is not None:
+            ev1.record()
+            prof.append((ev0, ev1, (n, m, Ck, n_dev, m_dev)))
     res.row_idx, res.col_best = row_idx, col_best
     if not run_k3:  # raw kernel-2 neighbours (inner-product order), no cosine re-ranking
         return res
     dists = _empty((n, 2), torch.float32, dev)
     weight = _empty((n,), torch.float32, dev)
-    mutual = _empty((n,), torch.uint8, dev)
+    mflag = _empty((n,), torch.uint8, dev)
     if split and f16:
         L.call("mv_k3_ratio_mutual_f16c", L.ptr(A16), L.ptr(A_lo), L.ptr(B16), L.ptr(B_lo), C, ld, L.ptr(center_B), L.ptr(n_dev), n,
-               L.ptr(row_idx), L.ptr(col_best), int(ratio_test), L.ptr(dists), L.ptr(weight), L.ptr(mutual), st)
+               L.ptr(row_idx), L.ptr(col_best), int(ratio_test), L.ptr(dists), L.ptr(weight), L.ptr(mflag), st)
     elif split:
         L.call("mv_k3_ratio_mutual_split", L.ptr(A16), L.ptr(A_lo), L.ptr(B16), L.ptr(B_lo), C, L.ptr(n_dev), n,
-               L.ptr(row_idx), L.ptr(col_best), int(ratio_test), L.ptr(dists), L.ptr(weight), L.ptr(mutual), st)
+               L.ptr(row_idx), L.ptr(col_best), int(ratio_test), L.ptr(dists), L.ptr(weight), L.ptr(mflag), st)
     else:
         L.call("mv_k3_ratio_mutual", L.ptr(A32), L.ptr(B32), C, L.ptr(n_dev), n, L.ptr(row_idx), L.ptr(col_best),
-               int(ratio_test), L.ptr(dists), L.ptr(weight), L.ptr(mutual), st)
-    res.row_idx, res.dists, res.weight, res.mutual, res.col_best = row_idx, dists, weight, mutual, col_best
+               int(ratio_test), L.ptr(dists), L.ptr(weight), L.ptr(mflag), st)
+    res.row_idx, res.dists, res.weight, res.mutual, res.col_best = row_idx, dists, weight, mflag, col_best
+    if res.col_idx is not None:
+        # the reverse direction on the same rows: targets are the queries now (an f16c target row carries its centre)
+        cidx, cd, cw = res.col_idx, _empty((m, 2), torch.float32, dev), _empty((m,), torch.float32, dev)
+        if split and f16:
+            L.call("mv_k3_ratio_mutual_f16c_ab", L.ptr(B16), L.ptr(B_lo), L.ptr(A16), L.ptr(A_lo), C, ld, L.ptr(center_B), None,
+                   L.ptr(m_dev), m, L.ptr(cidx), None, 1, L.ptr(cd), L.ptr(cw), None, st)
+        elif split:
+            L.call("mv_k3_ratio_mutual_split", L.ptr(B16), L.ptr(B_lo), L.ptr(A16), L.ptr(A_lo), C, L.ptr(m_dev), m,
+                   L.ptr(cidx), None, 1, L.ptr(cd), L.ptr(cw), None, st)
+        else:
+            L.call("mv_k3_ratio_mutual", L.ptr(B32), L.ptr(A32), C, L.ptr(m_dev), m, L.ptr(cidx), None, 1, L.ptr(cd), L.ptr(cw),
+                   None, st)
+        res.col_dists, res.col_weight = cd, cw
     if want_topk:
-        k = min(int(num_corr), n)
-        res.k = k
-        res.sel_src = _empty((max(k, 1),), torch.int32, dev)
-        res.sel_dst = _empty((max(k, 1),), torch.int32, dev)
-        res.sel_weight = _empty((max(k, 1),), torch.float32, dev)
-        res.k_dev = _empty((1,), torch.int32, dev)
-        L.call("mv_k3_topk_matches", L.ptr(weight), L.ptr(row_idx), L.ptr(n_dev), n, k, L.ptr(res.sel_src),
-               L.ptr(res.sel_dst), L.ptr(res.sel_weight), L.ptr(res.k_dev), st)
+        _select(res, n, num_corr, ratio_test, n_dev)
     return res
+
+
+def _k2_cols(k2_A, k2_B, n, m, Ck, n_dev, m_dev, k2_dtype, row_val, row_idx, col_best):
+    """kernel 2 with the row top-2 and the column top-2 (mv_k2_sim_top2_cols_ld): fills row_val / row_idx / col_best like
+    mv_k2_sim_top2_ld and returns the (m, 2) int32 column candidates."""
+    dev = row_val.device
+    col_val = _empty((m, 2), torch.float32, dev)
+    col_idx = _empty((m, 2), torch.int32, dev)
+    ws_bytes = L.load().mv_k2_cols_workspace_bytes(n, m)
+    ws = _empty((ws_bytes,), torch.uint8, dev)
+    L.call("mv_k2_sim_top2_cols_ld", L.ptr(k2_A), k2_A.shape[1], L.ptr(k2_B), k2_B.shape[1], n, m, Ck, L.ptr(n_dev), L.ptr(m_dev),
+           k2_dtype, _CFG["cluster"], L.ptr(row_val), L.ptr(row_idx), L.ptr(col_val), L.ptr(col_idx), L.ptr(col_best), L.ptr(ws),
+           c_size_t(ws_bytes), _stream())
+    return col_idx
+
+
+def _select(res, n, num_corr, ratio_test, n_dev):
+    """the top-k of a match: the num_corr largest weights, or, with the reverse direction present, the num_corr largest
+    min(forward, reverse) weights of the mutual queries (k_dev = min(num_corr, #mutual))."""
+    dev = res.weight.device
+    st = _stream()
+    k = min(int(num_corr), n)
+    res.k = k
+    res.sel_src = _empty((max(k, 1),), torch.int32, dev)
+    res.sel_dst = _empty((max(k, 1),), torch.int32, dev)
+    res.sel_weight = _empty((max(k, 1),), torch.float32, dev)
+    res.k_dev = _empty((1,), torch.int32, dev)
+    if res.col_idx is None:
+        L.call("mv_k3_topk_matches", L.ptr(res.weight), L.ptr(res.row_idx), L.ptr(n_dev), n, k, L.ptr(res.sel_src),
+               L.ptr(res.sel_dst), L.ptr(res.sel_weight), L.ptr(res.k_dev), st)
+        return
+    res.mutual_weight = _empty((max(n, 1),), torch.float32, dev)
+    res.mutual_rr = _empty((max(n, 1),), torch.uint8, dev)
+    L.call("mv_k3_mutual_select", L.ptr(res.row_idx), L.ptr(res.weight), L.ptr(res.col_idx), L.ptr(res.col_weight), L.ptr(n_dev),
+           n, int(bool(ratio_test)), k, L.ptr(res.mutual_weight), L.ptr(res.mutual_rr), L.ptr(res.sel_src), L.ptr(res.sel_dst),
+           L.ptr(res.sel_weight), L.ptr(res.k_dev), st)
 
 
 def _gather(src, idx, k, k_dev=None):
@@ -547,6 +607,39 @@ def get_correspondences_ratio_test(P1_F, P2_F, num_corres, metric="cosine", bidi
     return idx1.to(in_dev), idx2.to(in_dev), w.to(in_dev)
 
 
+def _check_mutual_args(num_corres, ratio_test, mutual=False):
+    """type checks of the mutual-matching keywords (before any device work)."""
+    for name, v in (("ratio_test", ratio_test), ("mutual", mutual)):
+        if not isinstance(v, bool):
+            raise TypeError(f"{name} must be a bool, not {type(v).__name__}")
+    if isinstance(num_corres, bool) or not isinstance(num_corres, int) or num_corres < 0:
+        raise ValueError(f"num_corres must be a non-negative int, not {num_corres!r}")
+
+
+def get_mutual_correspondences(P1_F, P2_F, num_corres, ratio_test=True):
+    """(idx1, idx2, weight): mutual nearest neighbours under the cosine metric with a two-sided ratio test, from ONE
+    similarity product (kernel 2 keeps every row's and every column's two best, mv_k2_sim_top2_cols_ld).
+
+    Both directions are re-ranked in fp32 (1 - cos): query i matches j(i), its best target, and target j has its best
+    query i(j).  i is mutual iff i(j(i)) == i.  With ratio_test its weight is min(1 - d0/d1 forward, 1 - d0/d1 reverse at
+    j(i)); without, the forward d0 (the reference's ratio_test=False rule).  Returns the k = min(num_corres, #mutual)
+    largest weights among the mutual queries, sorted descending, ties to the lower query index; k may be below
+    num_corres.  Inputs on the CPU or a CUDA device, (N, C) features with C % 8 == 0; results on P1_F's device."""
+    _check_mutual_args(num_corres, ratio_test)
+    if P1_F.dim() != 2 or P2_F.dim() != 2 or P1_F.shape[1] != P2_F.shape[1]:
+        raise ValueError(f"get_mutual_correspondences: (N, C) features of equal C expected, got {tuple(P1_F.shape)} and {tuple(P2_F.shape)}")
+    _check_C(P1_F.shape[1])
+    n, m = P1_F.shape[0], P2_F.shape[0]
+    if n < 2 or m < 2:  # two candidates on each side
+        raise ValueError(f"get_mutual_correspondences: too few points to match ({n} vs {m})")
+    dev = _device()
+    in_dev = P1_F.device
+    (A16, A32), (B16, B32), mu = _rows_pair(P1_F, P2_F, dev)
+    r = match_rows(A16, A32, B16, B32, n, m, num_corres, ratio_test, center_B=mu, mutual=True)
+    k = int(r.k_dev.item())
+    return r.sel_src[:k].long().to(in_dev), r.sel_dst[:k].long().to(in_dev), r.sel_weight[:k].to(in_dev)
+
+
 def _ratio_test_euclidean(P1_F, P2_F, num_corres, bidirectional, ratio_test):
     """the metric="euclidean" branch (no call site in the reference; correspondence.py:70-102 followed literally):
     exact L2 2-NN (knn_points) -> ratio weights -> top-k through the library's selection kernel."""
@@ -751,9 +844,10 @@ def _lowrank_operands(s0, s1, n, m, n_dev, m_dev, exact=False):
     return A_op, B_op, hwp + 8
 
 
-def _match_lowrank_exact(s0, s1, n, m, num_corr, ratio_test=True, n_dev=None, m_dev=None, want_topk=True):
+def _match_lowrank_exact(s0, s1, n, m, num_corr, ratio_test=True, n_dev=None, m_dev=None, want_topk=True, mutual=False):
     """one directional match WITHOUT interpolated rows: kernel 2 on the low-rank operands, kernel 3's distances from the exact
-    Gram matrix of the source pixels (mv_k3_ratio_mutual_lr), then the usual top-k.  Same MatchResult as match_rows."""
+    Gram matrix of the source pixels (mv_k3_ratio_mutual_lr), then the usual top-k.  Same MatchResult as match_rows (mutual:
+    see there; the reverse pass reads the other orientation of the same Gram matrix)."""
     dev = s0.src.device
     st = _stream()
     A_op, B_op, Ck, x = _lowrank_operands(s0, s1, n, m, n_dev, m_dev, exact=True)
@@ -762,48 +856,49 @@ def _match_lowrank_exact(s0, s1, n, m, num_corr, ratio_test=True, n_dev=None, m_
     row_val = _empty((n, 2), torch.float32, dev)
     row_idx = _empty((n, 2), torch.int32, dev)
     col_best = _empty((m,), torch.int64, dev)
-    ws_bytes = L.load().mv_k2_workspace_bytes(n, m)
-    ws = _empty((ws_bytes,), torch.uint8, dev)
-    prof = _PROFILE.get("k2_events")
-    if prof is not None:
-        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        ev0.record()
-    L.call("mv_k2_sim_top2_ld", L.ptr(A_op), A_op.shape[1], L.ptr(B_op), B_op.shape[1], n, m, Ck, L.ptr(n_dev), L.ptr(m_dev),
-           L.MV_DTYPE_F16, _CFG["cluster"], L.ptr(row_val), L.ptr(row_idx), L.ptr(col_best), L.ptr(ws), c_size_t(ws_bytes), st)
-    if prof is not None:
-        ev1.record()
-        prof.append((ev0, ev1, (n, m, Ck, n_dev, m_dev)))
+    if mutual:
+        res.col_idx = _k2_cols(A_op, B_op, n, m, Ck, n_dev, m_dev, L.MV_DTYPE_F16, row_val, row_idx, col_best)
+    else:
+        ws_bytes = L.load().mv_k2_workspace_bytes(n, m)
+        ws = _empty((ws_bytes,), torch.uint8, dev)
+        prof = _PROFILE.get("k2_events")
+        if prof is not None:
+            ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            ev0.record()
+        L.call("mv_k2_sim_top2_ld", L.ptr(A_op), A_op.shape[1], L.ptr(B_op), B_op.shape[1], n, m, Ck, L.ptr(n_dev), L.ptr(m_dev),
+               L.MV_DTYPE_F16, _CFG["cluster"], L.ptr(row_val), L.ptr(row_idx), L.ptr(col_best), L.ptr(ws), c_size_t(ws_bytes), st)
+        if prof is not None:
+            ev1.record()
+            prof.append((ev0, ev1, (n, m, Ck, n_dev, m_dev)))
     dists = _empty((n, 2), torch.float32, dev)
     weight = _empty((n,), torch.float32, dev)
-    mutual = _empty((n,), torch.uint8, dev)
+    mflag = _empty((n,), torch.uint8, dev)
     L.call("mv_k3_ratio_mutual_lr", s0.mode, L.ptr(s0.coords), L.ptr(s1.coords), L.ptr(x["inv0"]), L.ptr(x["inv1"]), L.ptr(x["G"]),
            x["ld"], 0, x["off_t"], h, w, L.ptr(n_dev), n, L.ptr(row_idx), L.ptr(col_best), int(ratio_test), L.ptr(dists),
-           L.ptr(weight), L.ptr(mutual), st)
-    res.row_idx, res.dists, res.weight, res.mutual, res.col_best = row_idx, dists, weight, mutual, col_best
+           L.ptr(weight), L.ptr(mflag), st)
+    res.row_idx, res.dists, res.weight, res.mutual, res.col_best = row_idx, dists, weight, mflag, col_best
+    if res.col_idx is not None:  # the reverse pass: image 1's points are the queries
+        res.col_dists, res.col_weight = _empty((m, 2), torch.float32, dev), _empty((m,), torch.float32, dev)
+        L.call("mv_k3_ratio_mutual_lr", s1.mode, L.ptr(s1.coords), L.ptr(s0.coords), L.ptr(x["inv1"]), L.ptr(x["inv0"]), L.ptr(x["G"]),
+               x["ld"], x["off_t"], 0, h, w, L.ptr(m_dev), m, L.ptr(res.col_idx), None, 1, L.ptr(res.col_dists),
+               L.ptr(res.col_weight), None, st)
     if want_topk:
-        k = min(int(num_corr), n)
-        res.k = k
-        res.sel_src = _empty((max(k, 1),), torch.int32, dev)
-        res.sel_dst = _empty((max(k, 1),), torch.int32, dev)
-        res.sel_weight = _empty((max(k, 1),), torch.float32, dev)
-        res.k_dev = _empty((1,), torch.int32, dev)
-        L.call("mv_k3_topk_matches", L.ptr(weight), L.ptr(row_idx), L.ptr(n_dev), n, k, L.ptr(res.sel_src),
-               L.ptr(res.sel_dst), L.ptr(res.sel_weight), L.ptr(res.k_dev), st)
+        _select(res, n, num_corr, ratio_test, n_dev)
     return res
 
 
-def _match_sides(s0, s1, n0, n1, num_corr, ratio_test=True, n_dev=None, m_dev=None):
-    """s0 = query side, s1 = target side (prepared with the matching f16c roles, see _pair_maps)."""
+def _match_sides(s0, s1, n0, n1, num_corr, ratio_test=True, n_dev=None, m_dev=None, mutual=False):
+    """s0 = query side, s1 = target side (prepared with the matching f16c roles, see _pair_maps).  mutual: see match_rows."""
     proposal = None
     if s0.rows16 is None and s0.rows32 is None:  # prepared without rows (want_rows=False): the exact low-rank route
         if not (s0.fshape == s1.fshape and s0.mode == s1.mode and s1.rows16 is None and s1.rows32 is None):
             raise ValueError("sides prepared without rows need equal feature shapes and sampling modes")
-        return _match_lowrank_exact(s0, s1, n0, n1, num_corr, ratio_test, n_dev=n_dev, m_dev=m_dev)
+        return _match_lowrank_exact(s0, s1, n0, n1, num_corr, ratio_test, n_dev=n_dev, m_dev=m_dev, mutual=mutual)
     if (s0.src is not None and s1.src is not None and s0.fshape == s1.fshape and s0.mode == s1.mode and n0 > 0 and n1 > 0
             and s0.rows_lo is not None and lowrank_applies(*s0.fshape, n0, n1, s0.mode)):
         proposal = _lowrank_operands(s0, s1, n0, n1, n_dev, m_dev)
     return match_rows(s0.rows16, s0.rows32, s1.rows16, s1.rows32, n0, n1, num_corr, ratio_test, n_dev=n_dev, m_dev=m_dev,
-                      A_lo=s0.rows_lo, B_lo=s1.rows_lo, center_B=s1.center, proposal=proposal)
+                      A_lo=s0.rows_lo, B_lo=s1.rows_lo, center_B=s1.center, proposal=proposal, mutual=mutual)
 
 
 def _pair_maps(feat_0, feat_1, dev, grid_pixels=0, mode=None):
@@ -1015,7 +1110,7 @@ def _host_mat(M):
     return L.host_floats(M.detach().float().cpu().reshape(-1).tolist())
 
 
-def _graphed_helper(kind, feat_0, feat_1, grid_0, grid_1, num_corr, ratio_test, K=None):
+def _graphed_helper(kind, feat_0, feat_1, grid_0, grid_1, num_corr, ratio_test, K=None, mutual=False):
     """Fast path of the two dense helpers: the whole pair (kernels 1-3 + the gathers of the return tuple) is one
     cached CUDA graph; a call is 4 copies into static buffers (uploads for host tensors), one replay and ONE
     packed read-back (results + the three live counts), i.e. a single host sync.  Results are returned on the
@@ -1031,7 +1126,7 @@ def _graphed_helper(kind, feat_0, feat_1, grid_0, grid_1, num_corr, ratio_test, 
     split = on_host and bool(_CFG["helper_split"])
     # the intrinsics are NOT part of the key: they live in device memory and are refreshed per call (gm.load)
     key = (on_host, split, kind, tuple(feat_0.shape), tuple(grid_0.shape), int(num_corr), bool(ratio_test), _CFG["dtype"], _CFG["cluster"], _CFG["rows"], _CFG["k1_grid"], _CFG["lowrank"], _CFG["lowrank_k3"], fdt,
-           dev.index, layout)
+           dev.index, layout, mutual)
     gm = _HELPER_GRAPHS.get(key)
     if gm is None:
         import importlib
@@ -1041,7 +1136,7 @@ def _graphed_helper(kind, feat_0, feat_1, grid_0, grid_1, num_corr, ratio_test, 
             _HELPER_GRAPHS.pop(next(iter(_HELPER_GRAPHS)))
         gm = ev.GraphedPairMatcher(kind, tuple(feat_0.shape), tuple(grid_0.shape), num_corr, K=K, device=dev,
                                    ratio_test=ratio_test, with_outputs=True, feat_layout=layout, feat_dtype=fdt,
-                                   split=split).capture()
+                                   split=split, mutual=mutual).capture()
         _HELPER_GRAPHS[key] = gm
     if gm.split:  # host caller: image 1 uploads first and its side runs while image 0 uploads
         gm.load_and_replay_split(feat_0, feat_1, grid_0, grid_1, K=K)
@@ -1068,12 +1163,16 @@ def _graphed_helper(kind, feat_0, feat_1, grid_0, grid_1, num_corr, ratio_test, 
     return tuple(out)
 
 
-def estimate_correspondence_depth(feat_0, feat_1, depth_0, depth_1, K, num_corr=500):
-    """(corr_xyz0 (k, 3), corr_xyz1 (k, 3), corr_dist (k,)).  correspondence.py:218-232."""
+def estimate_correspondence_depth(feat_0, feat_1, depth_0, depth_1, K, num_corr=500, mutual=False):
+    """(corr_xyz0 (k, 3), corr_xyz1 (k, 3), corr_dist (k,)).  correspondence.py:218-232.
+    mutual=True: only mutual matches, weighted by the two-sided ratio test (get_mutual_correspondences), on whichever
+    route the call takes; k = min(num_corr, #mutual) may then be below num_corr."""
+    if mutual is not False:
+        _check_mutual_args(num_corr, True, mutual)
     dev = _device()
     in_dev = feat_0.device
     if _CFG["helper_graphs"]:
-        out = _graphed_helper("depth", feat_0, feat_1, depth_0, depth_1, num_corr, True, K=K)
+        out = _graphed_helper("depth", feat_0, feat_1, depth_0, depth_1, num_corr, True, K=K, mutual=mutual)
         if out is not None:
             return out
     Kc = K.detach().float().cpu()
@@ -1095,17 +1194,21 @@ def estimate_correspondence_depth(feat_0, feat_1, depth_0, depth_1, K, num_corr=
     with torch.cuda.stream(side):
         s1 = _finish_depth(fm1, d1, Kh, a1, n1, True, **kw1)
     _join_side(side, dev, s1)
-    r = _match_sides(s0, s1, n0, n1, num_corr)
-    k = r.k
+    r = _match_sides(s0, s1, n0, n1, num_corr, mutual=mutual)
+    k = int(r.k_dev.item()) if mutual else r.k
     return _return_packed([_gather(s0.xyz, r.sel_src, k), _gather(s1.xyz, r.sel_dst, k), r.sel_weight[:k]], in_dev)
 
 
-def estimate_correspondence_xyz(feat_0, feat_1, xyz_grid_0, xyz_grid_1, num_corr=500, ratio_test=True):
-    """(c_xyz0, c_xyz1, c_dist, c_uv0, c_uv1).  correspondence.py:235-263."""
+def estimate_correspondence_xyz(feat_0, feat_1, xyz_grid_0, xyz_grid_1, num_corr=500, ratio_test=True, mutual=False):
+    """(c_xyz0, c_xyz1, c_dist, c_uv0, c_uv1).  correspondence.py:235-263.
+    mutual=True: only mutual matches, weighted by the two-sided ratio test (get_mutual_correspondences), on whichever
+    route the call takes; k = min(num_corr, #mutual) may then be below num_corr."""
+    if mutual is not False:  # the default call keeps today's argument handling exactly
+        _check_mutual_args(num_corr, ratio_test, mutual)
     dev = _device()
     in_dev = feat_0.device
     if _CFG["helper_graphs"]:
-        out = _graphed_helper("xyz", feat_0, feat_1, xyz_grid_0, xyz_grid_1, num_corr, ratio_test)
+        out = _graphed_helper("xyz", feat_0, feat_1, xyz_grid_0, xyz_grid_1, num_corr, ratio_test, mutual=mutual)
         if out is not None:
             return out
     _check_C(feat_0.shape[0])
@@ -1123,7 +1226,7 @@ def estimate_correspondence_xyz(feat_0, feat_1, xyz_grid_0, xyz_grid_1, num_corr
     with torch.cuda.stream(side):
         s1 = _finish_xyz(fm1, g1, a1, n1, True, **kw1)
     _join_side(side, dev, s1)
-    r = _match_sides(s0, s1, n0, n1, num_corr, ratio_test)
-    k = r.k
+    r = _match_sides(s0, s1, n0, n1, num_corr, ratio_test, mutual=mutual)
+    k = int(r.k_dev.item()) if mutual else r.k
     return _return_packed([_gather(s0.xyz, r.sel_src, k), _gather(s1.xyz, r.sel_dst, k), r.sel_weight[:k],
                            _gather(s0.uv, r.sel_src, k), _gather(s1.uv, r.sel_dst, k)], in_dev)

@@ -33,6 +33,12 @@
 // compare-and-shift -- and does no column work.  A chunk is only looked at when its maximum beats the list's last entry;
 // then its best column is inserted and knocked out until none beats it.  Partial lists go to the workspace like the
 // top-2 records and k2_merge_topk_kernel folds them into (n_max, KP) outputs.  Stream-K is never used there.
+//
+// Mutual matching reads the column top-2 from the same product (k2_sim_top2_cols_kernel, mv_k2_sim_top2_cols_ld, KP ==
+// KP_COLS): the top-2 epilogue with its row work unchanged, and per column a second warp max after the winning lane is
+// masked; the four lane-quarter warps are folded in shared memory into one {v1, r1, v2, r2} record per (128-row block,
+// column), which goes to the workspace -- no atomics, so the bits do not depend on the CTA order.  k2_merge_cols_kernel
+// folds the row blocks in ascending order (ties: lower row) and also writes the packed col_best.  No stream-K either.
 #include <cuda.h>
 
 #include <stdlib.h>
@@ -72,15 +78,22 @@ constexpr int EPI_CW = 16;        // columns per TMEM read (chunk)
 constexpr int PART_COLS = BN / EPI_PARTS, PART_CHUNKS = PART_COLS / EPI_CW;
 constexpr int EPI_WARP0 = 4;
 constexpr int COL_SMEM_BYTES = 2 * 4 * BN * 8;  // [2 buffers][4 warps][256 columns] (max bits, ballot)
-// Epilogue shape of a kernel variant: KP == 0 is the top-2 + column arg-max epilogue above; KP > 0 the row top-KP one.
+constexpr int KP_COLS = -1;  // epilogue selector: the top-2 epilogue with the column top-2 instead of the column arg-max
+// Epilogue shape of a kernel variant: KP == 0 is the top-2 + column arg-max epilogue above; KP > 0 the row top-KP one;
+// KP == KP_COLS the top-2 one with 16-byte column slots (v1, lane1, v2, lane2): twice the column shared memory.
 template <int KP> struct Epi {
   // a 16-entry list (32 registers) spills at the 96 registers of 20 warps: 12 warps, 168 registers
   static constexpr int PARTS = KP == 16 ? 2 : EPI_PARTS;
   static constexpr int THREADS = 32 * EPI_WARP0 + 128 * PARTS;
   static constexpr int CHUNKS = BN / PARTS / EPI_CW;
+  static constexpr int COL_BYTES = KP == KP_COLS ? 2 * COL_SMEM_BYTES : COL_SMEM_BYTES;
 };
-static_assert(Epi<0>::THREADS == K2_THREADS, "the top-2 kernel keeps its 20 warps");
-template <bool PAIR> constexpr int k2_smem_bytes() { return 1024 /*align slack*/ + Ring<PAIR>::BYTES + COL_SMEM_BYTES + 256 /*barriers*/; }
+static_assert(Epi<0>::THREADS == K2_THREADS && Epi<KP_COLS>::THREADS == K2_THREADS, "the top-2 kernels keep their 20 warps");
+template <bool PAIR, int KP = 0> constexpr int k2_smem_bytes() {
+  return 1024 /*align slack*/ + Ring<PAIR>::BYTES + Epi<KP>::COL_BYTES + 256 /*barriers*/;
+}
+static_assert(k2_smem_bytes<false, KP_COLS>() <= 232448 && k2_smem_bytes<true, KP_COLS>() <= 232448,
+              "the column top-2 slots fit the 227 KB of dynamic shared memory of a CTA");
 
 struct K2Sched {
   // tiles are numbered t = sb * n_ct + ct and cut into tk work UNITS each; cluster c owns the units
@@ -118,6 +131,7 @@ struct K2Params {
   unsigned long long* col_best;
   float* S_out;     // optional (n_max, ld_s) fp32: the similarity tile is also written out (affinity consumers, mv_k2_affinity)
   int ld_s;
+  float4* col_rec;  // KP_COLS: (ceil(n_max / 128), m_max) column top-2 records {v1, r1, v2, r2} of every 128-row block
 };
 
 __host__ __device__ inline K2Sched make_sched(int n, int m, int mc, int clusters, int kblocks, int streamk) {
@@ -184,7 +198,8 @@ struct __align__(8) Barriers {
 template <bool TF32, int MC, bool PAIR, int KP>
 __device__ __forceinline__ void k2_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const K2Params& p) {
   static_assert(!PAIR || MC == 2, "a CTA pair is a cluster of two");
-  static_assert(KP == 0 || KP == 8 || KP == 16, "row lists of 8 or 16 entries");
+  static_assert(KP == 0 || KP == 8 || KP == 16 || KP == KP_COLS, "row lists of 8 or 16 entries, or the column top-2");
+  constexpr bool COLS2 = KP == KP_COLS;
   constexpr int STAGES = Ring<PAIR>::STAGES;
   constexpr int STAGE_BYTES = Ring<PAIR>::STAGE_BYTES;
   extern __shared__ uint8_t smem_raw[];
@@ -192,7 +207,7 @@ __device__ __forceinline__ void k2_body(const CUtensorMap& tmA, const CUtensorMa
   uint8_t* smem_al = smem_raw + (smem_base - smem_u32(smem_raw));
   constexpr int RING_BYTES = Ring<PAIR>::BYTES;
   uint2* col_smem = reinterpret_cast<uint2*>(smem_al + RING_BYTES);
-  Barriers* bars = reinterpret_cast<Barriers*>(smem_al + RING_BYTES + COL_SMEM_BYTES);
+  Barriers* bars = reinterpret_cast<Barriers*>(smem_al + RING_BYTES + Epi<KP>::COL_BYTES);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int rank = (MC > 1) ? (int)cluster_ctarank() : 0;
@@ -576,6 +591,20 @@ __device__ __forceinline__ void k2_body(const CUtensorMap& tmA, const CUtensorMa
         // 0.354 ms: at small K the tile time (~4.7 us per 128 x 256 tile) does not depend on K or on the operand traffic at
         // all, it is the epilogue's own instruction stream (TMEM reads alone: 128 KB per tile at 64 B/clk = 2048 of ~9000 clk).)
 #ifndef MV_K2_EXP_NO_COLS
+        if constexpr (COLS2) {
+          // the best two of the warp's 32 rows: the warp max, then the warp max with the first lane holding it masked
+          // (equal values: the lower lane = the lower row comes first)
+          uint4* colw2 = reinterpret_cast<uint4*>(col_smem) + (size_t)acc * (4 * BN) + ew * BN + ch * EPI_CW;
+#pragma unroll
+          for (int q = 0; q < EPI_CW; ++q) {
+            const float x = warp_max_f32(v[q]);
+            const int l1 = __ffs((int)__ballot_sync(0xffffffffu, v[q] == x)) - 1;
+            const float vm = lane == l1 ? -CUDART_INF_F : v[q];
+            const float y = warp_max_f32(vm);
+            const int l2 = __ffs((int)__ballot_sync(0xffffffffu, vm == y)) - 1;
+            if (lane == 0) colw2[q] = make_uint4(__float_as_uint(x), (uint32_t)l1, __float_as_uint(y), (uint32_t)l2);
+          }
+        } else
 #pragma unroll
         for (int q = 0; q < EPI_CW; q += 2) {
           const float x0 = warp_max_f32(v[q]), x1 = warp_max_f32(v[q + 1]);
@@ -597,7 +626,30 @@ __device__ __forceinline__ void k2_body(const CUtensorMap& tmA, const CUtensorMa
       // combine the 4 warps' column results of this part; thread e < PART_COLS owns column e + PART_COLS * half
       named_bar_sync(1 + half, 128);
       const uint2* colr = col_smem + (size_t)acc * (4 * BN);
-      if (e < PART_COLS) {
+      if constexpr (COLS2) {
+        // the warps' best two in row order -> the row block's best two, one record per (row block, column): each tile is
+        // computed by exactly one CTA (no stream-K), so nothing is combined across CTAs here
+        const int c = e + half * PART_COLS;
+        const int col = col0 + c;
+        if (e < PART_COLS && row0 < n && col < m) {
+          const uint4* colr2 = reinterpret_cast<const uint4*>(col_smem) + (size_t)acc * (4 * BN);
+          float v1 = -CUDART_INF_F, v2 = -CUDART_INF_F;
+          int r1 = -1, r2 = -1;
+#pragma unroll
+          for (int w = 0; w < 4; ++w) {
+            const uint4 r = colr2[w * BN + c];
+            const float xs[2] = {__uint_as_float(r.x), __uint_as_float(r.z)};
+            const int rs[2] = {row0 + w * 32 + (int)r.y, row0 + w * 32 + (int)r.w};
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+              if (!(xs[u] > -CUDART_INF_F)) continue;  // masked rows (past n) are never candidates
+              if (better(xs[u], rs[u], v1, r1)) { v2 = v1; r2 = r1; v1 = xs[u]; r1 = rs[u]; }
+              else if (better(xs[u], rs[u], v2, r2)) { v2 = xs[u]; r2 = rs[u]; }
+            }
+          }
+          p.col_rec[(size_t)(row0 / BM) * p.m_max + col] = make_float4(v1, __int_as_float(r1), v2, __int_as_float(r2));
+        }
+      } else if (e < PART_COLS) {
         const int c = e + half * PART_COLS;
         float best = -CUDART_INF_F;
         int brow = 0;
@@ -636,6 +688,12 @@ template <bool TF32, int MC, bool PAIR>
 __global__ void __launch_bounds__(K2_THREADS, 1)
     k2_sim_top2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, K2Params p) {
   k2_body<TF32, MC, PAIR, 0>(tmA, tmB, p);
+}
+
+template <bool TF32, int MC, bool PAIR>
+__global__ void __launch_bounds__(K2_THREADS, 1)
+    k2_sim_top2_cols_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, K2Params p) {
+  k2_body<TF32, MC, PAIR, KP_COLS>(tmA, tmB, p);
 }
 
 template <bool TF32, int MC, bool PAIR, int KP>
@@ -732,6 +790,36 @@ __global__ void k2_merge_rows_kernel(int clusters, int kblocks, int streamk, con
   row_idx[2 * (size_t)i + 1] = i2;
 }
 
+// fold the column top-2 records of the row blocks [0, ceil(n / 128)) in ascending order (ties: lower row); write
+// (m_max, 2) value / row pairs (missing: MV_MASKED_F / -1) and the packed arg-max of mv_k2_sim_top2's col_best
+__global__ void k2_merge_cols_kernel(const float4* __restrict__ col_rec, const int32_t* __restrict__ n_dev, int n_max,
+                                     const int32_t* __restrict__ m_dev, int m_max, float* __restrict__ col_val,
+                                     int32_t* __restrict__ col_idx, unsigned long long* __restrict__ col_best) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= m_max) return;
+  const int n = n_dev ? min(*n_dev, n_max) : n_max;
+  const int m = m_dev ? min(*m_dev, m_max) : m_max;
+  float v1 = -CUDART_INF_F, v2 = -CUDART_INF_F;
+  int r1 = -1, r2 = -1;
+  if (j < m) {
+    const int blocks = (n + BM - 1) / BM;
+    for (int b = 0; b < blocks; ++b) {
+      const float4 r = __ldcs(col_rec + (size_t)b * m_max + j);
+      const int ra = __float_as_int(r.y), rb = __float_as_int(r.w);
+      if (ra >= 0) {
+        if (better(r.x, ra, v1, r1)) { v2 = v1; r2 = r1; v1 = r.x; r1 = ra; }
+        else if (better(r.x, ra, v2, r2)) { v2 = r.x; r2 = ra; }
+      }
+      if (rb >= 0 && better(r.z, rb, v2, r2)) { v2 = r.z; r2 = rb; }  // a record's second never beats its first
+    }
+  }
+  col_val[2 * (size_t)j] = r1 >= 0 ? v1 : MV_MASKED_F;
+  col_val[2 * (size_t)j + 1] = r2 >= 0 ? v2 : MV_MASKED_F;
+  col_idx[2 * (size_t)j] = r1;
+  col_idx[2 * (size_t)j + 1] = r2;
+  col_best[j] = r1 >= 0 ? ((unsigned long long)f32_orderable(v1) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)r1) : 0ull;
+}
+
 __global__ void k2_unpack_col_kernel(const unsigned long long* __restrict__ col_best, int m, float* __restrict__ col_val,
                                      int32_t* __restrict__ col_idx) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
@@ -813,6 +901,7 @@ int pick_mc(int cluster) { return cluster <= 1 ? 1 : (cluster >= 4 ? 4 : 2); }
 template <bool TF32, int MC, bool PAIR, int KP>
 constexpr auto k2_kernel() {
   if constexpr (KP == 0) return k2_sim_top2_kernel<TF32, MC, PAIR>;
+  else if constexpr (KP == KP_COLS) return k2_sim_top2_cols_kernel<TF32, MC, PAIR>;
   else return k2_sim_topk_kernel<TF32, MC, PAIR, KP>;
 }
 
@@ -823,7 +912,7 @@ int k2_max_clusters() {
   if (cached) return cached;
   auto kern = k2_kernel<TF32, MC, PAIR, KP>();
   int n = mv_sm_count() / MC;
-  constexpr int K2_SMEM_BYTES = k2_smem_bytes<PAIR>();
+  constexpr int K2_SMEM_BYTES = k2_smem_bytes<PAIR, KP>();
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_BYTES) == cudaSuccess && MC > 1) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(mv_sm_count() / MC * MC);
@@ -857,7 +946,7 @@ int k2_grid(int mc, bool tf32, bool pair = false) {
 template <bool TF32, int MC, bool PAIR = false, int KP = 0>
 int launch_k2(const CUtensorMap& tmA, const CUtensorMap& tmB, const K2Params& p, int grid, cudaStream_t st) {
   auto kern = k2_kernel<TF32, MC, PAIR, KP>();
-  constexpr int K2_SMEM_BYTES = k2_smem_bytes<PAIR>();
+  constexpr int K2_SMEM_BYTES = k2_smem_bytes<PAIR, KP>();
   static bool done[MV_MAX_DEVICES];
   bool& attr_done = done[mv_device_slot()];
   if (!attr_done) {
@@ -979,6 +1068,17 @@ size_t k2_topk_workspace_bytes(int n_max, int kp) {
   size_t worst = 0;
   for (int mc = 1; mc <= 4; mc *= 2) {
     const size_t b = k2_topk_partial_bytes(n_max, mc, mv_sm_count() / mc, kp);
+    if (b > worst) worst = b;
+  }
+  return worst;
+}
+
+// column top-2 records behind the row records: (ceil(n_max / 128), m_max) float4
+size_t k2_col_rec_bytes(int n_max, int m_max) { return (size_t)((n_max + BM - 1) / BM) * (size_t)m_max * sizeof(float4); }
+size_t k2_cols_row_bytes(int n_max) {
+  size_t worst = 0;
+  for (int mc = 1; mc <= 4; mc *= 2) {
+    const size_t b = k2_partial_bytes(n_max, mc, mv_sm_count() / mc);
     if (b > worst) worst = b;
   }
   return worst;
@@ -1144,6 +1244,49 @@ int mv_k2_sim_topk_ld(const void* A, int lda, const void* B, int ldb, int n_max,
     else if (mc == 2) k2_merge_topk_kernel<2, 16><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
     else k2_merge_topk_kernel<4, 16><<<blocks, mt, 0, st>>>(p.clusters, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
   }
+  MV_LAUNCH_CHECK();
+  return MV_OK;
+}
+
+size_t mv_k2_cols_workspace_bytes(int n_max, int m_max) {
+  if (n_max <= 0 || m_max <= 0) return 0;
+  return k2_cols_row_bytes(n_max) + k2_col_rec_bytes(n_max, m_max);
+}
+
+int mv_k2_sim_top2_cols_ld(const void* A, int lda, const void* B, int ldb, int n_max, int m_max, int C, const int32_t* n_dev,
+                           const int32_t* m_dev, int dtype, int cluster, float* row_val, int32_t* row_idx, float* col_val,
+                           int32_t* col_idx, unsigned long long* col_best, void* workspace, size_t workspace_bytes,
+                           mv_stream_t stream) {
+  MV_REQUIRE(A && B && row_val && row_idx && col_val && col_idx && col_best && workspace, MV_E_ARG,
+             "mv_k2_sim_top2_cols_ld: null pointer");
+  int rc = k2_check_operands("mv_k2_sim_top2_cols_ld", lda, ldb, n_max, m_max, C, dtype, A, B, workspace);
+  if (rc) return rc;
+  // the worst case over the cluster forms, so that the check needs no device
+  const size_t row_bytes = k2_cols_row_bytes(n_max);
+  const size_t need = row_bytes + k2_col_rec_bytes(n_max, m_max);
+  MV_REQUIRE(workspace_bytes >= need, MV_E_WORKSPACE, "mv_k2_sim_top2_cols_ld: workspace has %zu bytes, %zu needed",
+             workspace_bytes, need);
+  K2Launch k;
+  rc = k2_prepare<KP_COLS>("mv_k2_sim_top2_cols_ld", n_max, m_max, C, n_dev, m_dev, dtype, cluster, k);
+  if (rc) return rc;
+  K2Params& p = k.p;
+  p.partial = reinterpret_cast<float4*>(workspace);
+  p.col_rec = reinterpret_cast<float4*>(reinterpret_cast<uint8_t*>(workspace) + row_bytes);
+  p.streamk = 0;  // tile-granular schedule only: every tile's column records come from one CTA
+
+  CUtensorMap tmA, tmB;
+  rc = k2_operand_maps(&tmA, &tmB, A, lda, B, ldb, n_max, m_max, C, dtype, k.mc);
+  if (rc) return rc;
+  cudaStream_t st = mv_cuda_stream(stream);
+  rc = launch_k2_form<KP_COLS>(k.tf32, k.mc, k.pair, tmA, tmB, p, k.grid, st);
+  if (rc) return rc;
+  const int mt = 256;
+  const int mc = k.mc;
+  if (mc == 1) k2_merge_rows_kernel<1><<<(n_max + mt - 1) / mt, mt, 0, st>>>(p.clusters, p.kblocks, 0, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+  else if (mc == 2) k2_merge_rows_kernel<2><<<(n_max + mt - 1) / mt, mt, 0, st>>>(p.clusters, p.kblocks, 0, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+  else k2_merge_rows_kernel<4><<<(n_max + mt - 1) / mt, mt, 0, st>>>(p.clusters, p.kblocks, 0, p.partial, n_dev, n_max, m_dev, m_max, row_val, row_idx);
+  MV_LAUNCH_CHECK();
+  k2_merge_cols_kernel<<<(m_max + mt - 1) / mt, mt, 0, st>>>(p.col_rec, n_dev, n_max, m_dev, m_max, col_val, col_idx, col_best);
   MV_LAUNCH_CHECK();
   return MV_OK;
 }

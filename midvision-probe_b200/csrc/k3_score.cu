@@ -3,6 +3,8 @@
 //   mv_k3_ratio_mutual   fp32 recompute of the two cosine distances per query, re-rank, Lowe ratio
 //                        weight, mutual-nearest-neighbour flag
 //   mv_k3_topk_matches   the num_corr largest weights, sorted (radix select + bitonic sort, one CTA)
+//   mv_k3_mutual_select  two-sided mutual test on the forward and reverse re-ranked candidates, min weight, and the
+//                        top num_corr of the mutual queries (k on the device)
 //   mv_k3_score          Rt transform, K projection, 3-D / 2-D errors, integer threshold hit counts
 //   mv_gather_rows       row gather for the helper's return tuples
 //   mv_k3_spair_errors   SPair keypoint error matrix, error_same / error_nn, PCK hit counts
@@ -55,6 +57,7 @@ struct RowsF16c {
   const __half* B_lo;
   const float* center_B;  // may be null
   int pitch;              // row pitch of the hi planes (>= C + 8)
+  const float* center_A;  // may be null: the reverse pass of a mutual match, whose query rows are target-role rows
 };
 
 __device__ __forceinline__ void f16c8(const __half* hi, const __half* lo, int c8, float (&out)[8]) {
@@ -136,6 +139,13 @@ __global__ void __launch_bounds__(RATIO_THREADS, 6) k3_ratio_mutual_kernel(ROWS 
         f16c8(xh, rows.A_lo + ox, c8, v);
         f16c8(ah, rows.B_lo + o0, c8, a);
         f16c8(bh, rows.B_lo + o1, c8, b);
+        if (rows.center_A) {
+          const float4 m0 = __ldg(reinterpret_cast<const float4*>(rows.center_A) + 2 * c8);
+          const float4 m1 = __ldg(reinterpret_cast<const float4*>(rows.center_A) + 2 * c8 + 1);
+          const float mu[8] = {m0.x, m0.y, m0.z, m0.w, m1.x, m1.y, m1.z, m1.w};
+#pragma unroll
+          for (int k = 0; k < 8; ++k) v[k] += mu[k];
+        }
         if (rows.center_B) {
           const float4 m0 = __ldg(reinterpret_cast<const float4*>(rows.center_B) + 2 * c8);
           const float4 m1 = __ldg(reinterpret_cast<const float4*>(rows.center_B) + 2 * c8 + 1);
@@ -188,6 +198,7 @@ __global__ void __launch_bounds__(RATIO_THREADS, 6) k3_ratio_mutual_kernel(ROWS 
       if (aa < F16C_ZERO_SS) xa = 0.f;
       if (bb < F16C_ZERO_SS) xb = 0.f;
     }
+    if (rows.center_A && xx < F16C_ZERO_SS) xa = xb = 0.f;
   }
   const float nx = fmaxf(sqrtf(xx), COS_EPS);
   float d0 = j0 >= 0 ? 1.f - xa / (nx * fmaxf(sqrtf(aa), COS_EPS)) : MISSING_DIST;
@@ -464,6 +475,39 @@ __global__ void __launch_bounds__(TOPK_THREADS) k3_topk_kernel(const float* __re
 }
 
 // ------------------------------------------------------------------------------------------
+// mutual matches: query i is mutual iff the re-ranked best row of its re-ranked best column is i again.  The selection
+// weight of a mutual query is min(w_f(i), w_r(j(i))) with the ratio test, w_f(i) (= d0) without; every other query gets
+// -inf, which sorts below every mutual one, and the count of mutual queries goes to *k_dev (zeroed before)
+// ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k3_mutual_combine_kernel(const int32_t* __restrict__ row_idx, const float* __restrict__ weight_f,
+                                                                const int32_t* __restrict__ col_idx, const float* __restrict__ weight_r,
+                                                                const int32_t* __restrict__ n_dev, int n_max, int ratio_test,
+                                                                float* __restrict__ weight, uint8_t* __restrict__ mutual,
+                                                                int32_t* __restrict__ count) {
+  __shared__ int s_count;
+  if (threadIdx.x == 0) s_count = 0;
+  __syncthreads();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int n = n_dev ? min(*n_dev, n_max) : n_max;
+  bool mu = false;
+  if (i < n) {
+    const int j = row_idx[2 * (size_t)i];
+    mu = j >= 0 && col_idx[2 * (size_t)j] == i;
+    const float wf = weight_f[i];
+    weight[i] = mu ? (ratio_test ? fminf(wf, weight_r[j]) : wf) : -CUDART_INF_F;
+    if (mutual) mutual[i] = mu ? 1 : 0;
+  }
+  const uint32_t b = __ballot_sync(0xffffffffu, mu);
+  if ((threadIdx.x & 31) == 0 && b) atomicAdd(&s_count, __popc(b));
+  __syncthreads();
+  if (threadIdx.x == 0 && s_count) atomicAdd(count, s_count);
+}
+
+__global__ void k3_clamp_count_kernel(int32_t* __restrict__ k_dev, int num_corr) {
+  if (*k_dev > num_corr) *k_dev = num_corr;
+}
+
+// ------------------------------------------------------------------------------------------
 // scoring
 // ------------------------------------------------------------------------------------------
 struct ScoreParams {
@@ -674,6 +718,45 @@ int mv_k3_ratio_mutual_f16c(const uint16_t* A_hi, const uint16_t* A_lo, const ui
   RowsF16c rows{reinterpret_cast<const __half*>(A_hi), reinterpret_cast<const __half*>(A_lo), reinterpret_cast<const __half*>(B_hi),
                 reinterpret_cast<const __half*>(B_lo), center_B, pitch};
   launch_ratio(rows, C, n_dev, n_max, row_idx, col_best, ratio_test, dists, weight, mutual, mv_cuda_stream(stream));
+  MV_LAUNCH_CHECK();
+  return MV_OK;
+}
+
+int mv_k3_ratio_mutual_f16c_ab(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* B_hi, const uint16_t* B_lo, int C,
+                               int pitch, const float* center_A, const float* center_B, const int32_t* n_dev, int n_max,
+                               int32_t* row_idx, const unsigned long long* col_best, int ratio_test, float* dists, float* weight,
+                               uint8_t* mutual, mv_stream_t stream) {
+  MV_REQUIRE(A_hi && A_lo && B_hi && B_lo && row_idx, MV_E_ARG, "mv_k3_ratio_mutual_f16c_ab: null pointer");
+  MV_REQUIRE(C > 0 && C % 8 == 0, MV_E_ALIGN, "mv_k3_ratio_mutual_f16c_ab: C=%d must be a positive multiple of 8", C);
+  MV_REQUIRE((((uintptr_t)A_hi | (uintptr_t)A_lo | (uintptr_t)B_hi | (uintptr_t)B_lo | (uintptr_t)center_A | (uintptr_t)center_B) & 15) == 0,
+             MV_E_ALIGN, "mv_k3_ratio_mutual_f16c_ab: the row planes and the centres must be 16-byte aligned");
+  MV_REQUIRE(n_max >= 0 && pitch >= C + 8 && pitch % 8 == 0, MV_E_ARG, "mv_k3_ratio_mutual_f16c_ab: negative n_max or bad pitch %d",
+             pitch);
+  if (n_max == 0) return MV_OK;
+  RowsF16c rows{reinterpret_cast<const __half*>(A_hi), reinterpret_cast<const __half*>(A_lo), reinterpret_cast<const __half*>(B_hi),
+                reinterpret_cast<const __half*>(B_lo), center_B, pitch, center_A};
+  launch_ratio(rows, C, n_dev, n_max, row_idx, col_best, ratio_test, dists, weight, mutual, mv_cuda_stream(stream));
+  MV_LAUNCH_CHECK();
+  return MV_OK;
+}
+
+int mv_k3_mutual_select(const int32_t* row_idx, const float* weight_f, const int32_t* col_idx, const float* weight_r,
+                        const int32_t* n_dev, int n_max, int ratio_test, int num_corr, float* weight, uint8_t* mutual,
+                        int32_t* sel_src, int32_t* sel_dst, float* sel_weight, int32_t* k_dev, mv_stream_t stream) {
+  MV_REQUIRE(row_idx && weight_f && col_idx && weight_r && weight && sel_src && sel_dst && sel_weight && k_dev, MV_E_ARG,
+             "mv_k3_mutual_select: null pointer");
+  MV_REQUIRE(n_max >= 0 && n_max <= (1 << 20), MV_E_RANGE, "mv_k3_mutual_select: n_max must be in [0, 2^20]");
+  MV_REQUIRE(num_corr >= 0 && num_corr <= 16384, MV_E_RANGE, "mv_k3_mutual_select: num_corr must be in [0, 16384]");
+  cudaStream_t st = mv_cuda_stream(stream);
+  MV_CUDA(cudaMemsetAsync(k_dev, 0, sizeof(int32_t), st));
+  if (n_max == 0 || num_corr == 0) return MV_OK;
+  k3_mutual_combine_kernel<<<(n_max + 255) / 256, 256, 0, st>>>(row_idx, weight_f, col_idx, weight_r, n_dev, n_max, ratio_test, weight,
+                                                                mutual, k_dev);
+  MV_LAUNCH_CHECK();
+  // the non-mutual queries carry -inf: the first min(num_corr, #mutual) selected are exactly the mutual ones
+  int rc = mv_k3_topk_matches(weight, row_idx, n_dev, n_max, num_corr, sel_src, sel_dst, sel_weight, nullptr, stream);
+  if (rc) return rc;
+  k3_clamp_count_kernel<<<1, 1, 0, st>>>(k_dev, num_corr);
   MV_LAUNCH_CHECK();
   return MV_OK;
 }

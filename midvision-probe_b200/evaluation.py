@@ -262,12 +262,18 @@ class GraphedPairMatcher:
     """
 
     def __init__(self, kind, feat_shape, grid_shape, num_corr, K=None, device=None, ratio_test=True, with_outputs=False,
-                 feat_layout="chw", feat_dtype=torch.float32, split=False):
+                 feat_layout="chw", feat_dtype=torch.float32, split=False, mutual=False):
         """feat_layout: memory layout of the static feature buffers -- "chw" (the reference's contiguous
         (C, h, w)) or "hwc" (channel-last views, the layout ViT tokens / channels_last CNN outputs already have:
-        loading such features is a flat copy and the transpose kernel is skipped)."""
+        loading such features is a flat copy and the transpose kernel is skipped).
+        mutual: select mutual matches with the two-sided ratio test (correspondence.get_mutual_correspondences) -- in the
+        single graph and in the split form alike; the selection's length stays on the device (match.k_dev <= match.k), which
+        RecallAccumulator.score reads there."""
         if kind not in ("xyz", "depth"):
             raise ValueError(kind)
+        if not isinstance(mutual, bool):
+            raise TypeError(f"mutual must be a bool, not {type(mutual).__name__}")
+        self.mutual = mutual
         if feat_layout not in ("chw", "hwc"):
             raise ValueError(feat_layout)
         # split: TWO graphs -- the target image's side (its map, the f16c centre, kernel 1) and everything else -- so that a
@@ -354,7 +360,7 @@ class GraphedPairMatcher:
         self.lowrank_exact = s0.rows16 is None and s0.rows32 is None
         self.lowrank_used = (not self.lowrank_exact and s0.rows_lo is not None and s0.fshape == s1.fshape
                              and C_.lowrank_applies(*s0.fshape, s0.n, s1.n, s0.mode))
-        r = C_._match_sides(s0, s1, s0.n, s1.n, self.num_corr, self.ratio_test, n_dev=s0.n_dev, m_dev=s1.n_dev)
+        r = C_._match_sides(s0, s1, s0.n, s1.n, self.num_corr, self.ratio_test, n_dev=s0.n_dev, m_dev=s1.n_dev, mutual=self.mutual)
         if self.with_outputs:
             # the helper's return tuple + the live counts in one buffer of column blocks (mv_pack_matches):
             # a single device -> host copy, and the host slices views out of it
@@ -491,11 +497,13 @@ class GraphedPairMatcher:
         # per image: (backproject) + compact + coords + chw_to_hwc + kernel 1; per pair: (centre: 2, pixel dots: 1) + kernel 2 (2) + ratio + top-k
         zero_copy = self.feat_layout == "hwc" and self.feat_dtype == torch.float32
         per_side = (5 if self.kind == "depth" else 4) - (1 if zero_copy else 0)
+        # mutual: kernel 2's column merge, the reverse kernel 3, and the combine + count clamp around the top-k
+        mutual = 4 if self.mutual else 0
         if getattr(self, "lowrank_exact", False):
             # per image everything but kernel 1; per pair: exact Gram (2), 2 builders, kernel 2 (2), kernel 3 on the Gram, top-k
-            return 2 * (per_side - 1) + 8 + (1 if self.with_outputs else 0)
+            return 2 * (per_side - 1) + 8 + (1 if self.with_outputs else 0) + mutual
         lowrank = 6 if getattr(self, "lowrank_used", False) else 0  # 2 unit-row launches, the Gram launch + its row merge, 2 builders
-        return 2 * per_side + 4 + (3 if C_._CFG["dtype"] != "bf16" else 0) + (1 if self.with_outputs else 0) + lowrank
+        return 2 * per_side + 4 + (3 if C_._CFG["dtype"] != "bf16" else 0) + (1 if self.with_outputs else 0) + lowrank + mutual
 
 
 class PairPipeline:

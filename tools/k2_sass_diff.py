@@ -1,11 +1,14 @@
 """Compare the SASS of kernel 2's top-2 instantiations between two builds of csrc/k2_sim.cu (no GPU needed).
 
     python tools/k2_sass_diff.py OLD.o NEW.o
+    python tools/k2_sass_diff.py --topk OLD.o NEW.o       (the same builds, top-KP instantiations)
     python tools/k2_sass_diff.py --spair OLD.o NEW.o      (two builds of csrc/spair_batch.cu)
 
 Each object's `cuobjdump -sass` is cut into functions; the k2_sim_top2_kernel instantiations are keyed by their template
 arguments (TF32, MC, PAIR) and compared instruction by instruction after stripping addresses, encodings and symbol names.
 Exit status 0 = every instantiation identical.  For changes that share kernel 2's main loop with another epilogue.
+
+--topk compares the row top-KP instantiations (k2_sim_topk_kernel) instead, keyed by (TF32, MC, PAIR, KP).
 
 --spair compares the fp32 instantiations of the SPair batch kernels instead: spair_stream_kernel keyed by (KT, MMA, TERMS)
 and spair_batch_kernel by KT.  Builds that template them on the map's element type as well carry a leading `f` in the
@@ -22,6 +25,11 @@ CUOBJDUMP = "/usr/local/cuda/bin/cuobjdump"
 def k2_key(name):
     t = re.search(r"k2_sim_top2_kernelILb(\d)ELi(\d)ELb(\d)E", name)
     return tuple(int(x) for x in t.groups()) if t else None
+
+
+def k2_topk_key(name):
+    t = re.search(r"k2_sim_topk_kernelILb(\d)ELi(\d)ELb(\d)ELi(\d+)E", name)
+    return ("topk",) + tuple(int(x) for x in t.groups()) if t else None
 
 
 def spair_key(name):
@@ -56,14 +64,17 @@ def top2_functions(obj, key_of=k2_key):
 def key_name(key):
     if key[0] == "stream":
         return "spair_stream_kernel KT=%d MMA=%d TERMS=%d" % key[1:]
+    if key[0] == "topk":
+        return "TF32=%d MC=%d PAIR=%d KP=%d" % key[1:]
     if key[0] == "batch":
         return "spair_batch_kernel KT=%d" % key[1:]
     return "TF32=%d MC=%d PAIR=%d" % key
 
 
-def main(old, new, spair=False):
-    a, b = top2_functions(old, spair_key if spair else k2_key), top2_functions(new, spair_key if spair else k2_key)
-    want = 24 if spair else 8  # spair: 6 key-point tiles x (3 streaming forms + the first form)
+def main(old, new, spair=False, topk=False):
+    key_of = spair_key if spair else (k2_topk_key if topk else k2_key)
+    a, b = top2_functions(old, key_of), top2_functions(new, key_of)
+    want = 24 if spair else (16 if topk else 8)  # spair: 6 key-point tiles x (3 streaming forms + the first form); topk: KP 8 and 16
     ok = True
     for key in sorted(set(a) | set(b)):
         name = key_name(key)
@@ -79,5 +90,5 @@ def main(old, new, spair=False):
 
 
 if __name__ == "__main__":
-    args = [x for x in sys.argv[1:] if x != "--spair"]
-    sys.exit(main(*args[:2], spair="--spair" in sys.argv[1:]))
+    args = [x for x in sys.argv[1:] if x not in ("--spair", "--topk")]
+    sys.exit(main(*args[:2], spair="--spair" in sys.argv[1:], topk="--topk" in sys.argv[1:]))
